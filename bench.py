@@ -3,6 +3,7 @@
 reference's CPU carve (the oracle restatement) timed on the same box.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config C4|C3|C5|C4-noisy|C1|C2|ref6] [--impl ours|reference]
+                  [--dump-outputs DIR]
 
 Step = one full carve (Model ctor state -> occupied + seen volumes complete) of the synthetic workload
 BASELINE.json quotes the metric on (default C4: 1024^3 x 72 views, 1920x1080 silhouettes; SURVEY §8d).
@@ -65,7 +66,13 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-color", action="store_true", help="skip the colour-reconstruction timing (uploads V x H x W x 3 image bytes)")
     ap.add_argument("--uniform-slabs", action="store_true", help="equal-height z-slabs instead of the planner's balanced ones")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.config in SMALL):
+        ap.error("--dump-outputs needs --impl ours and a synthetic config (C3, C4, C4-noisy, C5)")
+    return a
 
 
 def config_dict(w, n_gpus, name):
@@ -90,6 +97,24 @@ def workload_name(w):
 
 def grid_hash(words):
     return hashlib.blake2b(np.ascontiguousarray(words).view(np.uint8), digest_size=8).hexdigest()
+
+
+DUMP_SAMPLE_WORDS = 1 << 20
+
+
+def dump_outputs(out_dir, occ, seen):
+    """--dump-outputs: the occupied and seen volumes a caller of the timed step receives (uint32 words [Z][Y][ceil(X/32)]), cut to
+    a size that can be kept and compared between builds (C4: 32 MiB, C5: 56 MiB):
+      word_index.npy          flat word positions of a fixed sample (seed 0; every word when there are at most 2^20)
+      <volume>_words.npy      the words at those positions, float64 (exact for uint32)
+      <volume>_row_counts.npy set bits of every row [Z][Y], float32 (exact up to 2^24): every voxel counts somewhere"""
+    os.makedirs(out_dir, exist_ok=True)
+    n = occ.size
+    idx = np.arange(n) if n <= DUMP_SAMPLE_WORDS else np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE_WORDS, replace=False))
+    np.save(os.path.join(out_dir, "word_index.npy"), idx.astype(np.float64))
+    for name, vol in (("occupied", occ), ("seen", seen)):
+        np.save(os.path.join(out_dir, f"{name}_words.npy"), vol.reshape(-1)[idx].astype(np.float64))
+        np.save(os.path.join(out_dir, f"{name}_row_counts.npy"), np.bitwise_count(vol).sum(axis=-1, dtype=np.uint32).astype(np.float32))
 
 
 # ------------------------------------------------------------------------------ clocks
@@ -280,13 +305,13 @@ def run_small(args, reference_only=False):
                     e.synchronize()
                 for _ in range(args.warmup):
                     do_carve()
-                g["carve"] = wall(do_carve, max(args.steps, 5))
+                g["carve"] = wall(do_carve, args.steps)
                 g["carve_device_only"] = e.stats()["last_carve_ms"] if method == 1 else None
 
                 def do_color():
                     e.color(2), e.synchronize()
                 do_color()
-                g["color_avg"] = wall(do_color, max(args.steps, 5))
+                g["color_avg"] = wall(do_color, args.steps)
                 e.dense_from_volumes(apply_colors=True, handle_unseen=True), e.synchronize()
                 g["model_on_device"] = wall(lambda: (e.dense_from_volumes(apply_colors=True, handle_unseen=True), e.synchronize()), 5)
 
@@ -351,6 +376,8 @@ def run_ours(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device; the engine has no CPU fallback")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("bench.py: --dump-outputs writes the whole grid of a single-process run; each rank here holds only its slab")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
@@ -447,6 +474,7 @@ def run_ours(args):
         flush.fill_(1)
         step()
     ms_per_step = timed(step, args.steps)
+    dumped = (eng.download_occupied(), eng.download_seen()) if args.dump_outputs else None   # the last timed step's result
     n_tail = 0
     while time.perf_counter() - t_clk < 2.0:  # keep the same load up until the sampler has ~20 samples
         flush.fill_(1)
@@ -734,6 +762,8 @@ def run_ours(args):
         dist.barrier()
         dist.destroy_process_group()
     if rank == 0:
+        if dumped:
+            dump_outputs(args.dump_outputs, *dumped)
         emit(out)
     return 0
 
