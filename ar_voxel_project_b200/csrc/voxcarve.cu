@@ -588,6 +588,11 @@ int vc_set_views(vc_engine* e, int32_t V, int32_t W, int32_t H, const float* P, 
     if (!P) return fail(e, VC_ERR_ARG, "vc_set_views: P is null");
     if (V < 1 || V > VC_MAX_VIEWS) return fail(e, VC_ERR_ARG, "vc_set_views: V=%d outside [1,%d]", V, VC_MAX_VIEWS);
     if (W < 1 || H < 1 || W > (1 << 20) || H > (1 << 20)) return fail(e, VC_ERR_ARG, "vc_set_views: image size %dx%d outside [1,2^20]", W, H);
+    // every check before any state changes: a refused call leaves the engine's views, masks, tables and images as they were
+    const int Ww = (W + 31) / 32;
+    const size_t mask_bytes = (size_t)V * H * Ww * 4;
+    if ((unsigned long long)vc_sat_pitch(W) * (H + 1) > 0x7fffffffull) return fail(e, VC_ERR_ARG, "vc_set_views: image %dx%d too large for 32-bit SAT offsets", W, H);
+    if (mask_bytes / 4 > 0x7fffffffull) return fail(e, VC_ERR_ARG, "vc_set_views: %d views of %dx%d exceed 2^31 mask words", V, W, H);
     if (bind_device(e)) return VC_ERR_CUDA;
     VC_CUDA(e, cudaStreamSynchronize(e->stream));
     if (V != e->V || W != e->W || H != e->H) {  // geometry changed: masks / images no longer match
@@ -596,10 +601,8 @@ int vc_set_views(vc_engine* e, int32_t V, int32_t W, int32_t H, const float* P, 
         cudaFree(e->d_sat_tmp); e->d_sat_tmp = nullptr;
         cudaFree(e->d_images); e->d_images = nullptr;
     }
-    e->V = V; e->W = W; e->H = H; e->Ww = (W + 31) / 32;
-    e->mask_bytes = (size_t)V * H * e->Ww * 4;
-    if ((unsigned long long)vc_sat_pitch(W) * (H + 1) > 0x7fffffffull) return fail(e, VC_ERR_ARG, "vc_set_views: image %dx%d too large for 32-bit SAT offsets", W, H);
-    if (e->mask_bytes / 4 > 0x7fffffffull) return fail(e, VC_ERR_ARG, "vc_set_views: %d views of %dx%d exceed 2^31 mask words", V, W, H);
+    e->V = V; e->W = W; e->H = H; e->Ww = Ww;
+    e->mask_bytes = mask_bytes;
     e->h_view.resize(V);
     e->h_cam.assign((size_t)V * 4, 0.0f);
     e->h_filt.assign((size_t)V, VcViewFilter{});

@@ -120,7 +120,10 @@ VC_EXPORT int vc_set_profiling(vc_engine* e, int32_t on);
  * estimatePoseFromImage + pose.inv() of VoxelCarving.cpp:25-30, ColorReconstruction.h:17-21):
  *   P[v] = intr(CV_32F) * pose(3x4)  — first product of VoxelCarving.cpp:19, 12 f32 row-major
  *   M[v] = pose(3x4) world->camera   — only its translation column is used (ColorReconstruction.h:21);
- *          may be NULL if no colour pass is run. All pointers are HOST memory. */
+ *          may be NULL if no colour pass is run. All pointers are HOST memory.
+ * Accepted: V in [1,256]; W, H in [1,2^20]; pitch*(H+1) < 2^31 with pitch = 32*(ceil(W/32)+1) (32-bit row offsets of a
+ * view's summed-area table); V*H*ceil(W/32) < 2^31 mask words.  Anything else returns VC_ERR_ARG and changes nothing: the
+ * engine keeps its previous views, masks, tables and images. */
 VC_EXPORT int vc_set_views(vc_engine* e, int32_t V, int32_t W, int32_t H, const float* P, const float* M);
 /* Undistorted silhouette masks (VoxelCarving.cpp:36). VC_MASK_BITS: uint32[V][H][ceil(W/32)],
  * bit x&31 of word x>>5, 1 = background (pixel == (0,0,0), VoxelCarving.cpp:50).

@@ -80,8 +80,9 @@ def rect_of_box(P, lo, hi, s, W, H):
     return (4, fl(lo_u), fl(hi_u), fl(lo_v), fl(hi_v))
 
 
-def random_camera(rng, extent, W, H):
-    """P = K [R | t] in f32 looking roughly at the grid from a random place - from inside the grid to twenty extents away"""
+def random_camera(rng, extent, W, H, fit=False):
+    """P = K [R | t] in f32 looking roughly at the grid from a random place - from inside the grid to twenty extents away.
+    fit: the vertical focal length scales with H instead of W, so that projections reach across very wide or very tall images"""
     c = np.array([0.5, 0.5, -0.5]) * extent
     d = rng.normal(size=3); d /= np.linalg.norm(d)
     dist = extent * 10 ** rng.uniform(-1.0, 1.3)
@@ -90,9 +91,26 @@ def random_camera(rng, extent, W, H):
     upv = rng.normal(size=3); r = np.cross(f, upv); r /= np.linalg.norm(r); u = np.cross(f, r)
     R = np.stack([r, u, f]); t = -R @ eye
     fl = W * 10 ** rng.uniform(-0.5, 1.0)
-    K = np.array([[fl, 0, W * rng.uniform(0.2, 0.8)], [0, fl * rng.uniform(0.8, 1.25), H * rng.uniform(0.2, 0.8)], [0, 0, 1]])
+    K = np.array([[fl, 0, W * rng.uniform(0.2, 0.8)], [0, fl * rng.uniform(0.8, 1.25) * (H / W if fit else 1.0), H * rng.uniform(0.2, 0.8)], [0, 0, 1]])
     M = np.concatenate([R, t[:, None]], 1)[:, [1, 0, 2, 3]]   # world = (y s, x s, -z s): columns 0 and 1 act on (wy, wx) like the product's P
     return (K.astype(F) @ M.astype(F)).astype(F)
+
+
+# images at the ends of the accepted sizes: a long side of 2^16 + 1 and of 2^20 (where f32 pixel coordinates have an ulp of 1/8)
+WIDE_TALL = [(65537, 48), (1 << 20, 2046), (48, 1 << 20)]
+
+
+def tie_camera(W, H, offset):
+    """dyadic camera for voxel size 0.25: along the long side the coordinate is 2i + offset (i = x for a wide image, y for a tall
+    one), the other one 24.5 - 2z; with offset = k + 0.5 every voxel lies exactly on a pixel edge"""
+    if W >= H:
+        return np.array([[0, 8, 0, offset], [0, 0, 8, 24.5], [0, 0, 0, 1]], F)
+    return np.array([[0, 0, 8, 24.5], [8, 0, 0, offset], [0, 0, 0, 1]], F)
+
+
+def tie_offsets(W, H):
+    n = max(W, H)
+    return [float(n // 2) + 0.5, float(n) - 100.5]   # |c| > 2^19 for a side of 2^20; the far edge c = n - 0.5 (rounds to n: outside)
 
 
 def test_reference_pixels_equal_the_oracle(oracle):
@@ -107,6 +125,37 @@ def test_reference_pixels_equal_the_oracle(oracle):
             assert bool(ok) == bool(inside[i])
             if ok:
                 assert (opx, opy) == (int(px[i]), int(py[i]))
+    for W, H in WIDE_TALL:   # exact ties far from the origin round half away from zero, in the restatement and the oracle alike
+        for off in tie_offsets(W, H):
+            P = tie_camera(W, H, off)
+            i = np.arange(0, 96)
+            z = np.arange(0, 30)
+            ii, zz = (a.ravel() for a in np.meshgrid(i, z))
+            xs, ys = (ii, np.zeros_like(ii)) if W >= H else (np.zeros_like(ii), ii)
+            px, py, inside = reference_pixels(P, xs, ys, zz, F(0.25), W, H)
+            along = px if W >= H else py
+            assert np.array_equal(along, 2 * ii + off + 0.5)
+            for k in range(0, len(ii), 7):
+                ok, opx, opy, _ = oracle.pixel_of(P, int(xs[k]), int(ys[k]), int(zz[k]), F(0.25), W, H)
+                assert bool(ok) == bool(inside[k])
+                if ok:
+                    assert (opx, opy) == (int(px[k]), int(py[k]))
+
+
+def check_rectangle(P, lo, hi, s, W, H):
+    """rect_of_box's answer for the box [lo, hi] holds for every voxel in it; -> its code"""
+    res = rect_of_box(P, lo, hi, s, W, H)
+    if res[0] == 0:
+        return 0
+    g = np.meshgrid(np.arange(lo[0], hi[0] + 1), np.arange(lo[1], hi[1] + 1), np.arange(lo[2], hi[2] + 1), indexing="ij")
+    px, py, inside = reference_pixels(P, g[0].ravel(), g[1].ravel(), g[2].ravel(), s, W, H)
+    if res[0] == 1:
+        assert not inside.any()
+    else:
+        _, x0, x1, y0, y1 = res
+        assert inside.all()
+        assert px.min() >= x0 and px.max() <= x1 and py.min() >= y0 and py.max() <= y1
+    return res[0]
 
 
 @pytest.mark.parametrize("box", [(128, 32, 32), (32, 8, 8), (8, 8, 8), (8, 4, 4)])
@@ -119,20 +168,27 @@ def test_rectangle_contains_every_voxel_pixel(box):
         P = random_camera(rng, 0.28, W, H)
         lo = np.array([rng.integers(0, max(N - box[k], 1)) for k in range(3)])
         hi = np.minimum(lo + np.array(box) - 1, N - 1)
-        res = rect_of_box(P, lo, hi, s, W, H)
-        if res[0] == 0:
-            continue
-        g = np.meshgrid(np.arange(lo[0], hi[0] + 1), np.arange(lo[1], hi[1] + 1), np.arange(lo[2], hi[2] + 1), indexing="ij")
-        px, py, inside = reference_pixels(P, g[0].ravel(), g[1].ravel(), g[2].ravel(), s, W, H)
-        if res[0] == 1:
-            outside += 1
-            assert not inside.any()
-        else:
-            decided += 1
-            _, x0, x1, y0, y1 = res
-            assert inside.all()
-            assert px.min() >= x0 and px.max() <= x1 and py.min() >= y0 and py.max() <= y1
+        code = check_rectangle(P, lo, hi, s, W, H)
+        outside += code == 1
+        decided += code == 4
     assert decided > 50 and outside > 20   # the sampling exercises both answers
+    # very wide and very tall images, with cameras whose projections reach across them
+    for W, H in WIDE_TALL:
+        codes = []
+        for trial in range(150):
+            N = int(rng.choice([100, 512, 1024, 2048])); s = F(0.28 / N)
+            P = random_camera(rng, 0.28, W, H, fit=True)
+            lo = np.array([rng.integers(0, max(N - box[k], 1)) for k in range(3)])
+            codes.append(check_rectangle(P, lo, np.minimum(lo + np.array(box) - 1, N - 1), s, W, H))
+        # at a side of 2^20 the corner-projection radius exceeds its 1/4 pixel cap and every box stays undecided today (the
+        # check still guards a finer radius); at 2^16 + 1 both answers occur
+        if max(W, H) < 1 << 20:
+            assert codes.count(4) >= 5 and codes.count(1) >= 5, (W, H, codes.count(4), codes.count(1))
+        for off in tie_offsets(W, H):   # boxes whose voxels all lie on pixel edges, in the middle and across the far edge
+            P = tie_camera(W, H, off)
+            for i0 in (0, 40, 47, 50, 60):
+                lo = np.array([i0, 0, 3]) if W >= H else np.array([0, i0, 3])
+                check_rectangle(P, lo, lo + (np.array(box) - 1) // 4, F(0.25), W, H)
 
 
 def filter_constants(P, dims, s, W, H):
@@ -182,11 +238,33 @@ def test_filter_decisions_are_the_reference_pixels():
         W, H = (640, 480) if trial % 3 else (3840, 2160)
         P = random_camera(rng, 0.28, W, H)
         xs, ys, zs = (rng.integers(0, N, 20000) for _ in range(3))
-        consts = filter_constants(P, (N, N, N), s, W, H)
-        dec, px, py, ins = filter_pixels(P, xs, ys, zs, s, W, H, consts)
-        rpx, rpy, rin = reference_pixels(P, xs, ys, zs, s, W, H)
+        dec = check_filter(P, xs, ys, zs, (N, N, N), s, W, H)
         n_total += dec.size; n_decided += int(dec.sum())
-        assert np.array_equal(ins[dec], rin[dec])
-        both = dec & rin
-        assert np.array_equal(px[both], rpx[both].astype(np.int64)) and np.array_equal(py[both], rpy[both].astype(np.int64))
     assert n_decided > 0.5 * n_total   # the filter decides most voxel-views (it is switched off only for degenerate views)
+    # very wide and very tall images.  The radius grows with the image size: at a side of 2^20 the threshold 0.5 - D is about
+    # 1/4 and the view's term Cu |r| at least as large, so nothing is decided there today; the check guards a finer radius.
+    for W, H in WIDE_TALL:
+        n_decided = n_total = 0
+        for trial in range(50):
+            N = int(rng.choice([100, 512, 1024, 2048])); s = F(0.28 / N)
+            P = random_camera(rng, 0.28, W, H, fit=True)
+            xs, ys, zs = (rng.integers(0, N, 20000) for _ in range(3))
+            dec = check_filter(P, xs, ys, zs, (N, N, N), s, W, H)
+            n_total += dec.size; n_decided += int(dec.sum())
+        if max(W, H) < 1 << 20:
+            assert n_decided > 0.3 * n_total, (W, H, n_decided, n_total)
+        for off in tie_offsets(W, H):   # every voxel exactly on a pixel edge
+            i, z = (a.ravel() for a in np.meshgrid(np.arange(96), np.arange(30)))
+            xs, ys = (i, np.zeros_like(i)) if W >= H else (np.zeros_like(i), i)
+            check_filter(tie_camera(W, H, off), xs, ys, z, (96, 96, 30), F(0.25), W, H)
+
+
+def check_filter(P, xs, ys, zs, dims, s, W, H):
+    """every voxel-view the filter decides has the reference's pixel and inside test; -> the decided mask"""
+    consts = filter_constants(P, dims, s, W, H)
+    dec, px, py, ins = filter_pixels(P, xs, ys, zs, s, W, H, consts)
+    rpx, rpy, rin = reference_pixels(P, xs, ys, zs, s, W, H)
+    assert np.array_equal(ins[dec], rin[dec])
+    both = dec & rin
+    assert np.array_equal(px[both], rpx[both].astype(np.int64)) and np.array_equal(py[both], rpy[both].astype(np.int64))
+    return dec
