@@ -89,6 +89,7 @@ SIGNATURES = {
     "vc_dense_download": (C.c_int, [_P, _P]),
     "vc_mc_mesh": (C.c_int, [_P, C.c_float, C.POINTER(C.c_uint64)]),
     "vc_download_mesh": (C.c_int, [_P, _P, _P, C.c_uint64]),
+    "vc_mesh_from_volumes": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.POINTER(C.c_uint64)]),
     "vc_selftest": (C.c_int, [C.c_int32, C.c_int32, C.c_uint64, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "vc_measure_peaks": (C.c_int, [C.c_int32, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
 }

@@ -22,6 +22,8 @@
 #include "mc_tables.inc"
 #include "vc_kernels.cuh"
 
+static_assert(VC_MESH_MAX_CLOSURE == 2 * VC_CLOSURE_SMAX + 1, "vc_dilate_kernel's plane window holds 2 * VC_CLOSURE_SMAX + 1 planes");
+
 namespace {
 
 std::string g_create_error;
@@ -105,7 +107,8 @@ struct vc_engine {
     bool reset_pending = false;          // vc_reset not yet materialised (a VC_EXACT carve folds it into its fill pass)
     bool flags_valid = false;            // the brick / super-brick flags describe the volumes as they are (after a fresh whole-range VC_EXACT carve)
     bool carved_implies_seen = true;     // invariant of every state the engine produces; uploaded volumes may break it (vc_upload_volumes)
-    // grow-only scratch shared by vc_fast_carve (flood volume), vc_mc_mesh (column counts), raw uploads and the
+    // grow-only scratch shared by vc_fast_carve (flood volume), vc_mc_mesh (column counts), vc_mesh_from_volumes (column counts,
+    // record row table, dilated occupancy), raw uploads and the
     // carved-but-unseen path of vc_carve: none of them runs concurrently with another on this engine's stream
     uint32_t *d_sparse_idx = nullptr, *d_sparse_words = nullptr;  // vc_carve_download_sparse (grow-only)
     unsigned long long sparse_cap = 0;
@@ -1661,12 +1664,18 @@ int vc_measure_peaks(int32_t device, double* ffma_tflops, double* dfma_tflops) {
     return VC_OK;
 }
 
+static int load_mc_tables(vc_engine* e);
+
 static int dense_ready(vc_engine* e, const char* who, bool need_data) {
     if (!e->whole_grid()) return fail(e, VC_ERR_STATE, "%s: the dense Model needs the whole grid on one engine", who);
     if (bind_device(e)) return VC_ERR_CUDA;
     const size_t n = (size_t)e->g.X * e->g.Y * e->g.Z;
     if (!e->d_dense) VC_CUDA(e, cudaMalloc(&e->d_dense, n * sizeof(float4)));
     if (need_data && !e->have_dense) return fail(e, VC_ERR_STATE, "%s: no dense Model yet (vc_dense_upload / vc_dense_from_volumes)", who);
+    return load_mc_tables(e);
+}
+
+static int load_mc_tables(vc_engine* e) {
     static std::mutex m;
     static bool tables[64] = {};
     std::lock_guard<std::mutex> lk(m);
@@ -1761,6 +1770,29 @@ int vc_dense_download(vc_engine* e, float* rgba) {
     return VC_OK;
 }
 
+// exclusive scan of the per-column triangle counts into offsets (in place), then room for the triangles in the grow-only mesh
+// buffers.  Refused (VC_ERR_CAPACITY) before anything of the previous mesh is touched when the offsets would overflow.
+static int scan_mesh_counts(vc_engine* e, const char* who, uint32_t* d_counts, unsigned long long* d_sums, long long ncol, int nb,
+                            unsigned long long* total_out) {
+    vc_scan_block_kernel<<<nb, VC_SCAN_BLOCK, 0, e->stream>>>(d_counts, d_counts, d_sums, ncol);
+    vc_scan_sums_kernel<<<1, 1024, 0, e->stream>>>(d_sums, nb, d_sums + nb);
+    vc_scan_add_kernel<<<nb, VC_SCAN_BLOCK, 0, e->stream>>>(d_counts, d_sums, ncol);
+    VC_CUDA(e, cudaGetLastError());
+    unsigned long long total = 0;
+    VC_CUDA(e, cudaMemcpyAsync(&total, d_sums + nb, sizeof total, cudaMemcpyDeviceToHost, e->stream));
+    VC_CUDA(e, cudaStreamSynchronize(e->stream));
+    if (total > 0xffffffffull) return fail(e, VC_ERR_CAPACITY, "%s: %llu triangles exceed 32-bit offsets", who, total);
+    if (total > e->mesh_capacity) {  // triangle buffers are grow-only
+        e->have_mesh = false;
+        cudaFree(e->d_mesh_verts); cudaFree(e->d_mesh_rgb); e->d_mesh_verts = nullptr; e->d_mesh_rgb = nullptr; e->mesh_capacity = 0;
+        VC_CUDA(e, cudaMalloc(&e->d_mesh_verts, total * 9 * sizeof(float)));
+        VC_CUDA(e, cudaMalloc(&e->d_mesh_rgb, total * 3 * sizeof(uint32_t)));
+        e->mesh_capacity = total;
+    }
+    *total_out = total;
+    return VC_OK;
+}
+
 int vc_mc_mesh(vc_engine* e, float threshold, uint64_t* n_triangles) {
     if (!e || !n_triangles) return VC_ERR_ARG;
     PhaseRange nvtx("MarchingCubes");
@@ -1777,22 +1809,79 @@ int vc_mc_mesh(vc_engine* e, float threshold, uint64_t* n_triangles) {
     unsigned long long* d_sums = (unsigned long long*)((char*)sc + counts_bytes);
     VcDense d{e->d_dense, e->g.X, e->g.Y, e->g.Z};
     vc_mc_count_kernel<<<(unsigned)((ncol + 127) / 128), 128, 0, e->stream>>>(d, threshold, d_counts);
-    vc_scan_block_kernel<<<nb, VC_SCAN_BLOCK, 0, e->stream>>>(d_counts, d_counts, d_sums, ncol);
-    vc_scan_sums_kernel<<<1, 1024, 0, e->stream>>>(d_sums, nb, d_sums + nb);
-    vc_scan_add_kernel<<<nb, VC_SCAN_BLOCK, 0, e->stream>>>(d_counts, d_sums, ncol);
-    VC_CUDA(e, cudaGetLastError());
     unsigned long long total = 0;
-    VC_CUDA(e, cudaMemcpyAsync(&total, d_sums + nb, sizeof total, cudaMemcpyDeviceToHost, e->stream));
-    VC_CUDA(e, cudaStreamSynchronize(e->stream));
-    if (total > 0xffffffffull) return fail(e, VC_ERR_CAPACITY, "vc_mc_mesh: %llu triangles exceed 32-bit offsets", total);
-    if (total > e->mesh_capacity) {  // triangle buffers are grow-only
-        cudaFree(e->d_mesh_verts); cudaFree(e->d_mesh_rgb); e->d_mesh_verts = nullptr; e->d_mesh_rgb = nullptr; e->mesh_capacity = 0;
-        VC_CUDA(e, cudaMalloc(&e->d_mesh_verts, total * 9 * sizeof(float)));
-        VC_CUDA(e, cudaMalloc(&e->d_mesh_rgb, total * 3 * sizeof(uint32_t)));
-        e->mesh_capacity = total;
-    }
+    rc = scan_mesh_counts(e, "vc_mc_mesh", d_counts, d_sums, ncol, nb, &total);
+    if (rc) return rc;
     if (total) {
         vc_mc_emit_kernel<<<(unsigned)((ncol + 127) / 128), 128, 0, e->stream>>>(d, threshold, d_counts, e->d_mesh_verts, e->d_mesh_rgb);
+        VC_CUDA(e, cudaGetLastError());
+    }
+    e->n_mesh_tris = total;
+    e->have_mesh = true;
+    *n_triangles = total;
+    return VC_OK;
+}
+
+int vc_mesh_from_volumes(vc_engine* e, int32_t apply_colors, int32_t handle_unseen, int32_t closure_k, float threshold, uint64_t* n_triangles) {
+    if (!e || !n_triangles) return VC_ERR_ARG;
+    PhaseRange nvtx("MarchingCubes");
+    if (closure_k < 0 || closure_k > VC_MESH_MAX_CLOSURE || (closure_k != 0 && closure_k % 2 != 1))
+        return fail(e, VC_ERR_ARG, "vc_mesh_from_volumes: closure kernel size must be 0 (none) or odd in [1, %d], got %d", VC_MESH_MAX_CLOSURE, closure_k);
+    if (!e->whole_grid()) return fail(e, VC_ERR_STATE, "vc_mesh_from_volumes: meshing needs the whole grid on one engine");
+    if (apply_colors && !e->have_colors) return fail(e, VC_ERR_STATE, "vc_mesh_from_volumes: apply_colors needs a vc_color of the current volumes");
+    const long long ncol = (long long)(e->g.X + 1) * (e->g.Y + 1);
+    if (ncol > 0x7fffffffLL) return fail(e, VC_ERR_ARG, "vc_mesh_from_volumes: grid too large");
+    if (bind_device(e)) return VC_ERR_CUDA;
+    int rc = load_mc_tables(e);
+    if (rc) return rc;
+    rc = materialize_reset(e);
+    if (rc) return rc;
+    // alphas are 0 or 1: any other threshold puts every corner on one side (no triangles)
+    if (!(threshold > 0.f && threshold <= 1.f)) {
+        e->n_mesh_tris = 0;
+        e->have_mesh = true;
+        *n_triangles = 0;
+        return VC_OK;
+    }
+    const int s = closure_k > 0 ? (closure_k - 1) / 2 : 0;
+    const bool colors = apply_colors && e->n_surface > 0;
+    const long long n_rows = (long long)e->g.Y * e->g.Z;
+    const int nb = (int)((ncol + VC_SCAN_BLOCK - 1) / VC_SCAN_BLOCK);
+    // scratch: column counts | scan block sums | record row offsets (colours) | dilated occupancy (closure)
+    const size_t counts_bytes = ((size_t)ncol * 4 + 15) / 16 * 16;
+    const size_t sums_bytes = (((size_t)nb + 1) * sizeof(unsigned long long) + 15) / 16 * 16;
+    const size_t rows_bytes = colors ? ((size_t)(n_rows + 1) * 4 + 15) / 16 * 16 : 0;
+    const size_t dil_bytes = s > 0 ? (size_t)e->slab_words * 4 : 0;
+    void* sc = nullptr;
+    rc = ensure_scratch(e, counts_bytes + sums_bytes + rows_bytes + dil_bytes, &sc);
+    if (rc) return rc;
+    uint32_t* d_counts = (uint32_t*)sc;
+    unsigned long long* d_sums = (unsigned long long*)((char*)sc + counts_bytes);
+    uint32_t* d_rows = (uint32_t*)((char*)sc + counts_bytes + sums_bytes);
+    uint32_t* d_dil = (uint32_t*)((char*)sc + counts_bytes + sums_bytes + rows_bytes);
+    VcMeshSrc m{};
+    m.occ = e->occ_slab(); m.seen = e->seen_slab();
+    m.X = e->g.X; m.Y = e->g.Y; m.Z = e->g.Z; m.Wx = e->Wx;
+    m.unseen = handle_unseen ? 1 : 0;
+    m.s = s;
+    if (colors) {
+        m.rec_idx = e->d_color_idx; m.rec_rgbn = e->d_color_rgbn; m.row_start = d_rows;
+        vc_record_rows_kernel<<<(unsigned)((n_rows + 1 + 255) / 256), 256, 0, e->stream>>>(e->d_color_idx, (uint32_t)e->n_surface, e->g.X, n_rows, d_rows);
+    }
+    if (s > 0) {
+        int zchunk = 64;  // planes per thread (each chunk re-reads 2s planes of its neighbours)
+        while ((long long)e->g.Y * e->Wx * ((e->g.Z + zchunk - 1) / zchunk) > 0x7fffffffLL) zchunk *= 2;
+        const long long n_threads = (long long)e->g.Y * e->Wx * ((e->g.Z + zchunk - 1) / zchunk);
+        vc_dilate_kernel<<<(unsigned)((n_threads + 255) / 256), 256, 0, e->stream>>>(m, zchunk, d_dil);
+        m.dil = d_dil;
+    }
+    vc_mesh_count_kernel<<<(unsigned)((ncol + 255) / 256), 256, 0, e->stream>>>(m, d_counts);
+    unsigned long long total = 0;
+    rc = scan_mesh_counts(e, "vc_mesh_from_volumes", d_counts, d_sums, ncol, nb, &total);
+    if (rc) return rc;
+    if (total) {
+        vc_mesh_emit_kernel<<<(unsigned)((ncol + 127) / 128), 128, 0, e->stream>>>(m, d_counts, e->d_mesh_verts);
+        vc_mesh_color_kernel<<<(unsigned)((total + 255) / 256), 256, 0, e->stream>>>(m, e->d_mesh_verts, total, e->d_mesh_rgb);
         VC_CUDA(e, cudaGetLastError());
     }
     e->n_mesh_tris = total;

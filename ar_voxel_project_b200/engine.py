@@ -413,9 +413,22 @@ class VoxelEngine:
         """-> (verts float32[T,3,3] in voxel-index coordinates, rgb uint32[T,3]) in the reference's emission order"""
         n = C.c_uint64()
         self._check(self._lib.vc_mc_mesh(self._h, C.c_float(threshold), C.byref(n)))
-        verts = np.empty((n.value, 3, 3), np.float32)
-        rgb = np.empty((n.value, 3), np.uint32)
-        self._check(self._lib.vc_download_mesh(self._h, C.c_void_p(verts.ctypes.data), C.c_void_p(rgb.ctypes.data), n.value))
+        return self.download_mesh(n.value)
+
+    def mesh_from_volumes(self, apply_colors=False, handle_unseen=False, closure_k=0, threshold=0.5, download=True):
+        """marchingCubes of the Model dense_from_volumes(apply_colors, handle_unseen) [+ dense_closure(closure_k)] would build,
+        from the bit volumes and colour records without the dense Model (closure_k = 0: no closure).  Same (verts, rgb) as
+        that chain + mc_mesh(threshold); download=False leaves the mesh on the device and returns its triangle count."""
+        n = C.c_uint64()
+        self._check(self._lib.vc_mesh_from_volumes(self._h, int(bool(apply_colors)), int(bool(handle_unseen)), int(closure_k),
+                                                    C.c_float(threshold), C.byref(n)))
+        return self.download_mesh(n.value) if download else int(n.value)
+
+    def download_mesh(self, n_triangles):
+        """the mesh the last mc_mesh / mesh_from_volumes left on the device: (verts float32[T,3,3], rgb uint32[T,3])"""
+        verts = np.empty((n_triangles, 3, 3), np.float32)
+        rgb = np.empty((n_triangles, 3), np.uint32)
+        self._check(self._lib.vc_download_mesh(self._h, C.c_void_p(verts.ctypes.data), C.c_void_p(rgb.ctypes.data), n_triangles))
         return verts, rgb
 
     def stats(self):

@@ -283,6 +283,20 @@ VC_EXPORT int vc_dense_download(vc_engine* e, float* rgba);
 VC_EXPORT int vc_mc_mesh(vc_engine* e, float threshold, uint64_t* n_triangles);
 VC_EXPORT int vc_download_mesh(vc_engine* e, float* verts /* T*9 */, uint32_t* rgb /* T*3 */, uint64_t capacity_triangles);
 
+/* ---- the mesh straight from the bit volumes (main.cpp:291-303 without the dense Model) ---- */
+/* marchingCubes of the Model that vc_dense_from_volumes(apply_colors, handle_unseen) [+ vc_dense_closure(closure_k)] would build,
+ * computed from the bit volumes and the colour records without the dense Model: the same triangles, vertices and colours in the
+ * same order as that chain + vc_mc_mesh(threshold), left in the mesh buffers for vc_download_mesh.  closure_k = 0: no closure;
+ * otherwise odd, at most VC_MESH_MAX_CLOSURE (else VC_ERR_ARG).  Every alpha of such a Model is 0 or 1, so the geometry is marching
+ * cubes on occupied | ~seen (handle_unseen) dilated by the closure box, and every vertex sits on a voxel; a threshold outside
+ * (0, 1] gives no triangles.  Memory: one extra bit volume (closure only), a row table of the colour records (4 (Y*Z+1) bytes),
+ * 4 (X+1)(Y+1) bytes of column counts and the mesh; the dense Model is not allocated or touched.
+ * VC_ERR_STATE: a slab engine (whole grid only), or apply_colors without a vc_color of the current volumes.
+ * VC_ERR_CAPACITY: 2^32 triangles or more.  A refused call leaves the previous mesh as it was. */
+#define VC_MESH_MAX_CLOSURE 15
+VC_EXPORT int vc_mesh_from_volumes(vc_engine* e, int32_t apply_colors, int32_t handle_unseen, int32_t closure_k, float threshold,
+                                   uint64_t* n_triangles);
+
 /* ---- measurement helper (bench.py roofline denominators) ------------------------- */
 /* Register-resident FFMA and DFMA loops on `device`: measured CUDA-core peaks in TFLOP/s
  * (2 flops per FMA), timed with CUDA events, best of 5. Not part of the carve path. */

@@ -153,6 +153,17 @@ class Engine {
         check(vc_download_mesh(h_, verts.data(), rgb.data(), n));
         return n;
     }
+    // marchingCubes of the Model denseFromVolumes(applyColors, handleUnseen) [+ denseClosure(closureK)] would build, from the bit
+    // volumes and colour records without the dense Model (closureK = 0: no closure); same triangles as that chain + mcMesh
+    uint64_t meshFromVolumes(bool applyColors, bool handleUnseen, int closureK, float threshold, std::vector<float>& verts,
+                             std::vector<uint32_t>& rgb) {
+        uint64_t n = 0;
+        check(vc_mesh_from_volumes(h_, applyColors ? 1 : 0, handleUnseen ? 1 : 0, closureK, threshold, &n));
+        verts.resize(n * 9);
+        rgb.resize(n * 3);
+        check(vc_download_mesh(h_, verts.data(), rgb.data(), n));
+        return n;
+    }
     // multi-GPU plumbing: balanced z-slabs, one-plane halos, NCCL collectives inside the library (voxcarve.h)
     std::vector<int32_t> planSlabs(int n_parts) { std::vector<int32_t> b((size_t)n_parts + 1); check(vc_plan_slabs(h_, n_parts, b.data())); return b; }
     void setSlab(int z_begin, int z_end) { check(vc_set_slab(h_, z_begin, z_end)); check(vc_slab_words(h_, &words_)); }
@@ -476,6 +487,28 @@ bool marchingCubes(ModelT* model, float scale = 1.0f, const float* translation =
         return false;
     }
     std::cout << "LOG - MC: Mesh written, marchingCubes completed." << std::endl;
+    return true;
+}
+
+// main.cpp:260-303 from a ViewCache to the .off file, without a host Model: carve -> [reconstructClosestColor (colorMode 1) /
+// reconstructAvgColor (2)] -> handleUnseen -> [applyClosure(closureK), closureK = 0: none] -> marchingCubes(scale, translation,
+// threshold).  The volumes, colour records and mesh stay on the device until the triangles are downloaded, so grids whose dense
+// Model does not fit the GPU (2048^3: 128 GiB) are meshed too.  Returns false if the file cannot be written.
+inline bool carveToMesh(const ViewCache& views, int X, int Y, int Z, float size, int colorMode, int closureK, float scale = 1.0f,
+                        const float* translation = nullptr, float threshold = 0.5f, const std::string& outFileName = "out/mesh.off",
+                        int device = 0) {
+    Engine e(X, Y, Z, size, 0, -1, device);
+    e.setViews(views, colorMode != 0);
+    e.carve();
+    if (colorMode) e.color(colorMode);
+    std::vector<float> verts;
+    std::vector<uint32_t> rgb;
+    const uint64_t nt = e.meshFromVolumes(colorMode != 0, true, closureK, threshold, verts, rgb);
+    const float tx = translation ? translation[0] : 0.f, ty = translation ? translation[1] : 0.f, tz = translation ? translation[2] : 0.f;
+    if (!detail::writeOff(outFileName, nt, verts, rgb, scale * size, tx, ty, tz)) {
+        std::cout << "ERR - MC: unable to write output file!" << std::endl;
+        return false;
+    }
     return true;
 }
 
