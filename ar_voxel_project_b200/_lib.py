@@ -90,6 +90,9 @@ SIGNATURES = {
     "vc_mc_mesh": (C.c_int, [_P, C.c_float, C.POINTER(C.c_uint64)]),
     "vc_download_mesh": (C.c_int, [_P, _P, _P, C.c_uint64]),
     "vc_mesh_from_volumes": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.POINTER(C.c_uint64)]),
+    "vc_mesh_format_off": (C.c_int, [_P, C.c_float, C.c_float, C.c_float, C.c_float, C.POINTER(C.c_uint64)]),
+    "vc_download_mesh_off": (C.c_int, [_P, C.c_uint64, _P, C.c_uint64]),
+    "vc_format_g": (C.c_int, [C.c_int32, C.c_uint64, _P, _P, C.c_uint64, C.POINTER(C.c_uint64)]),
     "vc_selftest": (C.c_int, [C.c_int32, C.c_int32, C.c_uint64, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "vc_measure_peaks": (C.c_int, [C.c_int32, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
 }

@@ -133,6 +133,11 @@ struct vc_engine {
     uint32_t* d_mesh_rgb = nullptr;
     unsigned long long n_mesh_tris = 0, mesh_capacity = 0;
     bool have_dense = false, have_mesh = false;
+    unsigned long long mesh_version = 0;  // bumped whenever the mesh buffers are rewritten or freed
+    // .off text of the mesh (vc_mesh_format_off), grow-only; valid while mesh_version == text_version
+    char* d_text = nullptr;
+    unsigned long long text_capacity = 0, text_bytes = 0, text_version = 0;
+    bool have_text = false;
     bool have_calib = false;
     double calib_K[9] = {0}, calib_dist[8] = {0};
     vc_stats stats{};
@@ -541,7 +546,7 @@ void vc_destroy(vc_engine* e) {
     cudaFree(e->d_sat); cudaFree(e->d_sat_tmp); cudaFree(e->d_bgr_tmp); cudaFree(e->d_bricks); cudaFree(e->d_super); cudaFree(e->d_brick_flags); cudaFree(e->d_super_flags); cudaFree(e->d_super_list);
     cudaFree(e->d_block_sums);
     cudaFree(e->d_scalars); cudaFree(e->d_hist); cudaFree(e->d_filt); cudaFree(e->d_view64);
-    cudaFree(e->d_dense); cudaFree(e->d_dense_tmp); cudaFree(e->d_mesh_verts); cudaFree(e->d_mesh_rgb);
+    cudaFree(e->d_dense); cudaFree(e->d_dense_tmp); cudaFree(e->d_mesh_verts); cudaFree(e->d_mesh_rgb); cudaFree(e->d_text);
     cudaFree(e->d_sparse_idx); cudaFree(e->d_sparse_words);
     cudaFree(e->d_scratch); cudaFree(e->d_undist_ir); vol_free(e->d_occ_full_own); vol_free(e->d_seen_full_own); cudaFree(e->d_reduce);
     if (e->comm) vc_comm_destroy(e);
@@ -1784,6 +1789,7 @@ static int scan_mesh_counts(vc_engine* e, const char* who, uint32_t* d_counts, u
     if (total > 0xffffffffull) return fail(e, VC_ERR_CAPACITY, "%s: %llu triangles exceed 32-bit offsets", who, total);
     if (total > e->mesh_capacity) {  // triangle buffers are grow-only
         e->have_mesh = false;
+        e->mesh_version++;
         cudaFree(e->d_mesh_verts); cudaFree(e->d_mesh_rgb); e->d_mesh_verts = nullptr; e->d_mesh_rgb = nullptr; e->mesh_capacity = 0;
         VC_CUDA(e, cudaMalloc(&e->d_mesh_verts, total * 9 * sizeof(float)));
         VC_CUDA(e, cudaMalloc(&e->d_mesh_rgb, total * 3 * sizeof(uint32_t)));
@@ -1818,6 +1824,7 @@ int vc_mc_mesh(vc_engine* e, float threshold, uint64_t* n_triangles) {
     }
     e->n_mesh_tris = total;
     e->have_mesh = true;
+    e->mesh_version++;
     *n_triangles = total;
     return VC_OK;
 }
@@ -1840,6 +1847,7 @@ int vc_mesh_from_volumes(vc_engine* e, int32_t apply_colors, int32_t handle_unse
     if (!(threshold > 0.f && threshold <= 1.f)) {
         e->n_mesh_tris = 0;
         e->have_mesh = true;
+        e->mesh_version++;
         *n_triangles = 0;
         return VC_OK;
     }
@@ -1886,6 +1894,7 @@ int vc_mesh_from_volumes(vc_engine* e, int32_t apply_colors, int32_t handle_unse
     }
     e->n_mesh_tris = total;
     e->have_mesh = true;
+    e->mesh_version++;
     *n_triangles = total;
     return VC_OK;
 }
@@ -1900,6 +1909,119 @@ int vc_download_mesh(vc_engine* e, float* verts, uint32_t* rgb, uint64_t capacit
     VC_CUDA(e, cudaMemcpyAsync(verts, e->d_mesh_verts, e->n_mesh_tris * 9 * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
     VC_CUDA(e, cudaMemcpyAsync(rgb, e->d_mesh_rgb, e->n_mesh_tris * 3 * sizeof(uint32_t), cudaMemcpyDeviceToHost, e->stream));
     VC_CUDA(e, cudaStreamSynchronize(e->stream));
+    return VC_OK;
+}
+
+// Length pass and scan of a text's s.n_lines (>= 1) lines: d_lens (n_lines u32) becomes the lines' offsets inside their scan
+// block, d_sums (nb + 1 u64) the blocks' offsets with the total at [nb].  Ends in a synchronisation of `st`.
+static cudaError_t text_scan(const VcTextSrc& s, uint32_t* d_lens, unsigned long long* d_sums, cudaStream_t st, unsigned long long* total) {
+    const int nb = (int)((s.n_lines + VC_SCAN_BLOCK - 1) / VC_SCAN_BLOCK);
+    vc_text_len_kernel<<<(unsigned)((s.n_lines + 255) / 256), 256, 0, st>>>(s, d_lens);
+    vc_scan_block_kernel<<<nb, VC_SCAN_BLOCK, 0, st>>>(d_lens, d_lens, d_sums, (long long)s.n_lines);
+    vc_scan_sums_kernel<<<1, 1024, 0, st>>>(d_sums, nb, d_sums + nb);
+    cudaError_t r = cudaGetLastError();
+    if (r == cudaSuccess) r = cudaMemcpyAsync(total, d_sums + nb, sizeof *total, cudaMemcpyDeviceToHost, st);
+    if (r == cudaSuccess) r = cudaStreamSynchronize(st);
+    return r;
+}
+// the lines themselves, at byte `base` of d_text onwards (after text_scan on the same buffers)
+static cudaError_t text_emit(const VcTextSrc& s, const uint32_t* d_offs, const unsigned long long* d_sums, unsigned long long base, char* d_text,
+                             cudaStream_t st) {
+    const int nb = (int)((s.n_lines + VC_SCAN_BLOCK - 1) / VC_SCAN_BLOCK);
+    cudaError_t r = cudaFuncSetAttribute(vc_text_emit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, VC_TEXT_SMEM);
+    if (r != cudaSuccess) return r;
+    vc_text_emit_kernel<<<nb, VC_SCAN_BLOCK, VC_TEXT_SMEM, st>>>(s, d_offs, d_sums, base, d_text);
+    return cudaGetLastError();
+}
+
+int vc_mesh_format_off(vc_engine* e, float scale, float tx, float ty, float tz, uint64_t* n_bytes) {
+    if (!e || !n_bytes) return VC_ERR_ARG;
+    if (!e->have_mesh) return fail(e, VC_ERR_STATE, "vc_mesh_format_off: no mesh on the device (vc_mc_mesh / vc_mesh_from_volumes first)");
+    const unsigned long long T = e->n_mesh_tris, L = 4 * T;
+    if (L > VC_TEXT_MAX_LINES)
+        return fail(e, VC_ERR_CAPACITY, "vc_mesh_format_off: %llu triangles make %llu lines, more than the %llu one text takes", T, L, VC_TEXT_MAX_LINES);
+    if (bind_device(e)) return VC_ERR_CUDA;
+    PhaseRange nvtx("WriteMesh");
+    char hdr[64];
+    const int hl = snprintf(hdr, sizeof hdr, "OFF\n%llu %llu 0\n", 3 * T, T);
+    const VcTextSrc src{nullptr, e->d_mesh_verts, e->d_mesh_rgb, T, L, scale, {tx, ty, tz}};
+    const int nb = (int)((L + VC_SCAN_BLOCK - 1) / VC_SCAN_BLOCK);
+    const size_t lens_bytes = ((size_t)L * 4 + 15) / 16 * 16;
+    unsigned long long body = 0;
+    uint32_t* d_lens = nullptr;
+    unsigned long long* d_sums = nullptr;
+    if (L) {
+        void* sc = nullptr;
+        int rc = ensure_scratch(e, lens_bytes + ((size_t)nb + 1) * sizeof(unsigned long long), &sc);
+        if (rc) return rc;
+        d_lens = (uint32_t*)sc;
+        d_sums = (unsigned long long*)((char*)sc + lens_bytes);
+        VC_CUDA(e, text_scan(src, d_lens, d_sums, e->stream, &body));
+    }
+    const unsigned long long total = hl + body;
+    if (total > e->text_capacity) {  // grow-only; the previous text stays until the new buffer exists
+        char* t = nullptr;
+        VC_CUDA(e, cudaMalloc(&t, total));
+        cudaFree(e->d_text);
+        e->d_text = t;
+        e->text_capacity = total;
+    }
+    e->have_text = false;
+    VC_CUDA(e, cudaMemcpyAsync(e->d_text, hdr, hl, cudaMemcpyHostToDevice, e->stream));
+    if (L) VC_CUDA(e, text_emit(src, d_lens, d_sums, hl, e->d_text, e->stream));
+    VC_CUDA(e, cudaStreamSynchronize(e->stream));
+    e->text_bytes = total;
+    e->text_version = e->mesh_version;
+    e->have_text = true;
+    *n_bytes = total;
+    return VC_OK;
+}
+
+int vc_download_mesh_off(vc_engine* e, uint64_t offset, void* dst, uint64_t n_bytes) {
+    if (!e) return VC_ERR_ARG;
+    if (!e->have_text) return fail(e, VC_ERR_STATE, "vc_download_mesh_off: no text formatted (vc_mesh_format_off first)");
+    if (e->text_version != e->mesh_version) return fail(e, VC_ERR_STATE, "vc_download_mesh_off: the mesh changed since its text was formatted");
+    if (offset > e->text_bytes || n_bytes > e->text_bytes - offset)
+        return fail(e, VC_ERR_ARG, "vc_download_mesh_off: bytes [%llu, %llu + %llu) lie past the end of the %llu-byte text", (unsigned long long)offset,
+                    (unsigned long long)offset, (unsigned long long)n_bytes, e->text_bytes);
+    if (n_bytes == 0) return VC_OK;
+    if (!dst) return fail(e, VC_ERR_ARG, "vc_download_mesh_off: null buffer");
+    if (bind_device(e)) return VC_ERR_CUDA;
+    VC_CUDA(e, cudaMemcpyAsync(dst, e->d_text + offset, n_bytes, cudaMemcpyDeviceToHost, e->stream));
+    VC_CUDA(e, cudaStreamSynchronize(e->stream));
+    return VC_OK;
+}
+
+int vc_format_g(int32_t device, uint64_t n, const float* values, char* text, uint64_t capacity, uint64_t* n_bytes) {
+    if (!n_bytes || (n && !values)) return fail(nullptr, VC_ERR_ARG, "vc_format_g: null argument");
+    if (n > VC_TEXT_MAX_LINES) return fail(nullptr, VC_ERR_CAPACITY, "vc_format_g: %llu values, more than the %llu lines one text takes", (unsigned long long)n, VC_TEXT_MAX_LINES);
+    *n_bytes = 0;
+    if (n == 0) return VC_OK;
+    if (cudaSetDevice(device) != cudaSuccess) { cudaGetLastError(); return fail(nullptr, VC_ERR_CUDA, "vc_format_g: no CUDA device %d; this engine has no CPU fallback", device); }
+    const int nb = (int)((n + VC_SCAN_BLOCK - 1) / VC_SCAN_BLOCK);
+    float* d_values = nullptr;
+    uint32_t* d_lens = nullptr;
+    unsigned long long* d_sums = nullptr;
+    char* d_text = nullptr;
+    unsigned long long total = 0;
+    bool room = false;
+    cudaError_t s = cudaMalloc(&d_values, n * sizeof(float));
+    if (s == cudaSuccess) s = cudaMalloc(&d_lens, n * sizeof(uint32_t));
+    if (s == cudaSuccess) s = cudaMalloc(&d_sums, ((size_t)nb + 1) * sizeof(unsigned long long));
+    if (s == cudaSuccess) s = cudaMemcpy(d_values, values, n * sizeof(float), cudaMemcpyHostToDevice);
+    const VcTextSrc src{d_values, nullptr, nullptr, 0, n, 1.f, {0.f, 0.f, 0.f}};
+    if (s == cudaSuccess) s = text_scan(src, d_lens, d_sums, 0, &total);
+    if (s == cudaSuccess) {
+        *n_bytes = total;
+        room = total <= capacity && text;
+    }
+    if (s == cudaSuccess && room) s = cudaMalloc(&d_text, total);
+    if (s == cudaSuccess && room) s = text_emit(src, d_lens, d_sums, 0, d_text, 0);
+    if (s == cudaSuccess && room) s = cudaMemcpy(text, d_text, total, cudaMemcpyDeviceToHost);
+    cudaFree(d_values); cudaFree(d_lens); cudaFree(d_sums); cudaFree(d_text);
+    if (s != cudaSuccess) return fail(nullptr, VC_ERR_CUDA, "vc_format_g: %s", cudaGetErrorString(s));
+    if (!room) return fail(nullptr, total > capacity ? VC_ERR_CAPACITY : VC_ERR_ARG, "vc_format_g: the text has %llu bytes, the buffer %llu", total,
+                           text ? (unsigned long long)capacity : 0ull);
     return VC_OK;
 }
 

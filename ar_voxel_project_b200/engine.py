@@ -431,6 +431,35 @@ class VoxelEngine:
         self._check(self._lib.vc_download_mesh(self._h, C.c_void_p(verts.ctypes.data), C.c_void_p(rgb.ctypes.data), n_triangles))
         return verts, rgb
 
+    def format_off(self, scale=1.0, translation=(0.0, 0.0, 0.0)):
+        """format the .off text of the mesh on the device (SimpleMesh::WriteMesh, vertex = index coordinates * scale + translation
+        in f32) and keep it there; -> its size in bytes"""
+        n = C.c_uint64()
+        tx, ty, tz = (C.c_float(t) for t in translation)
+        self._check(self._lib.vc_mesh_format_off(self._h, C.c_float(scale), tx, ty, tz, C.byref(n)))
+        return int(n.value)
+
+    def download_mesh_off(self, offset, n_bytes):
+        """bytes [offset, offset + n_bytes) of the text format_off left on the device"""
+        out = np.empty(int(n_bytes), np.uint8)
+        self._check(self._lib.vc_download_mesh_off(self._h, int(offset), C.c_void_p(out.ctypes.data), int(n_bytes)))
+        return out.tobytes()
+
+    def mesh_off(self, scale=1.0, translation=(0.0, 0.0, 0.0)):
+        """the whole .off file of the mesh the last mc_mesh / mesh_from_volumes left on the device, formatted on the device"""
+        return self.download_mesh_off(0, self.format_off(scale, translation))
+
+    def write_mesh_off(self, path, scale=1.0, translation=(0.0, 0.0, 0.0), chunk=64 << 20):
+        """mesh_off written to `path`, downloaded in chunks of `chunk` bytes through one buffer"""
+        n = self.format_off(scale, translation)
+        buf = np.empty(min(n, int(chunk)), np.uint8)
+        with open(path, "wb") as f:
+            for o in range(0, n, len(buf)):
+                k = min(len(buf), n - o)
+                self._check(self._lib.vc_download_mesh_off(self._h, o, C.c_void_p(buf.ctypes.data), k))
+                f.write(memoryview(buf)[:k])
+        return n
+
     def stats(self):
         s = L.Stats()
         self._check(self._lib.vc_get_stats(self._h, C.byref(s)))
@@ -484,6 +513,18 @@ def selftest(which, n, seed=0, device=0):
     if rc != L.VC_OK:
         raise VoxCarveError(rc, lib.vc_last_error(None).decode())
     return a.value, b.value
+
+
+def format_g(values, device=0):
+    """printf("%g\\n") of every float32 of `values`, formatted on the GPU with the code of VoxelEngine.format_off -> bytes"""
+    lib = L.load()
+    v = np.ascontiguousarray(values, np.float32).reshape(-1)
+    need = C.c_uint64()
+    text = np.empty(13 * len(v), np.uint8)  # at most 12 characters and a newline per value
+    rc = lib.vc_format_g(int(device), len(v), C.c_void_p(v.ctypes.data), C.c_void_p(text.ctypes.data), len(text), C.byref(need))
+    if rc != L.VC_OK:
+        raise VoxCarveError(rc, lib.vc_last_error(None).decode())
+    return text[:need.value].tobytes()
 
 
 def undistort_bgr(images_bgr, K, dist, device=0):

@@ -297,6 +297,26 @@ VC_EXPORT int vc_download_mesh(vc_engine* e, float* verts /* T*9 */, uint32_t* r
 VC_EXPORT int vc_mesh_from_volumes(vc_engine* e, int32_t apply_colors, int32_t handle_unseen, int32_t closure_k, float threshold,
                                    uint64_t* n_triangles);
 
+/* ---- the .off file of the mesh, formatted on the device (SimpleMesh::WriteMesh, MarchingCubes.h:59-87) ---- */
+/* The complete text of the file WriteMesh writes for the mesh the last vc_mc_mesh / vc_mesh_from_volumes left on the device:
+ * "OFF\n", "3T T 0\n", 3T vertex lines "a b c\n" with a = fl(fl(x * scale) + tx) (no FMA, x86 NaN rules: a NaN operand keeps
+ * its sign, 0 * inf and inf - inf give -nan), then T face lines "3 3i 3i+1 3i+2 r g b\n" (rgb printed with %u).  Numbers are
+ * printed as a C++ ostream prints a float by default: printf("%g") of the float, 6 significant digits rounded correctly
+ * (ties to even) from the exact binary value, "C" locale; denormals, -0, inf, -inf, nan and -nan included.  scale multiplies
+ * the voxel-index coordinates of the mesh: the reference's scaleFactor = scale * voxel size (MarchingCubes.cpp:23).
+ * The text stays in a grow-only device buffer (n_bytes = its size, at most 39 bytes per vertex line and 71 per face line)
+ * until the next call; vc_download_mesh_off copies any byte range of it into HOST memory, so a caller can write the file
+ * in chunks.  Refusals leave the previous text as it was: VC_ERR_STATE without a mesh; VC_ERR_CAPACITY above
+ * VC_TEXT_MAX_LINES lines (4T lines: T > 2^29 triangles).  vc_download_mesh_off: VC_ERR_STATE when no text was formatted or
+ * the mesh has changed since; VC_ERR_ARG for a range that ends past the text. */
+#define VC_TEXT_MAX_LINES (1ull << 31) /* what one scan of u32 line lengths takes */
+VC_EXPORT int vc_mesh_format_off(vc_engine* e, float scale, float tx, float ty, float tz, uint64_t* n_bytes);
+VC_EXPORT int vc_download_mesh_off(vc_engine* e, uint64_t offset, void* dst, uint64_t n_bytes);
+/* Utility (HOST in / HOST out, on `device`): one line "%g\n" per value, with the device code of vc_mesh_format_off and no
+ * arithmetic on the values.  *n_bytes = the text's size; VC_ERR_CAPACITY (nothing written) when it exceeds `capacity`;
+ * at most VC_TEXT_MAX_LINES values. */
+VC_EXPORT int vc_format_g(int32_t device, uint64_t n, const float* values, char* text, uint64_t capacity, uint64_t* n_bytes);
+
 /* ---- measurement helper (bench.py roofline denominators) ------------------------- */
 /* Register-resident FFMA and DFMA loops on `device`: measured CUDA-core peaks in TFLOP/s
  * (2 flops per FMA), timed with CUDA events, best of 5. Not part of the carve path. */
