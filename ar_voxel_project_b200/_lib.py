@@ -13,6 +13,7 @@ VC_OK, VC_ERR_ARG, VC_ERR_CUDA, VC_ERR_STATE, VC_ERR_CAPACITY, VC_ERR_COMM = 0, 
 VC_EXACT, VC_FAST_F32, VC_EXACT_FLAT = 0, 1, 2
 VC_COLOR_CLOSEST, VC_COLOR_AVG = 1, 2
 VC_MASK_BITS, VC_MASK_BGR8, VC_MASK_BGR8_RAW = 0, 1, 2
+VC_MAX_TOTAL_VIEWS = 4096
 
 
 class GridDesc(C.Structure):
@@ -39,6 +40,7 @@ SIGNATURES = {
     "vc_synchronize": (C.c_int, [_P]),
     "vc_set_profiling": (C.c_int, [_P, C.c_int32]),
     "vc_set_views": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
+    "vc_append_views": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int32, _P]),
     "vc_set_masks": (C.c_int, [_P, _P, C.c_int32]),
     "vc_set_images": (C.c_int, [_P, _P]),
     "vc_set_calibration": (C.c_int, [_P, _P, _P, C.c_int32]),

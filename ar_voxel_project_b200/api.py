@@ -49,16 +49,23 @@ class ViewSet:
 
 
 def _engine_for(model, views, device=0, need_images=False):
+    """an engine holding all views: vc_set_views takes the first 256, vc_append_views the rest"""
+    if need_images and views.images_bgr is None:
+        raise ValueError("colour reconstruction needs the undistorted images")
     e = VoxelEngine(model.getX(), model.getY(), model.getZ(), model.getSize(), device=device)
-    e.set_views(views.P, views.W, views.H, views.M)
+    k = min(views.V, 256)
+    e.set_views(views.P[:k], views.W, views.H, None if views.M is None else views.M[:k])
     if views.mask_bits is not None:
-        e.set_masks_bits(views.mask_bits)
+        e.set_masks_bits(views.mask_bits[:k])
     else:
-        e.set_masks_bgr(views.mask_bgr)
+        e.set_masks_bgr(views.mask_bgr[:k])
     if need_images:
-        if views.images_bgr is None:
-            raise ValueError("colour reconstruction needs the undistorted images")
-        e.set_images(views.images_bgr)
+        e.set_images(views.images_bgr[:k])
+    if views.V > k:
+        e.append_views(views.P[k:], None if views.M is None else views.M[k:],
+                       mask_bits=None if views.mask_bits is None else views.mask_bits[k:],
+                       mask_bgr=None if views.mask_bits is not None else views.mask_bgr[k:],
+                       images_bgr=views.images_bgr[k:] if need_images else None)
     return e
 
 

@@ -28,9 +28,9 @@ namespace {
 
 std::string g_create_error;
 std::mutex g_const_mutex;
-// which (engine uid, views version) currently owns c_view / c_cam on each device
+// which (engine uid, views version, view group) currently owns c_view / c_cam on each device
 // and an event recorded after the owner's last launch that reads them: a new owner waits for it before overwriting the symbols
-struct ConstOwner { unsigned long long uid = 0, version = 0; cudaEvent_t last_use = nullptr; bool used = false; };
+struct ConstOwner { unsigned long long uid = 0, version = 0; int group = 0; cudaEvent_t last_use = nullptr; bool used = false; };
 ConstOwner g_const_owner[64];
 unsigned long long g_next_uid = 1;
 
@@ -91,6 +91,7 @@ struct vc_engine {
     uint32_t* d_mask = nullptr;
     VcViewFilter* d_filt = nullptr;      // global copy of c_filt for lane-divergent reads (sub-brick classification)
     VcViewConst* d_view64 = nullptr;     // global copy of c_view for lane-divergent reads (deferred exact evaluations)
+    float4* d_cam = nullptr;             // camera translations of all V views when V > VC_MAX_VIEWS (the colour pass over every group)
     vc_sat_t* d_sat = nullptr;           // summed-area tables of the background bits modulo 2^16, V x (H+1) x (W+1)
     uint32_t* d_sat_tmp = nullptr;       // V x H x Ww word-column prefixes used while building d_sat
     uint8_t* d_bgr_tmp = nullptr;        // staging for 8UC3 masks (grow-only)
@@ -333,22 +334,30 @@ static void vol_free(uint32_t* p) {
     cudaFree(p);
 }
 
-// upload this engine's view constants if another engine (or an older version) owns them
-int ensure_constants(vc_engine* e) {
+// Views come in groups of VC_MAX_VIEWS consecutive views, group g = views [g * VC_MAX_VIEWS, (g + 1) * VC_MAX_VIEWS); the
+// constant tables hold one group at a time.  An engine with at most VC_MAX_VIEWS views has one group and uploads it once.
+int n_groups(const vc_engine* e) { return (e->V + VC_MAX_VIEWS - 1) / VC_MAX_VIEWS; }
+
+// upload view group `group` of this engine to the constant tables if another engine (or another version or group) owns them
+int ensure_constants(vc_engine* e, int group = 0) {
     std::lock_guard<std::mutex> lk(g_const_mutex);
     ConstOwner& o = g_const_owner[e->g.device & 63];
-    if (o.uid == e->uid && o.version == e->views_version) return VC_OK;
+    if (o.uid == e->uid && o.version == e->views_version && o.group == group) return VC_OK;
     // c_view / c_cam / c_filt are per-device symbols shared by every engine on this GPU: kernels of the previous owner (another
-    // engine, or this one with older views) may still be reading them on another stream
-    if (o.used && o.last_use) VC_CUDA(e, cudaEventSynchronize(o.last_use));
+    // engine, or this one with older views) may still be reading them on another stream.  This engine's own kernels of another
+    // group run on e->stream, ahead of the copies below, so switching groups inside one call needs no host synchronisation.
+    if (o.used && o.last_use && (o.uid != e->uid || e->V <= VC_MAX_VIEWS)) VC_CUDA(e, cudaEventSynchronize(o.last_use));
     o.used = false;
-    VC_CUDA(e, cudaMemcpyToSymbolAsync(c_view, e->h_view.data(), sizeof(VcViewConst) * e->V, 0, cudaMemcpyHostToDevice, e->stream));
-    VC_CUDA(e, cudaMemcpyToSymbolAsync(c_cam, e->h_cam.data(), sizeof(float) * 4 * e->V, 0, cudaMemcpyHostToDevice, e->stream));
-    VC_CUDA(e, cudaMemcpyToSymbolAsync(c_filt, e->h_filt.data(), sizeof(VcViewFilter) * e->V, 0, cudaMemcpyHostToDevice, e->stream));
-    // the host vectors may change right after this call returns; make the copy complete first
-    VC_CUDA(e, cudaStreamSynchronize(e->stream));
+    const int v0 = group * VC_MAX_VIEWS, nv = std::min(VC_MAX_VIEWS, e->V - v0);
+    VC_CUDA(e, cudaMemcpyToSymbolAsync(c_view, e->h_view.data() + v0, sizeof(VcViewConst) * nv, 0, cudaMemcpyHostToDevice, e->stream));
+    VC_CUDA(e, cudaMemcpyToSymbolAsync(c_cam, e->h_cam.data() + (size_t)v0 * 4, sizeof(float) * 4 * nv, 0, cudaMemcpyHostToDevice, e->stream));
+    VC_CUDA(e, cudaMemcpyToSymbolAsync(c_filt, e->h_filt.data() + v0, sizeof(VcViewFilter) * nv, 0, cudaMemcpyHostToDevice, e->stream));
+    // the host vectors may change right after this call returns; make the copy complete first.  (With several groups they
+    // cannot: vc_set_views and vc_append_views synchronise the stream before they touch them.)
+    if (e->V <= VC_MAX_VIEWS) VC_CUDA(e, cudaStreamSynchronize(e->stream));
     o.uid = e->uid;
     o.version = e->views_version;
+    o.group = group;
     return VC_OK;
 }
 
@@ -451,13 +460,13 @@ void free_color(vc_engine* e) {
 // every factor rounded up.  T_i bounds sum_k |P_ik w_k| over the WHOLE grid (any slab of it), w = (y s, x s, -z s, 1) as f32
 // products.  A view whose matrix is not finite, or so large that the f32 evaluation could overflow, gets Cu = Cv = +inf:
 // its voxel-views are then never "decided" and all go through the exact path.
-void vc_filter_constants(vc_engine* e) {
+void vc_filter_constants(vc_engine* e, VcViewFilter* filt, int n) {
     const double up = 1.0 + ldexp(1.0, -22);  // f32 rounding of the coordinate products, with room to spare
     const double s = (double)e->g.voxel_size;
     const double ax = (double)(e->g.X - 1) * s * up, ay = (double)(e->g.Y - 1) * s * up, az = (double)(e->g.Z - 1) * s * up;
     const double W3 = (double)e->W + 3.0, H3 = (double)e->H + 3.0;
-    for (int v = 0; v < e->V; v++) {
-        VcViewFilter& f = e->h_filt[v];
+    for (int v = 0; v < n; v++) {
+        VcViewFilter& f = filt[v];
         double eta[3];
         bool ok = true;
         for (int i = 0; i < 3; i++) {
@@ -545,7 +554,7 @@ void vc_destroy(vc_engine* e) {
     vol_free(e->d_occ_own); vol_free(e->d_seen_own); cudaFree(e->d_mask); cudaFree(e->d_images);
     cudaFree(e->d_sat); cudaFree(e->d_sat_tmp); cudaFree(e->d_bgr_tmp); cudaFree(e->d_bricks); cudaFree(e->d_super); cudaFree(e->d_brick_flags); cudaFree(e->d_super_flags); cudaFree(e->d_super_list);
     cudaFree(e->d_block_sums);
-    cudaFree(e->d_scalars); cudaFree(e->d_hist); cudaFree(e->d_filt); cudaFree(e->d_view64);
+    cudaFree(e->d_scalars); cudaFree(e->d_hist); cudaFree(e->d_filt); cudaFree(e->d_view64); cudaFree(e->d_cam);
     cudaFree(e->d_dense); cudaFree(e->d_dense_tmp); cudaFree(e->d_mesh_verts); cudaFree(e->d_mesh_rgb); cudaFree(e->d_text);
     cudaFree(e->d_sparse_idx); cudaFree(e->d_sparse_words);
     cudaFree(e->d_scratch); cudaFree(e->d_undist_ir); vol_free(e->d_occ_full_own); vol_free(e->d_seen_full_own); cudaFree(e->d_reduce);
@@ -565,7 +574,7 @@ void vc_destroy(vc_engine* e) {
     {
         std::lock_guard<std::mutex> lk(g_const_mutex);
         ConstOwner& o = g_const_owner[e->g.device & 63];
-        if (o.uid == e->uid) { o.uid = 0; o.version = 0; o.used = false; }  // the stream was synchronised above; the event is kept for the device
+        if (o.uid == e->uid) { o.uid = 0; o.version = 0; o.group = 0; o.used = false; }  // the stream was synchronised above; the event is kept for the device
     }
     delete e;
 }
@@ -625,11 +634,29 @@ int vc_set_views(vc_engine* e, int32_t V, int32_t W, int32_t H, const float* P, 
         }
     }
     e->have_M = M != nullptr;
-    vc_filter_constants(e);
+    vc_filter_constants(e, e->h_filt.data(), V);
     VC_CUDA(e, cudaMemcpyAsync(e->d_filt, e->h_filt.data(), sizeof(VcViewFilter) * V, cudaMemcpyHostToDevice, e->stream));  // h_filt lives until the next vc_set_views, which synchronises first
     VC_CUDA(e, cudaMemcpyAsync(e->d_view64, e->h_view.data(), sizeof(VcViewConst) * V, cudaMemcpyHostToDevice, e->stream));
     e->views_version++;
     return VC_OK;
+}
+
+// bit packing (8UC3 input: bgr = the pixels of view v0, else nullptr) and summed-area tables of the views [v0, v1) into the
+// given mask / table buffers, on the engine's stream
+static cudaError_t build_view_tables(vc_engine* e, const uint8_t* bgr, uint32_t* mask, uint32_t* sat_tmp, vc_sat_t* sat, int v0, int v1) {
+    const size_t view_words = (size_t)e->H * e->Ww;
+    const int nv = v1 - v0;
+    uint32_t* m = mask + (size_t)v0 * view_words;
+    uint32_t* t = sat_tmp + (size_t)v0 * view_words;
+    const long long n_rows = (long long)nv * e->H;
+    const int n_cols = nv * e->Ww;
+    if (bgr) {
+        const long long warps = n_rows * e->Ww;
+        vc_pack_bgr_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, e->stream>>>(bgr, m, e->W, e->Ww, n_rows);
+    }
+    vc_sat_rowprefix_kernel<<<(unsigned)((n_rows + 7) / 8), 256, 0, e->stream>>>(m, t, e->Ww, n_rows);  // a warp per row
+    vc_sat_build_kernel<<<(unsigned)n_cols, 32 * VC_SAT_WARPS, 0, e->stream>>>(m, t, sat + (size_t)v0 * (e->H + 1) * vc_sat_pitch(e->W), e->W, e->H, e->Ww, nv);
+    return cudaGetLastError();
 }
 
 int vc_set_masks(vc_engine* e, const void* masks, int32_t format) {
@@ -643,7 +670,7 @@ int vc_set_masks(vc_engine* e, const void* masks, int32_t format) {
     const size_t sat_words = (size_t)e->V * (e->H + 1) * vc_sat_pitch(e->W);
     if (!e->d_sat) VC_CUDA(e, cudaMalloc(&e->d_sat, sat_words * sizeof(vc_sat_t)));
     if (!e->d_sat_tmp) VC_CUDA(e, cudaMalloc(&e->d_sat_tmp, e->mask_bytes));
-    const size_t view_words = (size_t)e->H * e->Ww, view_bgr = (size_t)e->H * e->W * 3;
+    const size_t view_bgr = (size_t)e->H * e->W * 3;
     const size_t bgr_bytes = (size_t)e->V * view_bgr;
     uint8_t* d_tmp = nullptr;
     if (format != VC_MASK_BITS) {
@@ -655,21 +682,6 @@ int vc_set_masks(vc_engine* e, const void* masks, int32_t format) {
         }
         d_tmp = e->d_bgr_tmp;
     }
-    // bit packing (8UC3 input) and summed-area tables of the views [v0, v1), on the engine's stream
-    auto build_views = [&](int v0, int v1) -> cudaError_t {
-        const int nv = v1 - v0;
-        uint32_t* m = e->d_mask + (size_t)v0 * view_words;
-        uint32_t* t = e->d_sat_tmp + (size_t)v0 * view_words;
-        const long long n_rows = (long long)nv * e->H;
-        const int n_cols = nv * e->Ww;
-        if (format != VC_MASK_BITS) {
-            const long long warps = n_rows * e->Ww;
-            vc_pack_bgr_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, e->stream>>>(d_tmp + (size_t)v0 * view_bgr, m, e->W, e->Ww, n_rows);
-        }
-        vc_sat_rowprefix_kernel<<<(unsigned)((n_rows + 7) / 8), 256, 0, e->stream>>>(m, t, e->Ww, n_rows);  // a warp per row
-        vc_sat_build_kernel<<<(unsigned)n_cols, 32 * VC_SAT_WARPS, 0, e->stream>>>(m, t, e->d_sat + (size_t)v0 * (e->H + 1) * vc_sat_pitch(e->W), e->W, e->H, e->Ww, nv);
-        return cudaGetLastError();
-    };
     // (Uploading the views in groups on a second stream, each group's tables built while the next one travels, was measured on
     // C4 with page-locked masks: 1.66 ms per end-to-end step instead of 1.45 ms - the 0.2 ms of overlap are less than what the
     // extra copies, events and 9 more launches cost the host.  One copy, one table build.)
@@ -687,7 +699,7 @@ int vc_set_masks(vc_engine* e, const void* masks, int32_t format) {
             if (us != cudaSuccess) return fail(e, VC_ERR_CUDA, "vc_set_masks: undistort failed: %s", cudaGetErrorString(us));
         }
     }
-    VC_CUDA(e, build_views(0, e->V));
+    VC_CUDA(e, build_view_tables(e, d_tmp, e->d_mask, e->d_sat_tmp, e->d_sat, 0, e->V));
     return VC_OK;
 }
 
@@ -817,6 +829,102 @@ int vc_set_images_raw(vc_engine* e, const uint8_t* images_bgr) {
     return VC_OK;
 }
 
+int vc_append_views(vc_engine* e, int32_t n, const float* P, const float* M, const void* masks, int32_t mask_format, const uint8_t* images_bgr) {
+    if (!e) return VC_ERR_ARG;
+    // every check before any state changes
+    if (e->V == 0 || !e->d_mask) return fail(e, VC_ERR_STATE, "vc_append_views: call vc_set_views and vc_set_masks first");
+    if (mask_format != VC_MASK_BITS && mask_format != VC_MASK_BGR8 && mask_format != VC_MASK_BGR8_RAW) return fail(e, VC_ERR_ARG, "vc_append_views: unknown mask format %d", mask_format);
+    if (mask_format == VC_MASK_BGR8_RAW && !e->have_calib) return fail(e, VC_ERR_STATE, "vc_append_views: raw masks need vc_set_calibration first");
+    if (n < 1) return fail(e, VC_ERR_ARG, "vc_append_views: n=%d views (need at least 1)", n);
+    if (!P || !masks) return fail(e, VC_ERR_ARG, "vc_append_views: P and masks are required");
+    if ((long long)e->V + n > VC_MAX_TOTAL_VIEWS) return fail(e, VC_ERR_ARG, "vc_append_views: %d + %d views exceed %d", e->V, n, VC_MAX_TOTAL_VIEWS);
+    const int V1 = e->V + n;
+    const size_t view_words = (size_t)e->H * e->Ww, view_bgr = (size_t)e->H * e->W * 3;
+    if ((size_t)V1 * view_words > 0x7fffffffull) return fail(e, VC_ERR_ARG, "vc_append_views: %d views of %dx%d exceed 2^31 mask words", V1, e->W, e->H);
+    if ((M != nullptr) != e->have_M) return fail(e, VC_ERR_ARG, "vc_append_views: M must be given if and only if the engine's views have M (%s)", e->have_M ? "they do" : "they do not");
+    if ((images_bgr != nullptr) != (e->d_images != nullptr))
+        return fail(e, VC_ERR_ARG, "vc_append_views: images must be given if and only if the engine holds images (%s)", e->d_images ? "it does" : "it does not");
+    if (bind_device(e)) return VC_ERR_CUDA;
+    VC_CUDA(e, cudaStreamSynchronize(e->stream));  // earlier work may still read the host view vectors and the buffers replaced below
+    // host side of the new views
+    std::vector<VcViewConst> hv(e->h_view);
+    std::vector<float> hc(e->h_cam);
+    std::vector<VcViewFilter> hf(e->h_filt);
+    hv.resize(V1); hc.resize((size_t)V1 * 4, 0.0f); hf.resize(V1, VcViewFilter{});
+    for (int i = 0; i < n; i++) {
+        const int v = e->V + i;
+        for (int k = 0; k < 12; k++) hv[v].P[k] = (double)P[i * 12 + k];
+        for (int k = 0; k < 12; k++) hf[v].P[k] = P[i * 12 + k];
+        if (M) { hc[v * 4 + 0] = M[i * 12 + 3]; hc[v * 4 + 1] = M[i * 12 + 7]; hc[v * 4 + 2] = M[i * 12 + 11]; hc[v * 4 + 3] = 1.0f; }
+    }
+    vc_filter_constants(e, hf.data() + e->V, n);  // (it also rewrites hDu / hDv, which depend on W and H only: same values)
+    // new buffers for all V1 views; the engine's own are replaced only once everything has succeeded
+    const bool raw = mask_format == VC_MASK_BGR8_RAW;
+    const size_t sat_view = (size_t)(e->H + 1) * vc_sat_pitch(e->W);
+    uint32_t *mask = nullptr, *sat_tmp = nullptr;
+    vc_sat_t* sat = nullptr;
+    uint8_t *images = nullptr, *stage = nullptr;
+    VcViewFilter* filt = nullptr;
+    VcViewConst* view64 = nullptr;
+    float4* cam = nullptr;
+    const size_t stage_bytes = mask_format != VC_MASK_BITS ? (size_t)n * view_bgr * (raw ? 2 : 1) : 0;  // 8UC3 masks [+ undistorted copy]; raw images reuse it
+    cudaError_t s = cudaMalloc(&mask, (size_t)V1 * view_words * 4);
+    if (s == cudaSuccess) s = cudaMalloc(&sat_tmp, (size_t)V1 * view_words * 4);
+    if (s == cudaSuccess) s = cudaMalloc(&sat, (size_t)V1 * sat_view * sizeof(vc_sat_t));
+    if (s == cudaSuccess && images_bgr) s = cudaMalloc(&images, (size_t)V1 * view_bgr);
+    if (s == cudaSuccess && stage_bytes) s = cudaMalloc(&stage, stage_bytes);
+    // never fewer than VC_MAX_VIEWS entries: a later vc_set_views writes up to that many into these buffers without reallocating
+    const size_t view_cap = (size_t)std::max(V1, VC_MAX_VIEWS);
+    if (s == cudaSuccess) s = cudaMalloc(&filt, view_cap * sizeof(VcViewFilter));
+    if (s == cudaSuccess) s = cudaMalloc(&view64, view_cap * sizeof(VcViewConst));
+    if (s == cudaSuccess) s = cudaMalloc(&cam, (size_t)V1 * sizeof(float4));
+    // the earlier views' masks, tables and images as they are, the new views' after them
+    if (s == cudaSuccess) s = cudaMemcpyAsync(mask, e->d_mask, e->mask_bytes, cudaMemcpyDeviceToDevice, e->stream);
+    if (s == cudaSuccess) s = cudaMemcpyAsync(sat, e->d_sat, (size_t)e->V * sat_view * sizeof(vc_sat_t), cudaMemcpyDeviceToDevice, e->stream);
+    if (s == cudaSuccess && images_bgr) s = cudaMemcpyAsync(images, e->d_images, (size_t)e->V * view_bgr, cudaMemcpyDeviceToDevice, e->stream);
+    if (s == cudaSuccess) s = cudaMemcpyAsync(filt, hf.data(), (size_t)V1 * sizeof(VcViewFilter), cudaMemcpyHostToDevice, e->stream);
+    if (s == cudaSuccess) s = cudaMemcpyAsync(view64, hv.data(), (size_t)V1 * sizeof(VcViewConst), cudaMemcpyHostToDevice, e->stream);
+    if (s == cudaSuccess) s = cudaMemcpyAsync(cam, hc.data(), (size_t)V1 * sizeof(float4), cudaMemcpyHostToDevice, e->stream);
+    const uint8_t* bgr = nullptr;  // the new views' 8UC3 masks on the device
+    if (s == cudaSuccess) {
+        if (mask_format == VC_MASK_BITS) {
+            s = cudaMemcpyAsync(mask + (size_t)e->V * view_words, masks, (size_t)n * view_words * 4, cudaMemcpyDefault, e->stream);  // host or device memory
+        } else {
+            s = cudaMemcpyAsync(stage, masks, (size_t)n * view_bgr, cudaMemcpyHostToDevice, e->stream);
+            bgr = stage;
+            if (s == cudaSuccess && raw) {  // cv::undistort(mask, ...) (VoxelCarving.cpp:36)
+                s = undistort_device(stage, stage + (size_t)n * view_bgr, n, e->W, e->H, e->calib_K, e->calib_dist, e->stream, &e->d_undist_ir, &e->undist_ir_count);
+                bgr = stage + (size_t)n * view_bgr;
+            }
+        }
+    }
+    if (s == cudaSuccess) s = build_view_tables(e, bgr, mask, sat_tmp, sat, e->V, V1);
+    if (s == cudaSuccess && images_bgr) {
+        uint8_t* dst = images + (size_t)e->V * view_bgr;
+        if (raw) {  // ColorReconstruction.h:23
+            s = cudaMemcpyAsync(stage, images_bgr, (size_t)n * view_bgr, cudaMemcpyHostToDevice, e->stream);
+            if (s == cudaSuccess) s = undistort_device(stage, dst, n, e->W, e->H, e->calib_K, e->calib_dist, e->stream, &e->d_undist_ir, &e->undist_ir_count);
+        } else {
+            s = cudaMemcpyAsync(dst, images_bgr, (size_t)n * view_bgr, cudaMemcpyHostToDevice, e->stream);
+        }
+    }
+    if (s == cudaSuccess) s = cudaStreamSynchronize(e->stream);  // the host vectors above are locals, and any error surfaces here
+    cudaFree(stage);
+    if (s != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(mask); cudaFree(sat_tmp); cudaFree(sat); cudaFree(images); cudaFree(filt); cudaFree(view64); cudaFree(cam);
+        return fail(e, VC_ERR_CUDA, "vc_append_views: %s (the engine is unchanged)", cudaGetErrorString(s));
+    }
+    cudaFree(e->d_mask); cudaFree(e->d_sat_tmp); cudaFree(e->d_sat); cudaFree(e->d_filt); cudaFree(e->d_view64); cudaFree(e->d_cam);
+    e->d_mask = mask; e->d_sat_tmp = sat_tmp; e->d_sat = sat; e->d_filt = filt; e->d_view64 = view64; e->d_cam = cam;
+    if (images_bgr) { cudaFree(e->d_images); e->d_images = images; }
+    e->h_view.swap(hv); e->h_cam.swap(hc); e->h_filt.swap(hf);
+    e->V = V1;
+    e->mask_bytes = (size_t)V1 * view_words * 4;
+    e->views_version++;
+    return VC_OK;
+}
+
 int vc_download_masks(vc_engine* e, uint32_t* bits) {
     if (!e) return VC_ERR_ARG;
     if (!bits) return fail(e, VC_ERR_ARG, "vc_download_masks: null buffer");
@@ -907,14 +1015,32 @@ static VcCarveParams carve_params(vc_engine* e, int view_begin, int view_end) {
     return p;
 }
 
+// The part of the view range [v0, v1) that lies in view group g, as carve parameters relative to the group's first view: the
+// kernels index the constant tables and the per-view buffers from there, so their view offsets stay what they are for one group.
+static VcCarveParams group_params(const vc_engine* e, VcCarveParams p, int g, int v0, int v1) {
+    const int base = g * VC_MAX_VIEWS;
+    p.v0 = std::max(v0, base) - base;
+    p.v1 = std::max(std::min(v1, base + VC_MAX_VIEWS) - base, p.v0);
+    p.mask = e->d_mask + (size_t)base * p.mask_plane;
+    return p;
+}
+// the view groups [g0, g1] that [v0, v1) intersects; an empty range still gets the group of v0 (a fresh carve writes the reset)
+static void group_span(const vc_engine* e, int v0, int v1, int& g0, int& g1) {
+    g0 = std::min(v0, e->V - 1) / VC_MAX_VIEWS;
+    g1 = v1 > v0 ? (v1 - 1) / VC_MAX_VIEWS : g0;
+}
+
 static bool blind_fill_enabled() {  // VOXCARVE_BLIND_FILL=0: the r1 scheme (flag-driven fill by the first blocks of vc_carve_bricks), for comparison
     static const bool off = [] { const char* v = getenv("VOXCARVE_BLIND_FILL"); return v && v[0] == '0'; }();
     return !off;
 }
 
 // VC_EXACT on the planes [zl0, zl1) of the slab (zl0 a multiple of the super-brick height, so bricks sit where they
-// would in a whole-slab pass): classify super-bricks, classify bricks, fill, evaluate the undecided pairs.
-static int carve_exact_range(vc_engine* e, VcCarveParams p, int zl0, int zl1, bool count, bool fresh, bool record_mid, uint64_t* n_bricks_out) {
+// would in a whole-slab pass): classify super-bricks, classify bricks, fill, evaluate the undecided pairs.  vbase: first view
+// of the group whose constants are loaded (p from group_params); the per-view device arrays are read from there.
+static int carve_exact_range(vc_engine* e, VcCarveParams p, int zl0, int zl1, bool count, bool fresh, bool record_mid, uint64_t* n_bricks_out,
+                             int vbase = 0) {
+    const vc_sat_t* sat = e->d_sat + (size_t)vbase * (e->H + 1) * vc_sat_pitch(e->W);
     const long long off = (long long)zl0 * e->plane_words;
     p.occ += off; p.seen += off;
     p.z_begin = e->g.z_begin + zl0; p.nz = zl1 - zl0;
@@ -957,7 +1083,7 @@ static int carve_exact_range(vc_engine* e, VcCarveParams p, int zl0, int zl1, bo
     VC_CUDA(e, cudaMemsetAsync(e->d_scalars + 6, 0, 2 * sizeof(unsigned long long), e->stream));
     VcBrickParams bp{};
     bp.list = e->d_bricks; bp.n_list = d_nlist; bp.n_list_back = d_work + 1; bp.list_cap = (unsigned)n_bricks;
-    bp.brick_flags = e->d_brick_flags; bp.sat = e->d_sat;
+    bp.brick_flags = e->d_brick_flags; bp.sat = sat;
     bp.super_flags = e->d_super_flags; bp.super_list = e->d_super_list; bp.n_super_list = d_nlist + 1;
     bp.executed = count ? e->d_scalars + 5 : nullptr;
     bp.X = e->g.X; bp.Y = e->g.Y; bp.Wx = e->Wx; bp.nz = p.nz; bp.z_begin = p.z_begin;
@@ -1012,9 +1138,9 @@ static int carve_exact_range(vc_engine* e, VcCarveParams p, int zl0, int zl1, bo
     (void)pdl;
     const VcBrickState* list_c = e->d_bricks;
     const unsigned int *n_front_c = d_nlist, *n_back_c = d_work + 1;
-    const vc_sat_t* sat_c = e->d_sat;
-    const VcViewFilter* filt_c = e->d_filt;
-    const VcViewConst* view_c = e->d_view64;
+    const vc_sat_t* sat_c = sat;
+    const VcViewFilter* filt_c = e->d_filt + vbase;
+    const VcViewConst* view_c = e->d_view64 + vbase;
     if (count) VC_CUDA(e, launch_pdl(vc_carve_bricks<true>, dim3(pgrid), dim3(256), e->stream, pdl_cb, p, list_c, n_front_c, n_back_c, (unsigned)n_bricks, d_work, nbx, nby, sat_c, fresh ? 1 : 0, filt_c, view_c, fp));
     else VC_CUDA(e, launch_pdl(vc_carve_bricks<false>, dim3(pgrid), dim3(256), e->stream, pdl_cb, p, list_c, n_front_c, n_back_c, (unsigned)n_bricks, d_work, nbx, nby, sat_c, fresh ? 1 : 0, filt_c, view_c, fp));
     VC_CUDA(e, cudaGetLastError());
@@ -1032,7 +1158,7 @@ static int carve_check(vc_engine* e, const char* who, int32_t mode, int32_t& vie
     if (bind_device(e)) return VC_ERR_CUDA;
     int rc = ensure_volumes(e);
     if (rc) return rc;
-    return ensure_constants(e);
+    return e->V > VC_MAX_VIEWS ? VC_OK : ensure_constants(e);  // several groups: uploaded group by group
 }
 
 // NVTX range named after a phase of the reference's Benchmark singleton (Benchmark.h:86-124): Carving, Coloring,
@@ -1071,11 +1197,36 @@ int vc_carve(vc_engine* e, int32_t mode, int32_t view_begin, int32_t view_end, i
     e->have_mid = mode == VC_EXACT;
     e->stats.bricks_total = 0;
     e->stats.bricks_listed = 0;
+    uint64_t listed_in_groups = 0;  // counting run over several view groups: listed bricks summed over the groups
     if (mode == VC_EXACT) {
         if (e->use_graphs < 0) { const char* ng = getenv("VOXCARVE_NO_GRAPH"); e->use_graphs = (ng && atoi(ng) != 0) ? 0 : 1; }
         const bool fresh = e->reset_pending;
         bool launched = false;
-        if (e->use_graphs && !e->profiling && !count_executed && view_begin == 0 && view_end == e->V) {
+        if (e->V > VC_MAX_VIEWS) {
+            // One plain sequence per view group, the constants of each uploaded in stream order behind the previous group's
+            // kernels; only the first group starts from a pending reset, the others accumulate onto its result.
+            int g0, g1;
+            group_span(e, view_begin, view_end, g0, g1);
+            for (int g = g0; g <= g1; g++) {
+                rc = ensure_constants(e, g);
+                if (rc) return rc;
+                uint64_t nb = 0;
+                rc = carve_exact_range(e, group_params(e, p, g, view_begin, view_end), 0, e->nz, count_executed != 0, fresh && g == g0, false,
+                                       &nb, g * VC_MAX_VIEWS);
+                if (rc) return rc;
+                e->stats.bricks_total = nb;
+                if (count_executed) {  // the next group resets the list lengths
+                    unsigned long long nl = 0, nw = 0;
+                    VC_CUDA(e, cudaMemcpyAsync(&nl, e->d_scalars + 6, sizeof nl, cudaMemcpyDeviceToHost, e->stream));
+                    VC_CUDA(e, cudaMemcpyAsync(&nw, e->d_scalars + 7, sizeof nw, cudaMemcpyDeviceToHost, e->stream));
+                    VC_CUDA(e, cudaStreamSynchronize(e->stream));
+                    listed_in_groups += (nl & 0xffffffffull) + (nw >> 32);
+                }
+            }
+            e->have_mid = false;
+            launched = true;
+        }
+        if (!launched && e->use_graphs && !e->profiling && !count_executed && view_begin == 0 && view_end == e->V) {
             CarveGraphKey k;
             memset(&k, 0, sizeof k);  // padding bytes too: the key is compared with memcmp
             k.p = p;
@@ -1114,7 +1265,18 @@ int vc_carve(vc_engine* e, int32_t mode, int32_t view_begin, int32_t view_end, i
             if (rc) return rc;
         }
         e->reset_pending = false;
-        e->flags_valid = fresh && view_begin == 0 && view_end == e->V;  // the flags of this call say everything about the volumes
+        // the flags of this call say everything about the volumes (with several groups, no single group's flags do)
+        e->flags_valid = fresh && view_begin == 0 && view_end == e->V && e->V <= VC_MAX_VIEWS;
+    } else if (e->V > VC_MAX_VIEWS) {
+        int g0, g1;
+        group_span(e, view_begin, view_end, g0, g1);
+        for (int g = g0; g <= g1; g++) {
+            rc = ensure_constants(e, g);
+            if (rc) return rc;
+            rc = launch_carve<4>(e, mode == VC_EXACT_FLAT ? VC_EXACT : mode, group_params(e, p, g, view_begin, view_end), count_executed != 0);
+            if (rc) return rc;
+        }
+        e->flags_valid = false;
     } else {
         rc = launch_carve<4>(e, mode == VC_EXACT_FLAT ? VC_EXACT : mode, p, count_executed != 0);
         if (rc) return rc;
@@ -1141,7 +1303,7 @@ int vc_carve(vc_engine* e, int32_t mode, int32_t view_begin, int32_t view_end, i
         VC_CUDA(e, cudaMemcpyAsync(&nl, e->d_scalars + 6, sizeof nl, cudaMemcpyDeviceToHost, e->stream));
         VC_CUDA(e, cudaMemcpyAsync(&nw, e->d_scalars + 7, sizeof nw, cudaMemcpyDeviceToHost, e->stream));
         VC_CUDA(e, cudaStreamSynchronize(e->stream));
-        e->stats.bricks_listed = mode == VC_EXACT ? (nl & 0xffffffffull) + (nw >> 32) : 0;  // front + back of the work list
+        e->stats.bricks_listed = mode != VC_EXACT ? 0 : e->V > VC_MAX_VIEWS ? listed_in_groups : (nl & 0xffffffffull) + (nw >> 32);  // front + back of the work list
         e->stats.executed_voxel_views = ex + (mode == VC_EXACT ? bc : 0);
         e->stats.brick_corner_views = mode == VC_EXACT ? bc : 0;
         if (mode == VC_EXACT) { e->stats.filter_rows = fl[0]; e->stats.filter_slow_rows = fl[1]; e->stats.filter_mismatches = fl[2]; e->stats.subbrick_corner_views = fl[3]; }
@@ -1191,8 +1353,19 @@ int vc_carve_download(vc_engine* e, int32_t mode, uint32_t* occupied, uint32_t* 
     int c = 0;
     for (int zl0 = 0; zl0 < e->nz; zl0 += cz, c++) {
         const int zl1 = zl0 + cz < e->nz ? zl0 + cz : e->nz;
-        rc = carve_exact_range(e, p, zl0, zl1, false, fresh, false, &e->stats.bricks_total);
-        if (rc) return rc;
+        if (e->V <= VC_MAX_VIEWS) {
+            rc = carve_exact_range(e, p, zl0, zl1, false, fresh, false, &e->stats.bricks_total);
+            if (rc) return rc;
+        } else {
+            for (int g = 0; g < n_groups(e); g++) {  // the chunk's first group starts from the pending reset
+                rc = ensure_constants(e, g);
+                if (rc) return rc;
+                uint64_t nb = 0;
+                rc = carve_exact_range(e, group_params(e, p, g, v0, v1), zl0, zl1, false, fresh && g == 0, false, &nb, g * VC_MAX_VIEWS);
+                if (rc) return rc;
+                if (g == 0) e->stats.bricks_total += nb;
+            }
+        }
         VC_CUDA(e, cudaEventRecord(e->ev_chunk[c], e->stream));
         VC_CUDA(e, cudaStreamWaitEvent(e->copy_stream, e->ev_chunk[c], 0));
         const long long off = (long long)zl0 * e->plane_words, n = (long long)(zl1 - zl0) * e->plane_words;
@@ -1246,7 +1419,13 @@ int vc_carve_download_sparse(vc_engine* e, uint8_t* brick_flags, uint64_t flags_
     rc = ensure_scratch(e, (size_t)n_bricks, &sc);  // resolved flags (the per-brick array is only written under undecided super-bricks)
     if (rc) return rc;
     uint8_t* d_flags = (uint8_t*)sc;
-    vc_sparse_flags_kernel<<<(unsigned)((n_bricks + 255) / 256), 256, 0, e->stream>>>(e->d_brick_flags, e->d_super_flags, d_flags, nbx, nby, nbz, sbx, sby);
+    if (e->V <= VC_MAX_VIEWS) {
+        vc_sparse_flags_kernel<<<(unsigned)((n_bricks + 255) / 256), 256, 0, e->stream>>>(e->d_brick_flags, e->d_super_flags, d_flags, nbx, nby, nbz, sbx, sby);
+    } else {  // several view groups: the flags and the list come from the volumes (the work list's front, its back left empty)
+        VC_CUDA(e, cudaMemsetAsync(e->d_scalars + 6, 0, 2 * sizeof(unsigned long long), e->stream));
+        vc_sparse_volume_flags_kernel<<<(unsigned)((n_bricks * 32 + 255) / 256), 256, 0, e->stream>>>(
+            e->occ_slab(), e->seen_slab(), d_flags, e->d_bricks, (unsigned int*)(e->d_scalars + 6), e->g.X, e->g.Y, e->nz, e->Wx, nbx, nby, nbz);
+    }
     VC_CUDA(e, cudaGetLastError());
     unsigned int counts[4] = {0, 0, 0, 0};  // front length, super-list length, work counter, back length
     VC_CUDA(e, cudaMemcpyAsync(counts, e->d_scalars + 6, sizeof counts, cudaMemcpyDeviceToHost, e->stream));
@@ -1340,44 +1519,49 @@ int vc_plan_slabs(vc_engine* e, int32_t n_parts, int32_t* z_bounds) {
     if (n_parts < 1 || n_parts > e->nz) return fail(e, VC_ERR_ARG, "vc_plan_slabs: n_parts=%d outside [1,%d]", n_parts, e->nz);
     if (e->V == 0 || !e->d_mask) return fail(e, VC_ERR_STATE, "vc_plan_slabs: views and masks must be set first");
     if (bind_device(e)) return VC_ERR_CUDA;
-    int rc = ensure_constants(e);
-    if (rc) return rc;
+    int rc = VC_OK;
     for (int k = 0; k <= n_parts; k++) z_bounds[k] = e->g.z_begin + (int)((long long)k * e->nz / n_parts);  // uniform fallback
     const int nbx = e->Wx, nby = (e->g.Y + VC_BY - 1) / VC_BY, nbz = (e->nz + VC_BZ - 1) / VC_BZ;
     if (nbz < n_parts) return VC_OK;  // fewer brick layers than parts: keep the uniform split
     rc = ensure_brick_buffers(e);
     if (rc) return rc;
     e->flags_valid = false;
-    // both classification levels of VC_EXACT over the whole range, no volumes touched
+    // both classification levels of VC_EXACT over the whole range, no volumes touched; once per view group, costs summed
     const int sbx = (nbx + VC_SUPER - 1) / VC_SUPER, sby = (nby + VC_SUPER - 1) / VC_SUPER, sbz = (nbz + VC_SUPER - 1) / VC_SUPER;
     const long long n_super = (long long)sbx * sby * sbz;
     unsigned int* d_nlist = (unsigned int*)(e->d_scalars + 6);
-    VC_CUDA(e, cudaMemsetAsync(e->d_scalars + 6, 0, 2 * sizeof(unsigned long long), e->stream));
-    VcBrickParams bp{};
-    bp.list = e->d_bricks; bp.n_list = d_nlist; bp.n_list_back = d_nlist + 3; bp.list_cap = (unsigned)((long long)nbx * nby * nbz);
-    bp.brick_flags = e->d_brick_flags; bp.sat = e->d_sat;
-    bp.super_flags = e->d_super_flags; bp.super_list = e->d_super_list; bp.n_super_list = d_nlist + 1;
-    bp.X = e->g.X; bp.Y = e->g.Y; bp.Wx = e->Wx; bp.nz = e->nz; bp.z_begin = e->g.z_begin;
-    bp.nbx = nbx; bp.nby = nby; bp.nbz = nbz; bp.W = e->W; bp.H = e->H; bp.v0 = 0; bp.v1 = e->V; bp.s = e->g.voxel_size;
-    VcBrickParams sp = bp;
-    sp.dense = e->d_super; sp.nbx = sbx; sp.nby = sby; sp.nbz = sbz;
-    vc_brick_classify_kernel<1><<<(unsigned)((n_super + VC_CLS_L1_CH - 1) / VC_CLS_L1_CH), 256, 0, e->stream>>>(sp);  // VC_CLS_L1_CH super-bricks per block
-    bp.dense = e->d_super; bp.pbx = sbx; bp.pby = sby;
-    {   // level 0: the blocks walk the list of undecided super-bricks (length known on the device only)
-        const long long l0_grid = std::min<long long>(n_super, 8LL * e->sm_count);
-        vc_brick_classify_kernel<0><<<(unsigned)l0_grid, VC_CLS_L0_THREADS, 0, e->stream>>>(bp);
-    }
-    unsigned int counts[4] = {0, 0, 0, 0};  // front length, super-list length, (work counter), back length
-    VC_CUDA(e, cudaMemcpyAsync(counts, d_nlist, sizeof counts, cudaMemcpyDeviceToHost, e->stream));
-    VC_CUDA(e, cudaStreamSynchronize(e->stream));
-    std::vector<VcBrickState> h((size_t)counts[0] + counts[3]);  // the list is filled from both ends (VcBrickParams)
-    if (counts[0]) VC_CUDA(e, cudaMemcpy(h.data(), e->d_bricks, (size_t)counts[0] * sizeof(VcBrickState), cudaMemcpyDeviceToHost));
-    if (counts[3]) VC_CUDA(e, cudaMemcpy(h.data() + counts[0], e->d_bricks + (bp.list_cap - counts[3]), (size_t)counts[3] * sizeof(VcBrickState), cudaMemcpyDeviceToHost));
     // cost of a brick layer (8 planes): per-voxel work of its listed bricks (undecided views x voxels) plus a small constant
     // per plane for the classification and fill passes
     std::vector<double> cost((size_t)nbz, 0.0);
+    for (int grp = 0; grp < n_groups(e); grp++) {
+        rc = ensure_constants(e, grp);
+        if (rc) return rc;
+        const int vbase = grp * VC_MAX_VIEWS;
+        VC_CUDA(e, cudaMemsetAsync(e->d_scalars + 6, 0, 2 * sizeof(unsigned long long), e->stream));
+        VcBrickParams bp{};
+        bp.list = e->d_bricks; bp.n_list = d_nlist; bp.n_list_back = d_nlist + 3; bp.list_cap = (unsigned)((long long)nbx * nby * nbz);
+        bp.brick_flags = e->d_brick_flags; bp.sat = e->d_sat + (size_t)vbase * (e->H + 1) * vc_sat_pitch(e->W);
+        bp.super_flags = e->d_super_flags; bp.super_list = e->d_super_list; bp.n_super_list = d_nlist + 1;
+        bp.X = e->g.X; bp.Y = e->g.Y; bp.Wx = e->Wx; bp.nz = e->nz; bp.z_begin = e->g.z_begin;
+        bp.nbx = nbx; bp.nby = nby; bp.nbz = nbz; bp.W = e->W; bp.H = e->H; bp.v0 = 0; bp.v1 = std::min(VC_MAX_VIEWS, e->V - vbase); bp.s = e->g.voxel_size;
+        VcBrickParams sp = bp;
+        sp.dense = e->d_super; sp.nbx = sbx; sp.nby = sby; sp.nbz = sbz;
+        vc_brick_classify_kernel<1><<<(unsigned)((n_super + VC_CLS_L1_CH - 1) / VC_CLS_L1_CH), 256, 0, e->stream>>>(sp);  // VC_CLS_L1_CH super-bricks per block
+        bp.dense = e->d_super; bp.pbx = sbx; bp.pby = sby;
+        {   // level 0: the blocks walk the list of undecided super-bricks (length known on the device only)
+            const long long l0_grid = std::min<long long>(n_super, 8LL * e->sm_count);
+            vc_brick_classify_kernel<0><<<(unsigned)l0_grid, VC_CLS_L0_THREADS, 0, e->stream>>>(bp);
+        }
+        unsigned int counts[4] = {0, 0, 0, 0};  // front length, super-list length, (work counter), back length
+        VC_CUDA(e, cudaMemcpyAsync(counts, d_nlist, sizeof counts, cudaMemcpyDeviceToHost, e->stream));
+        VC_CUDA(e, cudaStreamSynchronize(e->stream));
+        std::vector<VcBrickState> h((size_t)counts[0] + counts[3]);  // the list is filled from both ends (VcBrickParams)
+        if (counts[0]) VC_CUDA(e, cudaMemcpy(h.data(), e->d_bricks, (size_t)counts[0] * sizeof(VcBrickState), cudaMemcpyDeviceToHost));
+        if (counts[3]) VC_CUDA(e, cudaMemcpy(h.data() + counts[0], e->d_bricks + (bp.list_cap - counts[3]), (size_t)counts[3] * sizeof(VcBrickState), cudaMemcpyDeviceToHost));
+        for (const VcBrickState& st : h) cost[st.brick / ((unsigned)nbx * (unsigned)nby)] += (double)st.n_und * (VC_BX * VC_BY * VC_BZ);
+    }
+    // (every group's kernels are complete: its list was read back above)
     double total = 0.0;
-    for (const VcBrickState& st : h) cost[st.brick / ((unsigned)nbx * (unsigned)nby)] += (double)st.n_und * (VC_BX * VC_BY * VC_BZ);
     for (int z = 0; z < nbz; z++) total += cost[z];
     const double floor_cost = total > 0 ? 0.03 * total / nbz : 1.0;
     total = 0.0;
@@ -1500,8 +1684,8 @@ int vc_color(vc_engine* e, int32_t color_mode) {
     if (bind_device(e)) return VC_ERR_CUDA;
     rc = materialize_reset(e);
     if (rc) return rc;
-    rc = ensure_constants(e);
-    if (rc) return rc;
+    const bool global_views = e->V > VC_MAX_VIEWS;  // one pass over every group: P and camera from global memory
+    if (!global_views) { rc = ensure_constants(e); if (rc) return rc; }
     const long long n = e->slab_words;
     if (n > 0x7fffffffLL) return fail(e, VC_ERR_ARG, "vc_color: slab of %lld words too large", n);
     if (e->nz > 65535) return fail(e, VC_ERR_ARG, "vc_color: slab of %d planes too deep (grid dimension limit 65535)", e->nz);
@@ -1536,12 +1720,20 @@ int vc_color(vc_engine* e, int32_t color_mode) {
         p.s = e->g.voxel_size;
         p.mode = color_mode;
         p.n_surface = total;
+        p.gview = e->d_view64; p.gcam = e->d_cam;
         vc_surface_pass_kernel<true><<<sgrid, 256, 0, e->stream>>>(g, e->g.z_begin, (unsigned)e->plane_words, e->d_block_sums, e->d_color_idx);
-        if (color_mode == VC_COLOR_CLOSEST) vc_surface_color_kernel<1><<<(unsigned)((total + 255) / 256), 256, 0, e->stream>>>(p);
-        else vc_surface_color_kernel<2><<<(unsigned)((total + 255) / 256), 256, 0, e->stream>>>(p);
-        VC_CUDA(e, cudaGetLastError());
-        rc = constants_used(e);
-        if (rc) return rc;
+        const unsigned cgrid = (unsigned)((total + 255) / 256);
+        if (global_views) {
+            if (color_mode == VC_COLOR_CLOSEST) vc_surface_color_kernel<1, true><<<cgrid, 256, 0, e->stream>>>(p);
+            else vc_surface_color_kernel<2, true><<<cgrid, 256, 0, e->stream>>>(p);
+            VC_CUDA(e, cudaGetLastError());
+        } else {
+            if (color_mode == VC_COLOR_CLOSEST) vc_surface_color_kernel<1><<<cgrid, 256, 0, e->stream>>>(p);
+            else vc_surface_color_kernel<2><<<cgrid, 256, 0, e->stream>>>(p);
+            VC_CUDA(e, cudaGetLastError());
+            rc = constants_used(e);
+            if (rc) return rc;
+        }
     }
     e->have_colors = true;
     return VC_OK;

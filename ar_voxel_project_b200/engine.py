@@ -129,6 +129,41 @@ class VoxelEngine:
         self._check(self._lib.vc_set_views(self._h, V, int(W), int(H), P.ctypes.data, Mp))
         self.V, self.W, self.H = V, int(W), int(H)
 
+    def append_views(self, P, M=None, mask_bits=None, mask_bgr=None, raw=False, images_bgr=None):
+        """append views [V, V+n) of the engine's W x H geometry (vc_append_views): P (and M, iff the engine's views have M), their
+        masks (mask_bits uint32[n][H][ceil(W/32)], host array or a CUDA tensor; or mask_bgr uint8[n][H][W][3], distorted if raw),
+        and their images iff the engine holds images (raw: distorted, like the masks).  Only the new views' tables are built."""
+        P = np.ascontiguousarray(P, np.float32).reshape(-1, 12)
+        n = P.shape[0]
+        Mp = None
+        if M is not None:
+            M = np.ascontiguousarray(M, np.float32).reshape(-1, 12)
+            if M.shape[0] != n:
+                raise ValueError("M and P must have the same number of views")
+            Mp = M.ctypes.data
+        if (mask_bits is None) == (mask_bgr is None):
+            raise ValueError("append_views needs exactly one of mask_bits / mask_bgr")
+        Ww = (self.W + 31) // 32
+        if mask_bits is not None:
+            if raw:
+                raise ValueError("raw masks are 8UC3 images: pass them as mask_bgr")
+            fmt = L.VC_MASK_BITS
+            if hasattr(mask_bits, "is_cuda") and mask_bits.is_cuda:
+                if not mask_bits.is_contiguous() or mask_bits.numel() * mask_bits.element_size() < n * self.H * Ww * 4:
+                    raise ValueError("device mask bits: must be contiguous and hold n*H*ceil(W/32) words")
+                maddr, mkeep = mask_bits.data_ptr(), mask_bits
+            else:
+                maddr, mkeep = _host_ptr(mask_bits, np.uint32, n * self.H * Ww * 4, "mask bits")
+        else:
+            fmt = L.VC_MASK_BGR8_RAW if raw else L.VC_MASK_BGR8
+            maddr, mkeep = _host_ptr(mask_bgr, np.uint8, n * self.H * self.W * 3, "mask bgr")
+        iaddr = None
+        if images_bgr is not None:
+            iaddr, ikeep = _host_ptr(images_bgr, np.uint8, n * self.H * self.W * 3, "images bgr")
+        self._check(self._lib.vc_append_views(self._h, n, P.ctypes.data, Mp, C.c_void_p(maddr), fmt,
+                                              None if iaddr is None else C.c_void_p(iaddr)))
+        self.V += n
+
     def set_masks_bits(self, bits):
         """uint32[V][H][ceil(W/32)], 1 = background (carve)."""
         need = self.V * self.H * ((self.W + 31) // 32) * 4

@@ -79,7 +79,8 @@ typedef struct vc_stats {
     uint64_t nominal_voxel_views;  /* X*Y*(z_end-z_begin)*V of the last vc_carve */
     uint64_t executed_voxel_views; /* projections actually evaluated, incl. brick corners (0 unless counting was on) */
     uint64_t brick_corner_views;   /* the part of executed_voxel_views spent on brick classification */
-    uint64_t bricks_total;         /* bricks of the slab / bricks that needed per-voxel work in the last VC_EXACT carve */
+    uint64_t bricks_total;         /* bricks of the slab / bricks that needed per-voxel work in the last VC_EXACT carve (with more
+                                      than 256 views: summed over the view groups, so a brick listed in two groups counts twice) */
     uint64_t bricks_listed;
     uint64_t flood_rounds;         /* sweep rounds of the last vc_fast_carve */
     uint64_t carve_launches;       /* kernel launches issued by this engine so far */
@@ -123,8 +124,27 @@ VC_EXPORT int vc_set_profiling(vc_engine* e, int32_t on);
  *          may be NULL if no colour pass is run. All pointers are HOST memory.
  * Accepted: V in [1,256]; W, H in [1,2^20]; pitch*(H+1) < 2^31 with pitch = 32*(ceil(W/32)+1) (32-bit row offsets of a
  * view's summed-area table); V*H*ceil(W/32) < 2^31 mask words.  Anything else returns VC_ERR_ARG and changes nothing: the
- * engine keeps its previous views, masks, tables and images. */
+ * engine keeps its previous views, masks, tables and images.  An accepted call replaces every view, also on an engine that
+ * vc_append_views had grown past 256: afterwards it holds exactly these V views. */
 VC_EXPORT int vc_set_views(vc_engine* e, int32_t V, int32_t W, int32_t H, const float* P, const float* M);
+/* More views than one vc_set_views takes: appends views [V, V+n) of the engine's W x H geometry, up to VC_MAX_TOTAL_VIEWS in all.
+ * P (and M) hold n*12 floats as in vc_set_views; M must be given if and only if the engine's views have M.  masks: the n new
+ * masks in a format of vc_set_masks (VC_MASK_BITS also takes a DEVICE pointer; VC_MASK_BGR8_RAW needs vc_set_calibration, and
+ * then images_bgr are raw too, undistorted on the device).  images_bgr: the n new 8UC3 images, required if and only if the
+ * engine holds images (vc_set_images / vc_set_images_raw).  Only the new views' summed-area tables are built; the masks, tables
+ * and images of the earlier views, the volumes, colour records, mesh and .off text stay as they were, so a capture can grow
+ * while the volumes stay on the device: carve just the new frames onto them with vc_carve(e, mode, V_old, -1, 0).
+ * Views are processed in groups of 256 consecutive views (one constant-memory batch each); carving is order-independent, and
+ * vc_color makes one pass over all views in order, so every result equals that of one engine holding all views at once.
+ * VC_ERR_STATE before vc_set_views + vc_set_masks, or for raw masks without calibration; VC_ERR_ARG for n < 1, V+n above
+ * VC_MAX_TOTAL_VIEWS, (V+n)*H*ceil(W/32) >= 2^31 mask words, or an M / images_bgr that does not match the engine.  Every check
+ * runs and every buffer is allocated before any state changes: a refused call (a failed allocation too) leaves the engine as
+ * it was. */
+#define VC_MAX_TOTAL_VIEWS 4096
+VC_EXPORT int vc_append_views(vc_engine* e, int32_t n, const float* P, const float* M, const void* masks, int32_t mask_format,
+                              const uint8_t* images_bgr);
+/* vc_set_masks, vc_set_images, vc_set_images_raw, vc_download_masks and vc_download_images take or deliver all V views of the
+ * engine, also more than 256 after vc_append_views. */
 /* Undistorted silhouette masks (VoxelCarving.cpp:36). VC_MASK_BITS: uint32[V][H][ceil(W/32)],
  * bit x&31 of word x>>5, 1 = background (pixel == (0,0,0), VoxelCarving.cpp:50).
  * VC_MASK_BGR8: the 8UC3 images themselves, uint8[V][H][W][3]; packed on the device. HOST memory (VC_MASK_BITS also takes a
@@ -160,7 +180,9 @@ VC_EXPORT int vc_carve_download(vc_engine* e, int32_t mode, uint32_t* occupied, 
  * pageable buffers the call degrades to the plain carve + two downloads.) */
 /* carve() over all views of a FRESH Model (vc_reset pending) + download of the result in SPARSE form: after a fresh carve
  * most 32x8x8-voxel bricks are uniform (C4: 96 %) and one flag byte says everything about them; only the bricks the engine
- * evaluated voxel by voxel need their words.  C4: 0.5 MB + 10 MB over PCIe instead of 268 MB.
+ * evaluated voxel by voxel need their words.  C4: 0.5 MB + 10 MB over PCIe instead of 268 MB.  With more than 256 views no
+ * single classification pass describes the result: the flags are then derived from the carved volumes, and the listed bricks
+ * are exactly those that are neither carved whole nor untouched with uniform seen (in no particular order).
  *   brick_flags[b], b = bx + nbx*(by + nby*bz) (vc_sparse_dims; brick = voxels [32bx, 32bx+32) x [8by, 8by+8) x slab planes
  *     [8bz, 8bz+8)): bit 0 (1) = every voxel carved (occupied 0, seen 1), bit 1 (2) = every voxel seen, bit 3 (8) = listed;
  *     a brick that is neither carved nor listed is untouched (occupied 1), one that is not listed has seen = bit 1.
@@ -182,8 +204,8 @@ VC_EXPORT int vc_mc_classify(vc_engine* e);
 
 /* ---- multi-GPU plumbing ---------------------------------------------------------- */
 /* Balanced contiguous z-slabs for n_parts GPUs.  Runs only the two brick-classification passes of VC_EXACT over this
- * engine's z-range (needs views + masks, allocates no volumes), takes the per-voxel work left per layer of 8 planes
- * (undecided views x voxels of the listed bricks) and returns n_parts+1 boundaries (interior ones multiples of 8 planes
+ * engine's z-range (needs views + masks, allocates no volumes; with more than 256 views once per group of 256, the costs summed),
+ * takes the per-voxel work left per layer of 8 planes (undecided views x voxels of the listed bricks) and returns n_parts+1 boundaries (interior ones multiples of 8 planes
  * from z_begin) with z_bounds[0] = z_begin, z_bounds[n_parts] = z_end.
  * Deterministic: every rank computes the same split from the same inputs. */
 VC_EXPORT int vc_plan_slabs(vc_engine* e, int32_t n_parts, int32_t* z_bounds);

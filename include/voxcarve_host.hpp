@@ -79,17 +79,24 @@ class Engine {
     Engine(const Engine&) = delete;
     Engine& operator=(const Engine&) = delete;
 
+    // all V views of the cache, up to VC_MAX_TOTAL_VIEWS: vc_set_views takes the first 256, vc_append_views the rest
     void setViews(const ViewCache& c, bool with_images) {
         if ((int)c.P.size() != c.V * 12) throw Error(VC_ERR_ARG, "ViewCache.P must hold V*12 floats");
-        check(vc_set_views(h_, c.V, c.W, c.H, c.P.data(), c.M.empty() ? nullptr : c.M.data()));
+        if (c.V > VC_MAX_TOTAL_VIEWS) throw Error(VC_ERR_ARG, "ViewCache holds " + std::to_string(c.V) + " views, more than VC_MAX_TOTAL_VIEWS");
+        if (with_images && c.images_bgr.empty()) throw Error(VC_ERR_ARG, "colour reconstruction needs ViewCache.images_bgr");
+        const int k = std::min(c.V, 256);
+        check(vc_set_views(h_, k, c.W, c.H, c.P.data(), c.M.empty() ? nullptr : c.M.data()));
         if (c.raw) check(vc_set_calibration(h_, c.K, c.dist.data(), (int32_t)c.dist.size()));
         if (!c.mask_bits.empty()) check(vc_set_masks(h_, c.mask_bits.data(), VC_MASK_BITS));
         else if (!c.mask_bgr.empty()) check(vc_set_masks(h_, c.mask_bgr.data(), c.raw ? VC_MASK_BGR8_RAW : VC_MASK_BGR8));
-        if (with_images) {
-            if (c.images_bgr.empty()) throw Error(VC_ERR_ARG, "colour reconstruction needs ViewCache.images_bgr");
-            check(c.raw ? vc_set_images_raw(h_, c.images_bgr.data()) : vc_set_images(h_, c.images_bgr.data()));
-        }
+        if (with_images) check(c.raw ? vc_set_images_raw(h_, c.images_bgr.data()) : vc_set_images(h_, c.images_bgr.data()));
+        if (c.V > k) append(c, k, c.V, with_images);
         check(vc_synchronize(h_));  // the cache may be a temporary
+    }
+    // every view of `c` after the engine's current ones (same W x H; masks, M, raw-ness and images as the engine's own views)
+    void appendViews(const ViewCache& c, bool with_images) {
+        if ((int)c.P.size() != c.V * 12) throw Error(VC_ERR_ARG, "ViewCache.P must hold V*12 floats");
+        append(c, 0, c.V, with_images);
     }
     void reset() { check(vc_reset(h_)); }
     void carve(int mode = VC_EXACT, int v0 = 0, int v1 = -1) { check(vc_carve(h_, mode, v0, v1, 0)); }
@@ -204,6 +211,14 @@ class Engine {
 
    private:
     void check(int rc) { if (rc != VC_OK) throw Error(rc, vc_last_error(h_)); }
+    void append(const ViewCache& c, int v0, int v1, bool with_images) {
+        const size_t bgr = (size_t)c.H * c.W * 3, words = (size_t)c.H * ((c.W + 31) / 32);
+        if (with_images && c.images_bgr.empty()) throw Error(VC_ERR_ARG, "colour reconstruction needs ViewCache.images_bgr");
+        const void* masks = !c.mask_bits.empty() ? (const void*)(c.mask_bits.data() + v0 * words) : (const void*)(c.mask_bgr.data() + v0 * bgr);
+        const int fmt = !c.mask_bits.empty() ? VC_MASK_BITS : (c.raw ? VC_MASK_BGR8_RAW : VC_MASK_BGR8);
+        check(vc_append_views(h_, v1 - v0, c.P.data() + (size_t)v0 * 12, c.M.empty() ? nullptr : c.M.data() + (size_t)v0 * 12, masks, fmt,
+                              with_images ? c.images_bgr.data() + v0 * bgr : nullptr));
+    }
     vc_engine* h_ = nullptr;
     uint64_t words_ = 0;
     int X_, Y_, Z_;
