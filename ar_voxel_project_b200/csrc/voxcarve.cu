@@ -47,7 +47,7 @@ static cudaError_t undistort_device(const uint8_t* d_src, uint8_t* d_dst, int n,
 struct CarveGraphKey {
     VcCarveParams p;
     const void* ptrs[10];
-    int fresh, sm_count, nbx_pad;
+    int fresh, sm_count;
 };
 struct CarveGraphSlot {
     cudaGraphExec_t exec = nullptr;
@@ -382,39 +382,6 @@ VcVolView vol_view(const vc_engine* e) {
         g.base = e->occ_slab() - (long long)lo * e->plane_words; g.cz0 = e->g.z_begin - lo; g.cz1 = e->g.z_end + hi;
     }
     return g;
-}
-
-// pin the silhouette set in L2 for the carve launches (access-policy window on the stream)
-void set_mask_window(vc_engine* e, bool on) {
-    cudaStreamAttrValue a{};
-    int dev = e->g.device, max_win = 0, persist_max = 0;
-    cudaDeviceGetAttribute(&max_win, cudaDevAttrMaxAccessPolicyWindowSize, dev);
-    cudaDeviceGetAttribute(&persist_max, cudaDevAttrMaxPersistingL2CacheSize, dev);
-    if (max_win <= 0 || persist_max <= 0 || !e->d_mask) { e->stats.l2_persist_bytes = 0; return; }
-    size_t bytes = e->mask_bytes < (size_t)max_win ? e->mask_bytes : (size_t)max_win;
-    // Off unless VOXCARVE_L2_PERSIST_MB=<cap in MB> asks for it.  Measured on B200: the silhouettes stay L2-resident on their
-    // own (C4, 18.7 MB: 0.50 ms with and without the window), and a large persisting carve-out starves everything else -
-    // C5 (74.6 MB of masks): 4.81 ms with the full window, 3.07 ms capped at 48 MB, 2.36 ms at 24 MB, 2.06 ms without.
-    const char* cap = getenv("VOXCARVE_L2_PERSIST_MB");
-    const long cap_mb = cap ? atol(cap) : 0;
-    if (cap_mb <= 0) { e->stats.l2_persist_bytes = 0; return; }
-    if ((size_t)cap_mb << 20 < (size_t)persist_max) persist_max = (int)((size_t)cap_mb << 20);
-    if (on) {
-        size_t carve_out = bytes < (size_t)persist_max ? bytes : (size_t)persist_max;
-        cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, carve_out);
-        a.accessPolicyWindow.base_ptr = e->d_mask;
-        a.accessPolicyWindow.num_bytes = bytes;
-        a.accessPolicyWindow.hitRatio = bytes <= carve_out ? 1.0f : (float)carve_out / (float)bytes;
-        a.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        a.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-        e->stats.l2_persist_bytes = carve_out;
-    } else {
-        a.accessPolicyWindow.num_bytes = 0;
-    }
-    if (cudaStreamSetAttribute(e->stream, cudaStreamAttributeAccessPolicyWindow, &a) != cudaSuccess) {
-        cudaGetLastError();
-        e->stats.l2_persist_bytes = 0;
-    }
 }
 
 // launch with programmatic stream serialization: the kernel may begin while the previous kernel of the stream drains (it
@@ -975,13 +942,26 @@ int vc_reset(vc_engine* e) {
     return VC_OK;
 }
 
+// The brick grid of `nz` planes of the slab (bricks of VC_BX x VC_BY x VC_BZ voxels, VC_BX = 32: one brick per word column)
+// and the super-brick grid over it (VC_SUPER^3 bricks each)
+struct BrickGeom {
+    int nbx, nby, nbz, sbx, sby, sbz;
+    long long n_bricks, n_super;
+};
+static BrickGeom brick_geom(const vc_engine* e, int nz) {
+    BrickGeom b;
+    b.nbx = e->Wx; b.nby = (e->g.Y + VC_BY - 1) / VC_BY; b.nbz = (nz + VC_BZ - 1) / VC_BZ;
+    b.sbx = (b.nbx + VC_SUPER - 1) / VC_SUPER; b.sby = (b.nby + VC_SUPER - 1) / VC_SUPER; b.sbz = (b.nbz + VC_SUPER - 1) / VC_SUPER;
+    b.n_bricks = (long long)b.nbx * b.nby * b.nbz;
+    b.n_super = (long long)b.sbx * b.sby * b.sbz;
+    return b;
+}
+
 // Buffers of the brick classifier, sized for the whole slab (a z-chunk uses a prefix of each).
 static int ensure_brick_buffers(vc_engine* e) {
-    const int nbx = e->Wx, nby = (e->g.Y + VC_BY - 1) / VC_BY, nbz = (e->nz + VC_BZ - 1) / VC_BZ;
-    const long long n_bricks = (long long)nbx * nby * nbz;
-    if (n_bricks > 0x7fffffffLL) return fail(e, VC_ERR_ARG, "slab too large for one launch (%lld bricks)", n_bricks);
-    const int sbx = (nbx + VC_SUPER - 1) / VC_SUPER, sby = (nby + VC_SUPER - 1) / VC_SUPER, sbz = (nbz + VC_SUPER - 1) / VC_SUPER + 1;
-    const long long n_super = (long long)sbx * sby * sbz;
+    const BrickGeom b = brick_geom(e, e->nz);
+    if (b.n_bricks > 0x7fffffffLL) return fail(e, VC_ERR_ARG, "slab too large for one launch (%lld bricks)", b.n_bricks);
+    const long long n_super = (long long)b.sbx * b.sby * (b.sbz + 1);
     if (e->resident_blocks < 1) {  // persistent grid of vc_carve_bricks: as many blocks of 8 warps as are resident at once
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&e->resident_blocks, vc_carve_bricks<false>, 256, 0) != cudaSuccess || e->resident_blocks < 1) { cudaGetLastError(); e->resident_blocks = 2; }
     }
@@ -991,9 +971,9 @@ static int ensure_brick_buffers(vc_engine* e) {
         VC_CUDA(e, cudaEventCreateWithFlags(&e->ev_fill_join, cudaEventDisableTiming));
     }
     if (e->d_bricks) return VC_OK;
-    VC_CUDA(e, cudaMalloc(&e->d_bricks, (size_t)n_bricks * sizeof(VcBrickState)));
+    VC_CUDA(e, cudaMalloc(&e->d_bricks, (size_t)b.n_bricks * sizeof(VcBrickState)));
     VC_CUDA(e, cudaMalloc(&e->d_super, (size_t)n_super * sizeof(VcBrickState)));
-    VC_CUDA(e, cudaMalloc(&e->d_brick_flags, (size_t)n_bricks));
+    VC_CUDA(e, cudaMalloc(&e->d_brick_flags, (size_t)b.n_bricks));
     VC_CUDA(e, cudaMalloc(&e->d_super_flags, (size_t)n_super));
     VC_CUDA(e, cudaMalloc(&e->d_super_list, (size_t)n_super * sizeof(unsigned int)));
     return VC_OK;
@@ -1030,36 +1010,49 @@ static void group_span(const vc_engine* e, int v0, int v1, int& g0, int& g1) {
     g1 = v1 > v0 ? (v1 - 1) / VC_MAX_VIEWS : g0;
 }
 
-static bool blind_fill_enabled() {  // VOXCARVE_BLIND_FILL=0: the r1 scheme (flag-driven fill by the first blocks of vc_carve_bricks), for comparison
-    static const bool off = [] { const char* v = getenv("VOXCARVE_BLIND_FILL"); return v && v[0] == '0'; }();
-    return !off;
+// Both levels of the brick classifier on the planes [z_begin, z_begin + nz) of the grid (geometry b), for the views [v0, v1) of
+// the group whose tables start at view vbase: the list lengths are reset, the super-bricks classified into the dense array,
+// then the bricks of the undecided ones into the flags and the work list.  executed: the corner-projection counter of a
+// counting run, or null.  pdl: level 0 may start while level 1 drains.
+static int classify_bricks(vc_engine* e, const BrickGeom& b, int z_begin, int nz, int v0, int v1, int vbase, unsigned long long* executed, bool pdl) {
+    unsigned int* d_nlist = (unsigned int*)(e->d_scalars + 6);  // [6] = front list length | super-list length, [7] = work counter | back list length
+    VC_CUDA(e, cudaMemsetAsync(e->d_scalars + 6, 0, 2 * sizeof(unsigned long long), e->stream));
+    VcBrickParams bp{};
+    bp.list = e->d_bricks; bp.n_list = d_nlist; bp.n_list_back = d_nlist + 3; bp.list_cap = (unsigned)b.n_bricks;
+    bp.brick_flags = e->d_brick_flags; bp.sat = e->d_sat + (size_t)vbase * (e->H + 1) * vc_sat_pitch(e->W);
+    bp.super_flags = e->d_super_flags; bp.super_list = e->d_super_list; bp.n_super_list = d_nlist + 1;
+    bp.executed = executed;
+    bp.X = e->g.X; bp.Y = e->g.Y; bp.Wx = e->Wx; bp.nz = nz; bp.z_begin = z_begin;
+    bp.nbx = b.nbx; bp.nby = b.nby; bp.nbz = b.nbz; bp.W = e->W; bp.H = e->H; bp.v0 = v0; bp.v1 = v1; bp.s = e->g.voxel_size;
+    VcBrickParams sp = bp;  // level 1: super-bricks into the dense array
+    sp.dense = e->d_super; sp.nbx = b.sbx; sp.nby = b.sby; sp.nbz = b.sbz;
+    vc_brick_classify_kernel<1><<<(unsigned)((b.n_super + VC_CLS_L1_CH - 1) / VC_CLS_L1_CH), 256, 0, e->stream>>>(sp);  // VC_CLS_L1_CH super-bricks per block
+    bp.dense = e->d_super; bp.pbx = b.sbx; bp.pby = b.sby;
+    // level 0: the blocks walk the list of undecided super-bricks (length known on the device only)
+    const long long l0_grid = std::min<long long>(b.n_super, 8LL * e->sm_count);
+    VC_CUDA(e, launch_pdl(vc_brick_classify_kernel<0>, dim3((unsigned)l0_grid), dim3(VC_CLS_L0_THREADS), e->stream, pdl, bp));
+    return VC_OK;
 }
 
 // VC_EXACT on the planes [zl0, zl1) of the slab (zl0 a multiple of the super-brick height, so bricks sit where they
 // would in a whole-slab pass): classify super-bricks, classify bricks, fill, evaluate the undecided pairs.  vbase: first view
 // of the group whose constants are loaded (p from group_params); the per-view device arrays are read from there.
-static int carve_exact_range(vc_engine* e, VcCarveParams p, int zl0, int zl1, bool count, bool fresh, bool record_mid, uint64_t* n_bricks_out,
-                             int vbase = 0) {
-    const vc_sat_t* sat = e->d_sat + (size_t)vbase * (e->H + 1) * vc_sat_pitch(e->W);
+static int carve_exact_range(vc_engine* e, VcCarveParams p, int zl0, int zl1, bool count, bool fresh, bool record_mid, int vbase = 0) {
     const long long off = (long long)zl0 * e->plane_words;
     p.occ += off; p.seen += off;
     p.z_begin = e->g.z_begin + zl0; p.nz = zl1 - zl0;
-    const int nbx = e->Wx, nby = (e->g.Y + VC_BY - 1) / VC_BY, nbz = (p.nz + VC_BZ - 1) / VC_BZ;
-    const long long n_bricks = (long long)nbx * nby * nbz;
-    const int sbx = (nbx + VC_SUPER - 1) / VC_SUPER, sby = (nby + VC_SUPER - 1) / VC_SUPER, sbz = (nbz + VC_SUPER - 1) / VC_SUPER;
-    const long long n_super = (long long)sbx * sby * sbz;
+    const BrickGeom b = brick_geom(e, p.nz);
     if (p.nz > 65535) return fail(e, VC_ERR_ARG, "vc_carve: slab of %d planes exceeds the fill grid", p.nz);
-    unsigned int* d_nlist = (unsigned int*)(e->d_scalars + 6);   // [6] = front list length | super-list length, [7] = work counter | back list length
     unsigned int* d_work = (unsigned int*)(e->d_scalars + 7);
+    const bool quads = e->Wx % 4 == 0;
+    const unsigned Q = (unsigned)e->Wx / 4u;  // quads per row
+    int q_shift = -1;                         // log2(Q) when the rows are whole quads and Q is a power of two
+    if (quads) for (int k = 0; k < 31; k++) if (Q == (1u << k)) q_shift = k;
     // Fresh carve: most words end up "carved and seen".  That pattern is written everywhere first, by a kernel that needs nothing
     // from the classification and runs next to it on a second stream (a fork / join the graph capture follows); the fill pass
     // inside vc_carve_bricks then only writes the words of bricks that are neither carved nor listed.
-    const bool blind = fresh && e->Wx % 4 == 0 && blind_fill_enabled();
     bool fill_forked = false;
-    if (blind) {
-        const unsigned Q = (unsigned)e->Wx / 4u;
-        int q_shift = -1;
-        for (int b = 0; b < 31; b++) if (Q == (1u << b)) q_shift = b;
+    if (fresh && quads) {
         const int rem = e->g.X - (e->Wx - 1) * 32;
         const size_t n_quads = (size_t)p.nz * e->g.Y * Q;
         // As a branch of the captured graph it runs next to the classification.  Plain launches (profiling mode, VOXCARVE_NO_GRAPH,
@@ -1078,74 +1071,87 @@ static int carve_exact_range(vc_engine* e, VcCarveParams p, int zl0, int zl1, bo
         vc_blind_fill_kernel<<<bgrid, 256, 0, fs>>>((uint4*)p.occ, (uint4*)p.seen, n_quads, Q, q_shift, rem >= 32 ? 0xffffffffu : ((1u << rem) - 1u));
         VC_CUDA(e, cudaGetLastError());
         if (fill_forked) VC_CUDA(e, cudaEventRecord(e->ev_fill_join, e->fill_stream));
-        e->stats.carve_launches += 1;
     }
-    VC_CUDA(e, cudaMemsetAsync(e->d_scalars + 6, 0, 2 * sizeof(unsigned long long), e->stream));
-    VcBrickParams bp{};
-    bp.list = e->d_bricks; bp.n_list = d_nlist; bp.n_list_back = d_work + 1; bp.list_cap = (unsigned)n_bricks;
-    bp.brick_flags = e->d_brick_flags; bp.sat = sat;
-    bp.super_flags = e->d_super_flags; bp.super_list = e->d_super_list; bp.n_super_list = d_nlist + 1;
-    bp.executed = count ? e->d_scalars + 5 : nullptr;
-    bp.X = e->g.X; bp.Y = e->g.Y; bp.Wx = e->Wx; bp.nz = p.nz; bp.z_begin = p.z_begin;
-    bp.nbx = nbx; bp.nby = nby; bp.nbz = nbz; bp.W = e->W; bp.H = e->H; bp.v0 = p.v0; bp.v1 = p.v1; bp.s = e->g.voxel_size;
-    VcBrickParams sp = bp;  // level 1: super-bricks into the dense array
-    sp.dense = e->d_super; sp.nbx = sbx; sp.nby = sby; sp.nbz = sbz;
-    vc_brick_classify_kernel<1><<<(unsigned)((n_super + VC_CLS_L1_CH - 1) / VC_CLS_L1_CH), 256, 0, e->stream>>>(sp);  // VC_CLS_L1_CH super-bricks per block
-    bp.dense = e->d_super; bp.pbx = sbx; bp.pby = sby;
-    const bool pdl = !record_mid;  // an event record between two kernels would keep them from overlapping anyway
-    {   // level 0: the blocks walk the list of undecided super-bricks (length known on the device only)
-        const long long l0_grid = std::min<long long>(n_super, 8LL * e->sm_count);
-        VC_CUDA(e, launch_pdl(vc_brick_classify_kernel<0>, dim3((unsigned)l0_grid), dim3(VC_CLS_L0_THREADS), e->stream, pdl, bp));
-    }
+    // level 0 overlaps level 1 unless the mid-point event is recorded: an event record would keep the kernels apart anyway
+    int rc =classify_bricks(e, b, p.z_begin, p.nz, p.v0, p.v1, vbase, count ? e->d_scalars + 5 : nullptr, !record_mid);
+    if (rc) return rc;
     if (record_mid) VC_CUDA(e, cudaEventRecord(e->evm, e->stream));  // (profiling / counting runs only: it sits between two kernels that otherwise overlap their launch)
-    if (e->resident_blocks < 1) {  // persistent grid: as many blocks of 8 warps as are resident at once
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&e->resident_blocks, vc_carve_bricks<false>, 256, 0) != cudaSuccess || e->resident_blocks < 1) { cudaGetLastError(); e->resident_blocks = 2; }
-    }
-    const int resident = e->resident_blocks;
-    const unsigned pgrid = (unsigned)e->sm_count * (unsigned)resident;
+    const unsigned pgrid = (unsigned)e->sm_count * (unsigned)e->resident_blocks;  // persistent grid (ensure_brick_buffers)
     // Fill pass (volume words implied by the brick flags).  Fresh carve, rows of whole quads: the first blocks of the persistent
-    // kernel do it themselves, skipping the listed bricks, whose words the work items own.  Otherwise it runs first, in
-    // stream order (it must apply the flags before the per-voxel kernel reads the state; rows of other widths go word by word).
+    // kernel patch what the blind fill got wrong, skipping the listed bricks, whose words the work items own.  Otherwise it runs
+    // first, in stream order (it must apply the flags before the per-voxel kernel reads the state; rows of other widths go word
+    // by word).
     VcFillParams fp{};
     fp.occ = p.occ; fp.seen = p.seen; fp.brick_flags = e->d_brick_flags; fp.super_flags = e->d_super_flags;
-    fp.X = e->g.X; fp.Y = e->g.Y; fp.Wx = e->Wx; fp.nby = nby; fp.pbx = sbx; fp.pby = sby;
-    fp.fresh = fresh ? 1 : 0; fp.skip_listed = fresh ? 1 : 0; fp.nz = p.nz; fp.q_shift = -1; fp.n_fill_blocks = 0;
-    fp.blind = blind ? 1 : 0;
+    fp.X = e->g.X; fp.Y = e->g.Y; fp.Wx = e->Wx; fp.nby = b.nby; fp.pbx = b.sbx; fp.pby = b.sby;
+    fp.nz = p.nz; fp.q_shift = q_shift; fp.n_fill_blocks = 0;
     if (fill_forked) VC_CUDA(e, cudaStreamWaitEvent(e->stream, e->ev_fill_join, 0));  // before anything else writes the volumes
-    const bool quads = e->Wx % 4 == 0;
-    if (quads) {
-        const unsigned Q = (unsigned)e->Wx / 4u;
-        for (int b = 0; b < 31; b++) if (Q == (1u << b)) fp.q_shift = b;
-        fp.per_plane = (unsigned)(((long long)e->g.Y * Q + 255) / 256);
-    }
+    if (quads) fp.per_plane = (unsigned)(((long long)e->g.Y * Q + 255) / 256);
     if (fresh && quads) {
         // ONE fill block per SM (blocks are dealt round-robin).  More of them when the slab has many brick layers was the r1
         // heuristic; measured on C5 (256 layers): 1 / 2 / 3 / 4 fill blocks per SM = 1.90 / 1.96 / 1.99 / 2.02 ms - the kernel is
         // bound by its computing blocks, so the fill gets as few as keep the stores flowing.
-        const unsigned per_sm = 1;
-        fp.n_fill_blocks = (unsigned)e->sm_count * per_sm < pgrid ? (unsigned)e->sm_count * per_sm : pgrid;
+        fp.n_fill_blocks = std::min((unsigned)e->sm_count, pgrid);
     } else if (quads) {
-        vc_fill4_kernel<<<dim3(fp.per_plane, (unsigned)nbz), 256, 0, e->stream>>>(fp);  // one block per (256 quads, brick layer)
+        vc_fill4_kernel<<<dim3(fp.per_plane, (unsigned)b.nbz), 256, 0, e->stream>>>(fp);  // one block per (256 quads, brick layer)
     } else {
         vc_fill_kernel<<<dim3((e->g.Y + 7) / 8, p.nz, (e->Wx + 31) / 32), dim3(32, 8), 0, e->stream>>>(
-            p.occ, p.seen, e->d_brick_flags, e->d_super_flags, e->g.X, e->g.Y, e->Wx, nby, sbx, sby, fresh ? 1 : 0, 0);
+            p.occ, p.seen, e->d_brick_flags, e->d_super_flags, e->g.X, e->g.Y, e->Wx, b.nby, b.sbx, b.sby, fresh ? 1 : 0, 0);
     }
     // The per-voxel kernel is launched plainly, onto an empty GPU.  Its fill pass relies on the first blocks of the grid landing
     // on different SMs (one fill block per SM, HBM-bound, next to three computing blocks); as a programmatic dependent launch
     // its blocks take whatever slots the classification frees first, the fill blocks pile up on a few SMs, and slabs that are
     // mostly fill get 30 % slower (C5, slab 0 of 8: 0.30 -> 0.39 ms).  Only the level-0 classification overlaps its predecessor.
-    const bool pdl_cb = false;
-    (void)pdl;
-    const VcBrickState* list_c = e->d_bricks;
-    const unsigned int *n_front_c = d_nlist, *n_back_c = d_work + 1;
-    const vc_sat_t* sat_c = sat;
-    const VcViewFilter* filt_c = e->d_filt + vbase;
-    const VcViewConst* view_c = e->d_view64 + vbase;
-    if (count) VC_CUDA(e, launch_pdl(vc_carve_bricks<true>, dim3(pgrid), dim3(256), e->stream, pdl_cb, p, list_c, n_front_c, n_back_c, (unsigned)n_bricks, d_work, nbx, nby, sat_c, fresh ? 1 : 0, filt_c, view_c, fp));
-    else VC_CUDA(e, launch_pdl(vc_carve_bricks<false>, dim3(pgrid), dim3(256), e->stream, pdl_cb, p, list_c, n_front_c, n_back_c, (unsigned)n_bricks, d_work, nbx, nby, sat_c, fresh ? 1 : 0, filt_c, view_c, fp));
+    const unsigned int* d_nlist = (const unsigned int*)(e->d_scalars + 6);
+    const vc_sat_t* sat = e->d_sat + (size_t)vbase * (e->H + 1) * vc_sat_pitch(e->W);
+    if (count) vc_carve_bricks<true><<<pgrid, 256, 0, e->stream>>>(p, e->d_bricks, d_nlist, d_work + 1, (unsigned)b.n_bricks, d_work, b.nbx, b.nby, sat, fresh ? 1 : 0, e->d_filt + vbase, e->d_view64 + vbase, fp);
+    else vc_carve_bricks<false><<<pgrid, 256, 0, e->stream>>>(p, e->d_bricks, d_nlist, d_work + 1, (unsigned)b.n_bricks, d_work, b.nbx, b.nby, sat, fresh ? 1 : 0, e->d_filt + vbase, e->d_view64 + vbase, fp);
     VC_CUDA(e, cudaGetLastError());
-    e->stats.carve_launches += (fresh && quads) ? 3 : 4;
-    if (n_bricks_out) *n_bricks_out += (uint64_t)n_bricks;
+    e->stats.carve_launches += 4;  // blind fill or fill pass, two classification levels, per-voxel kernel
+    return VC_OK;
+}
+
+// One carve of the views [v0, v1) on the planes [zl0, zl1) of the slab, view group by view group: each group's constants are
+// uploaded in stream order behind the previous group's kernels, and only the first group starts from a pending reset (`fresh`);
+// the others accumulate onto its result.  With one group (at most VC_MAX_VIEWS views) this is one plain sequence.  Counting
+// runs of VC_EXACT add the bricks each group listed for per-voxel work to *listed.
+static int carve_groups(vc_engine* e, int32_t mode, const VcCarveParams& p, int v0, int v1, int zl0, int zl1, bool count, bool fresh,
+                        bool record_mid, uint64_t* listed) {
+    int g0, g1;
+    group_span(e, v0, v1, g0, g1);
+    for (int g = g0; g <= g1; g++) {
+        int rc = ensure_constants(e, g);
+        if (rc) return rc;
+        const VcCarveParams pg = group_params(e, p, g, v0, v1);
+        if (mode == VC_EXACT) rc = carve_exact_range(e, pg, zl0, zl1, count, fresh && g == g0, record_mid, g * VC_MAX_VIEWS);
+        else rc = launch_carve<4>(e, mode == VC_EXACT_FLAT ? VC_EXACT : mode, pg, count);
+        if (rc) return rc;
+        if (count && mode == VC_EXACT) {  // the next group resets the list lengths
+            unsigned long long nl = 0, nw = 0;
+            VC_CUDA(e, cudaMemcpyAsync(&nl, e->d_scalars + 6, sizeof nl, cudaMemcpyDeviceToHost, e->stream));
+            VC_CUDA(e, cudaMemcpyAsync(&nw, e->d_scalars + 7, sizeof nw, cudaMemcpyDeviceToHost, e->stream));
+            VC_CUDA(e, cudaStreamSynchronize(e->stream));
+            *listed += (nl & 0xffffffffull) + (nw >> 32);  // front + back of the work list
+        }
+    }
+    return VC_OK;
+}
+
+// after the last kernel of a carve (vc_carve, vc_carve_download): its end event, the view constants released, the per-call
+// statistics reset, and everything derived from the volumes marked stale
+static int carve_finish(vc_engine* e, uint64_t nominal_voxel_views) {
+    VC_CUDA(e, cudaEventRecord(e->ev1, e->stream));
+    int rc = constants_used(e);
+    if (rc) return rc;
+    e->stats.nominal_voxel_views = nominal_voxel_views;
+    e->stats.executed_voxel_views = 0;
+    e->stats.brick_corner_views = 0;
+    e->stats.filter_rows = e->stats.filter_slow_rows = e->stats.filter_mismatches = e->stats.subbrick_corner_views = 0;
+    e->stats.last_carve_ms = -1.0;  // resolved lazily in vc_get_stats
+    e->gathered = false;
+    e->halo_lo = e->halo_hi = false;  // the neighbours carve too: their planes are stale
+    e->have_colors = false;
+    e->have_mc = false;
     return VC_OK;
 }
 
@@ -1192,126 +1198,67 @@ int vc_carve(vc_engine* e, int32_t mode, int32_t view_begin, int32_t view_end, i
         vc_unseen_begin_kernel<<<(unsigned)((e->slab_words + 255) / 256), 256, 0, e->stream>>>(e->occ_slab(), e->seen_slab(), d_saved_occ, e->slab_words, e->Wx, e->g.X);
         VC_CUDA(e, cudaGetLastError());
     }
-    set_mask_window(e, true);
     VC_CUDA(e, cudaEventRecord(e->ev0, e->stream));
-    e->have_mid = mode == VC_EXACT;
-    e->stats.bricks_total = 0;
+    e->stats.bricks_total = mode == VC_EXACT ? (uint64_t)brick_geom(e, e->nz).n_bricks : 0;
     e->stats.bricks_listed = 0;
-    uint64_t listed_in_groups = 0;  // counting run over several view groups: listed bricks summed over the groups
-    if (mode == VC_EXACT) {
-        if (e->use_graphs < 0) { const char* ng = getenv("VOXCARVE_NO_GRAPH"); e->use_graphs = (ng && atoi(ng) != 0) ? 0 : 1; }
-        const bool fresh = e->reset_pending;
-        bool launched = false;
-        if (e->V > VC_MAX_VIEWS) {
-            // One plain sequence per view group, the constants of each uploaded in stream order behind the previous group's
-            // kernels; only the first group starts from a pending reset, the others accumulate onto its result.
-            int g0, g1;
-            group_span(e, view_begin, view_end, g0, g1);
-            for (int g = g0; g <= g1; g++) {
-                rc = ensure_constants(e, g);
-                if (rc) return rc;
-                uint64_t nb = 0;
-                rc = carve_exact_range(e, group_params(e, p, g, view_begin, view_end), 0, e->nz, count_executed != 0, fresh && g == g0, false,
-                                       &nb, g * VC_MAX_VIEWS);
-                if (rc) return rc;
-                e->stats.bricks_total = nb;
-                if (count_executed) {  // the next group resets the list lengths
-                    unsigned long long nl = 0, nw = 0;
-                    VC_CUDA(e, cudaMemcpyAsync(&nl, e->d_scalars + 6, sizeof nl, cudaMemcpyDeviceToHost, e->stream));
-                    VC_CUDA(e, cudaMemcpyAsync(&nw, e->d_scalars + 7, sizeof nw, cudaMemcpyDeviceToHost, e->stream));
-                    VC_CUDA(e, cudaStreamSynchronize(e->stream));
-                    listed_in_groups += (nl & 0xffffffffull) + (nw >> 32);
-                }
-            }
-            e->have_mid = false;
-            launched = true;
+    uint64_t listed = 0;  // counting run of VC_EXACT: listed bricks summed over the view groups
+    const bool fresh = mode == VC_EXACT && e->reset_pending;
+    if (mode == VC_EXACT && e->use_graphs < 0) { const char* ng = getenv("VOXCARVE_NO_GRAPH"); e->use_graphs = (ng && atoi(ng) != 0) ? 0 : 1; }
+    // a whole-range VC_EXACT carve of one view group (its constants uploaded by carve_check) is one cached CUDA graph
+    const bool graph = mode == VC_EXACT && e->use_graphs && !e->profiling && !count_executed && view_begin == 0 && view_end == e->V &&
+                       e->V <= VC_MAX_VIEWS;
+    e->have_mid = mode == VC_EXACT && !graph && e->V <= VC_MAX_VIEWS && (e->profiling || count_executed != 0);
+    if (graph) {
+        CarveGraphKey k;
+        memset(&k, 0, sizeof k);  // padding bytes too: the key is compared with memcmp
+        k.p = p;
+        const void* ptrs[10] = {e->d_bricks, e->d_super, e->d_brick_flags, e->d_super_flags, e->d_super_list, e->d_sat, e->d_filt, e->d_view64, e->d_scalars, e->evm};
+        memcpy(k.ptrs, ptrs, sizeof ptrs);
+        k.fresh = fresh ? 1 : 0; k.sm_count = e->sm_count;
+        CarveGraphSlot& gs = e->graph_slot[fresh ? 1 : 0];
+        bool captured_now = false;
+        if (!gs.valid || memcmp(&gs.key, &k, sizeof k) != 0) {
+            captured_now = true;
+            if (gs.exec) { cudaGraphExecDestroy(gs.exec); gs.exec = nullptr; }
+            gs.valid = false;
+            cudaGraph_t g = nullptr;
+            VC_CUDA(e, cudaStreamBeginCapture(e->stream, cudaStreamCaptureModeThreadLocal));
+            rc = carve_exact_range(e, p, 0, e->nz, false, fresh, false);
+            const cudaError_t ce = cudaStreamEndCapture(e->stream, &g);  // always end the capture, also after a failed launch
+            if (rc) { if (g) cudaGraphDestroy(g); return rc; }
+            if (ce != cudaSuccess) return fail(e, VC_ERR_CUDA, "vc_carve: stream capture failed: %s", cudaGetErrorString(ce));
+            const cudaError_t ci = cudaGraphInstantiate(&gs.exec, g, 0);
+            cudaGraphDestroy(g);
+            if (ci != cudaSuccess) { gs.exec = nullptr; return fail(e, VC_ERR_CUDA, "vc_carve: cudaGraphInstantiate failed: %s", cudaGetErrorString(ci)); }
+            gs.key = k;
+            gs.valid = true;
         }
-        if (!launched && e->use_graphs && !e->profiling && !count_executed && view_begin == 0 && view_end == e->V) {
-            CarveGraphKey k;
-            memset(&k, 0, sizeof k);  // padding bytes too: the key is compared with memcmp
-            k.p = p;
-            const void* ptrs[10] = {e->d_bricks, e->d_super, e->d_brick_flags, e->d_super_flags, e->d_super_list, e->d_sat, e->d_filt, e->d_view64, e->d_scalars, e->evm};
-            memcpy(k.ptrs, ptrs, sizeof ptrs);
-            k.fresh = fresh ? 1 : 0; k.sm_count = e->sm_count; k.nbx_pad = 0;
-            CarveGraphSlot& gs = e->graph_slot[fresh ? 1 : 0];
-            bool captured_now = false;
-            if (!gs.valid || memcmp(&gs.key, &k, sizeof k) != 0) {
-                captured_now = true;
-                if (gs.exec) { cudaGraphExecDestroy(gs.exec); gs.exec = nullptr; }
-                gs.valid = false;
-                cudaGraph_t graph = nullptr;
-                VC_CUDA(e, cudaStreamBeginCapture(e->stream, cudaStreamCaptureModeThreadLocal));
-                uint64_t nb_dummy = 0;
-                rc = carve_exact_range(e, p, 0, e->nz, false, fresh, false, &nb_dummy);
-                const cudaError_t ce = cudaStreamEndCapture(e->stream, &graph);  // always end the capture, also after a failed launch
-                if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
-                if (ce != cudaSuccess) return fail(e, VC_ERR_CUDA, "vc_carve: stream capture failed: %s", cudaGetErrorString(ce));
-                const cudaError_t ci = cudaGraphInstantiate(&gs.exec, graph, 0);
-                cudaGraphDestroy(graph);
-                if (ci != cudaSuccess) { gs.exec = nullptr; return fail(e, VC_ERR_CUDA, "vc_carve: cudaGraphInstantiate failed: %s", cudaGetErrorString(ci)); }
-                gs.key = k;
-                gs.valid = true;
-            }
-            VC_CUDA(e, cudaGraphLaunch(gs.exec, e->stream));
-            if (!captured_now) e->stats.carve_launches += (fresh && e->Wx % 4 == 0 && !blind_fill_enabled()) ? 3 : 4;  // the capture counted its own
-            const int nby = (e->g.Y + VC_BY - 1) / VC_BY, nbz = (e->nz + VC_BZ - 1) / VC_BZ;
-            e->stats.bricks_total = (uint64_t)e->Wx * nby * nbz;
-            e->have_mid = false;
-            launched = true;
-        }
-        if (!launched) {
-            e->have_mid = e->profiling || count_executed != 0;
-            rc = carve_exact_range(e, p, 0, e->nz, count_executed != 0, fresh, e->have_mid, &e->stats.bricks_total);
-            if (rc) return rc;
-        }
-        e->reset_pending = false;
-        // the flags of this call say everything about the volumes (with several groups, no single group's flags do)
-        e->flags_valid = fresh && view_begin == 0 && view_end == e->V && e->V <= VC_MAX_VIEWS;
-    } else if (e->V > VC_MAX_VIEWS) {
-        int g0, g1;
-        group_span(e, view_begin, view_end, g0, g1);
-        for (int g = g0; g <= g1; g++) {
-            rc = ensure_constants(e, g);
-            if (rc) return rc;
-            rc = launch_carve<4>(e, mode == VC_EXACT_FLAT ? VC_EXACT : mode, group_params(e, p, g, view_begin, view_end), count_executed != 0);
-            if (rc) return rc;
-        }
-        e->flags_valid = false;
+        VC_CUDA(e, cudaGraphLaunch(gs.exec, e->stream));
+        if (!captured_now) e->stats.carve_launches += 4;  // the capture counted its own
     } else {
-        rc = launch_carve<4>(e, mode == VC_EXACT_FLAT ? VC_EXACT : mode, p, count_executed != 0);
+        rc = carve_groups(e, mode, p, view_begin, view_end, 0, e->nz, count_executed != 0, fresh, e->have_mid, &listed);
         if (rc) return rc;
-        e->flags_valid = false;
     }
+    if (mode == VC_EXACT) e->reset_pending = false;
+    // the flags of a fresh whole-range VC_EXACT carve say everything about the volumes (with several groups, no single group's flags do)
+    e->flags_valid = fresh && view_begin == 0 && view_end == e->V && e->V <= VC_MAX_VIEWS;
     if (d_saved_occ) {
         vc_unseen_end_kernel<<<(unsigned)((e->slab_words + 255) / 256), 256, 0, e->stream>>>(e->occ_slab(), d_saved_occ, e->slab_words);
         VC_CUDA(e, cudaGetLastError());
     }
-    VC_CUDA(e, cudaEventRecord(e->ev1, e->stream));
-    rc = constants_used(e);
+    rc = carve_finish(e, (uint64_t)e->g.X * e->g.Y * e->nz * (uint64_t)(view_end - view_begin));
     if (rc) return rc;
-    set_mask_window(e, false);
-    e->stats.nominal_voxel_views = (uint64_t)e->g.X * e->g.Y * e->nz * (uint64_t)(view_end - view_begin);
-    e->stats.executed_voxel_views = 0;
-    e->stats.brick_corner_views = 0;
-    e->stats.filter_rows = e->stats.filter_slow_rows = e->stats.filter_mismatches = e->stats.subbrick_corner_views = 0;
-    e->stats.last_carve_ms = -1.0;  // resolved lazily in vc_get_stats
     if (count_executed) {
-        unsigned long long ex = 0, bc = 0, nl = 0, nw = 0, fl[4] = {0, 0, 0, 0};
+        unsigned long long ex = 0, bc = 0, fl[4] = {0, 0, 0, 0};
         VC_CUDA(e, cudaMemcpyAsync(fl, e->d_scalars + 8, sizeof fl, cudaMemcpyDeviceToHost, e->stream));
         VC_CUDA(e, cudaMemcpyAsync(&ex, e->d_scalars + 2, sizeof ex, cudaMemcpyDeviceToHost, e->stream));
         VC_CUDA(e, cudaMemcpyAsync(&bc, e->d_scalars + 5, sizeof bc, cudaMemcpyDeviceToHost, e->stream));
-        VC_CUDA(e, cudaMemcpyAsync(&nl, e->d_scalars + 6, sizeof nl, cudaMemcpyDeviceToHost, e->stream));
-        VC_CUDA(e, cudaMemcpyAsync(&nw, e->d_scalars + 7, sizeof nw, cudaMemcpyDeviceToHost, e->stream));
         VC_CUDA(e, cudaStreamSynchronize(e->stream));
-        e->stats.bricks_listed = mode != VC_EXACT ? 0 : e->V > VC_MAX_VIEWS ? listed_in_groups : (nl & 0xffffffffull) + (nw >> 32);  // front + back of the work list
+        e->stats.bricks_listed = listed;
         e->stats.executed_voxel_views = ex + (mode == VC_EXACT ? bc : 0);
         e->stats.brick_corner_views = mode == VC_EXACT ? bc : 0;
         if (mode == VC_EXACT) { e->stats.filter_rows = fl[0]; e->stats.filter_slow_rows = fl[1]; e->stats.filter_mismatches = fl[2]; e->stats.subbrick_corner_views = fl[3]; }
     }
-    e->gathered = false;
-    e->halo_lo = e->halo_hi = false;  // the neighbours carve too: their planes are stale
-    e->have_colors = false;
-    e->have_mc = false;
     return VC_OK;
 }
 
@@ -1344,28 +1291,16 @@ int vc_carve_download(vc_engine* e, int32_t mode, uint32_t* occupied, uint32_t* 
     }
     VcCarveParams p = carve_params(e, v0, v1);
     const int cz = ((e->nz + n_chunks - 1) / n_chunks + LZ - 1) / LZ * LZ;  // planes per chunk, a multiple of the super-brick height
-    set_mask_window(e, true);
     VC_CUDA(e, cudaEventRecord(e->ev0, e->stream));
     e->have_mid = false;
-    e->stats.bricks_total = 0;
+    e->stats.bricks_total = (uint64_t)brick_geom(e, e->nz).n_bricks;
     e->stats.bricks_listed = 0;
     const bool fresh = e->reset_pending;
     int c = 0;
     for (int zl0 = 0; zl0 < e->nz; zl0 += cz, c++) {
         const int zl1 = zl0 + cz < e->nz ? zl0 + cz : e->nz;
-        if (e->V <= VC_MAX_VIEWS) {
-            rc = carve_exact_range(e, p, zl0, zl1, false, fresh, false, &e->stats.bricks_total);
-            if (rc) return rc;
-        } else {
-            for (int g = 0; g < n_groups(e); g++) {  // the chunk's first group starts from the pending reset
-                rc = ensure_constants(e, g);
-                if (rc) return rc;
-                uint64_t nb = 0;
-                rc = carve_exact_range(e, group_params(e, p, g, v0, v1), zl0, zl1, false, fresh && g == 0, false, &nb, g * VC_MAX_VIEWS);
-                if (rc) return rc;
-                if (g == 0) e->stats.bricks_total += nb;
-            }
-        }
+        rc = carve_groups(e, VC_EXACT, p, v0, v1, zl0, zl1, false, fresh, false, nullptr);  // the chunk's first group starts from the pending reset
+        if (rc) return rc;
         VC_CUDA(e, cudaEventRecord(e->ev_chunk[c], e->stream));
         VC_CUDA(e, cudaStreamWaitEvent(e->copy_stream, e->ev_chunk[c], 0));
         const long long off = (long long)zl0 * e->plane_words, n = (long long)(zl1 - zl0) * e->plane_words;
@@ -1374,18 +1309,8 @@ int vc_carve_download(vc_engine* e, int32_t mode, uint32_t* occupied, uint32_t* 
     }
     e->reset_pending = false;
     e->flags_valid = false;  // the flag arrays were re-used chunk by chunk
-    VC_CUDA(e, cudaEventRecord(e->ev1, e->stream));
-    rc = constants_used(e);
+    rc = carve_finish(e, (uint64_t)e->g.X * e->g.Y * e->nz * (uint64_t)e->V);
     if (rc) return rc;
-    set_mask_window(e, false);
-    e->stats.nominal_voxel_views = (uint64_t)e->g.X * e->g.Y * e->nz * (uint64_t)e->V;
-    e->stats.executed_voxel_views = 0;
-    e->stats.brick_corner_views = 0;
-    e->stats.last_carve_ms = -1.0;
-    e->gathered = false;
-    e->halo_lo = e->halo_hi = false;
-    e->have_colors = false;
-    e->have_mc = false;
     VC_CUDA(e, cudaStreamSynchronize(e->copy_stream));
     VC_CUDA(e, cudaStreamSynchronize(e->stream));
     return VC_OK;
@@ -1396,9 +1321,8 @@ int vc_carve_download(vc_engine* e, int32_t mode, uint32_t* occupied, uint32_t* 
 // flags + 10 MB of words instead of 268 MB over PCIe.
 int vc_sparse_dims(const vc_engine* e, uint32_t* nbx, uint32_t* nby, uint32_t* nbz) {
     if (!e || !nbx || !nby || !nbz) return VC_ERR_ARG;
-    *nbx = (uint32_t)e->Wx;
-    *nby = (uint32_t)((e->g.Y + VC_BY - 1) / VC_BY);
-    *nbz = (uint32_t)((e->nz + VC_BZ - 1) / VC_BZ);
+    const BrickGeom b = brick_geom(e, e->nz);
+    *nbx = (uint32_t)b.nbx; *nby = (uint32_t)b.nby; *nbz = (uint32_t)b.nbz;
     return VC_OK;
 }
 
@@ -1408,23 +1332,22 @@ int vc_carve_download_sparse(vc_engine* e, uint8_t* brick_flags, uint64_t flags_
     PhaseRange nvtx("Carving");
     if (!brick_flags || !listed || !words || !n_listed) return fail(e, VC_ERR_ARG, "vc_carve_download_sparse: null argument");
     *n_listed = 0;
-    const int nbx = e->Wx, nby = (e->g.Y + VC_BY - 1) / VC_BY, nbz = (e->nz + VC_BZ - 1) / VC_BZ;
-    const long long n_bricks = (long long)nbx * nby * nbz;
+    const BrickGeom b = brick_geom(e, e->nz);
+    const long long n_bricks = b.n_bricks;
     if (flags_capacity < (uint64_t)n_bricks) return fail(e, VC_ERR_CAPACITY, "vc_carve_download_sparse: flag buffer holds %llu bytes, the slab has %lld bricks", (unsigned long long)flags_capacity, n_bricks);
     if (!e->reset_pending) return fail(e, VC_ERR_STATE, "vc_carve_download_sparse: describes a carve that starts from the Model constructor state: call vc_reset first");
     int rc = vc_carve(e, VC_EXACT, 0, -1, 0);
     if (rc) return rc;
-    const int sbx = (nbx + VC_SUPER - 1) / VC_SUPER, sby = (nby + VC_SUPER - 1) / VC_SUPER;
     void* sc = nullptr;
     rc = ensure_scratch(e, (size_t)n_bricks, &sc);  // resolved flags (the per-brick array is only written under undecided super-bricks)
     if (rc) return rc;
     uint8_t* d_flags = (uint8_t*)sc;
     if (e->V <= VC_MAX_VIEWS) {
-        vc_sparse_flags_kernel<<<(unsigned)((n_bricks + 255) / 256), 256, 0, e->stream>>>(e->d_brick_flags, e->d_super_flags, d_flags, nbx, nby, nbz, sbx, sby);
+        vc_sparse_flags_kernel<<<(unsigned)((n_bricks + 255) / 256), 256, 0, e->stream>>>(e->d_brick_flags, e->d_super_flags, d_flags, b.nbx, b.nby, b.nbz, b.sbx, b.sby);
     } else {  // several view groups: the flags and the list come from the volumes (the work list's front, its back left empty)
         VC_CUDA(e, cudaMemsetAsync(e->d_scalars + 6, 0, 2 * sizeof(unsigned long long), e->stream));
         vc_sparse_volume_flags_kernel<<<(unsigned)((n_bricks * 32 + 255) / 256), 256, 0, e->stream>>>(
-            e->occ_slab(), e->seen_slab(), d_flags, e->d_bricks, (unsigned int*)(e->d_scalars + 6), e->g.X, e->g.Y, e->nz, e->Wx, nbx, nby, nbz);
+            e->occ_slab(), e->seen_slab(), d_flags, e->d_bricks, (unsigned int*)(e->d_scalars + 6), e->g.X, e->g.Y, e->nz, e->Wx, b.nbx, b.nby, b.nbz);
     }
     VC_CUDA(e, cudaGetLastError());
     unsigned int counts[4] = {0, 0, 0, 0};  // front length, super-list length, work counter, back length
@@ -1442,7 +1365,7 @@ int vc_carve_download_sparse(vc_engine* e, uint8_t* brick_flags, uint64_t flags_
         e->sparse_cap = n;
     }
     vc_sparse_pack_kernel<<<(unsigned)((n + 3) / 4), 256, 0, e->stream>>>(e->d_bricks, counts[0], (unsigned)n, (unsigned)n_bricks, e->occ_slab(), e->seen_slab(),
-                                                                         e->g.Y, e->nz, e->Wx, nbx, nby, e->d_sparse_idx, e->d_sparse_words);
+                                                                         e->g.Y, e->nz, e->Wx, b.nbx, b.nby, e->d_sparse_idx, e->d_sparse_words);
     VC_CUDA(e, cudaGetLastError());
     VC_CUDA(e, cudaMemcpyAsync(listed, e->d_sparse_idx, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, e->stream));
     VC_CUDA(e, cudaMemcpyAsync(words, e->d_sparse_words, n * 128 * sizeof(uint32_t), cudaMemcpyDeviceToHost, e->stream));
@@ -1521,15 +1444,13 @@ int vc_plan_slabs(vc_engine* e, int32_t n_parts, int32_t* z_bounds) {
     if (bind_device(e)) return VC_ERR_CUDA;
     int rc = VC_OK;
     for (int k = 0; k <= n_parts; k++) z_bounds[k] = e->g.z_begin + (int)((long long)k * e->nz / n_parts);  // uniform fallback
-    const int nbx = e->Wx, nby = (e->g.Y + VC_BY - 1) / VC_BY, nbz = (e->nz + VC_BZ - 1) / VC_BZ;
+    const BrickGeom b = brick_geom(e, e->nz);
+    const int nbz = b.nbz;
     if (nbz < n_parts) return VC_OK;  // fewer brick layers than parts: keep the uniform split
     rc = ensure_brick_buffers(e);
     if (rc) return rc;
     e->flags_valid = false;
     // both classification levels of VC_EXACT over the whole range, no volumes touched; once per view group, costs summed
-    const int sbx = (nbx + VC_SUPER - 1) / VC_SUPER, sby = (nby + VC_SUPER - 1) / VC_SUPER, sbz = (nbz + VC_SUPER - 1) / VC_SUPER;
-    const long long n_super = (long long)sbx * sby * sbz;
-    unsigned int* d_nlist = (unsigned int*)(e->d_scalars + 6);
     // cost of a brick layer (8 planes): per-voxel work of its listed bricks (undecided views x voxels) plus a small constant
     // per plane for the classification and fill passes
     std::vector<double> cost((size_t)nbz, 0.0);
@@ -1537,28 +1458,15 @@ int vc_plan_slabs(vc_engine* e, int32_t n_parts, int32_t* z_bounds) {
         rc = ensure_constants(e, grp);
         if (rc) return rc;
         const int vbase = grp * VC_MAX_VIEWS;
-        VC_CUDA(e, cudaMemsetAsync(e->d_scalars + 6, 0, 2 * sizeof(unsigned long long), e->stream));
-        VcBrickParams bp{};
-        bp.list = e->d_bricks; bp.n_list = d_nlist; bp.n_list_back = d_nlist + 3; bp.list_cap = (unsigned)((long long)nbx * nby * nbz);
-        bp.brick_flags = e->d_brick_flags; bp.sat = e->d_sat + (size_t)vbase * (e->H + 1) * vc_sat_pitch(e->W);
-        bp.super_flags = e->d_super_flags; bp.super_list = e->d_super_list; bp.n_super_list = d_nlist + 1;
-        bp.X = e->g.X; bp.Y = e->g.Y; bp.Wx = e->Wx; bp.nz = e->nz; bp.z_begin = e->g.z_begin;
-        bp.nbx = nbx; bp.nby = nby; bp.nbz = nbz; bp.W = e->W; bp.H = e->H; bp.v0 = 0; bp.v1 = std::min(VC_MAX_VIEWS, e->V - vbase); bp.s = e->g.voxel_size;
-        VcBrickParams sp = bp;
-        sp.dense = e->d_super; sp.nbx = sbx; sp.nby = sby; sp.nbz = sbz;
-        vc_brick_classify_kernel<1><<<(unsigned)((n_super + VC_CLS_L1_CH - 1) / VC_CLS_L1_CH), 256, 0, e->stream>>>(sp);  // VC_CLS_L1_CH super-bricks per block
-        bp.dense = e->d_super; bp.pbx = sbx; bp.pby = sby;
-        {   // level 0: the blocks walk the list of undecided super-bricks (length known on the device only)
-            const long long l0_grid = std::min<long long>(n_super, 8LL * e->sm_count);
-            vc_brick_classify_kernel<0><<<(unsigned)l0_grid, VC_CLS_L0_THREADS, 0, e->stream>>>(bp);
-        }
+        rc = classify_bricks(e, b, e->g.z_begin, e->nz, 0, std::min(VC_MAX_VIEWS, e->V - vbase), vbase, nullptr, false);
+        if (rc) return rc;
         unsigned int counts[4] = {0, 0, 0, 0};  // front length, super-list length, (work counter), back length
-        VC_CUDA(e, cudaMemcpyAsync(counts, d_nlist, sizeof counts, cudaMemcpyDeviceToHost, e->stream));
+        VC_CUDA(e, cudaMemcpyAsync(counts, e->d_scalars + 6, sizeof counts, cudaMemcpyDeviceToHost, e->stream));
         VC_CUDA(e, cudaStreamSynchronize(e->stream));
         std::vector<VcBrickState> h((size_t)counts[0] + counts[3]);  // the list is filled from both ends (VcBrickParams)
         if (counts[0]) VC_CUDA(e, cudaMemcpy(h.data(), e->d_bricks, (size_t)counts[0] * sizeof(VcBrickState), cudaMemcpyDeviceToHost));
-        if (counts[3]) VC_CUDA(e, cudaMemcpy(h.data() + counts[0], e->d_bricks + (bp.list_cap - counts[3]), (size_t)counts[3] * sizeof(VcBrickState), cudaMemcpyDeviceToHost));
-        for (const VcBrickState& st : h) cost[st.brick / ((unsigned)nbx * (unsigned)nby)] += (double)st.n_und * (VC_BX * VC_BY * VC_BZ);
+        if (counts[3]) VC_CUDA(e, cudaMemcpy(h.data() + counts[0], e->d_bricks + (b.n_bricks - counts[3]), (size_t)counts[3] * sizeof(VcBrickState), cudaMemcpyDeviceToHost));
+        for (const VcBrickState& st : h) cost[st.brick / ((unsigned)b.nbx * (unsigned)b.nby)] += (double)st.n_und * (VC_BX * VC_BY * VC_BZ);
     }
     // (every group's kernels are complete: its list was read back above)
     double total = 0.0;
@@ -1779,10 +1687,9 @@ int vc_mc_classify(vc_engine* e) {
     (void)n;
     VcMcFlags mf{};
     mf.enabled = (e->flags_valid && e->d_brick_flags && !e->reset_pending) ? 1 : 0;
-    if (const char* nf = getenv("VOXCARVE_MC_NO_FLAGS")) if (atoi(nf)) mf.enabled = 0;  // (measurement switch)
     mf.brick_flags = e->d_brick_flags; mf.super_flags = e->d_super_flags;
-    mf.nby = (e->g.Y + VC_BY - 1) / VC_BY;
-    mf.pbx = (e->Wx + VC_SUPER - 1) / VC_SUPER; mf.pby = (mf.nby + VC_SUPER - 1) / VC_SUPER;
+    const BrickGeom b = brick_geom(e, e->nz);
+    mf.nby = b.nby; mf.pbx = b.sbx; mf.pby = b.sby;
     mf.z_begin = e->g.z_begin; mf.z_end = e->g.z_end;
     vc_mc_classify_kernel<<<(unsigned)blocks, 256, 0, e->stream>>>(vol_view(e), cz_begin, n_cz, Cw, e->d_hist, mf);
     VC_CUDA(e, cudaGetLastError());

@@ -84,8 +84,7 @@ typedef struct vc_stats {
     uint64_t bricks_listed;
     uint64_t flood_rounds;         /* sweep rounds of the last vc_fast_carve */
     uint64_t carve_launches;       /* kernel launches issued by this engine so far */
-    uint64_t l2_persist_bytes;     /* bytes of the mask set pinned by the L2 access-policy window; 0 unless the environment
-                                      variable VOXCARVE_L2_PERSIST_MB enables it (measured neutral to harmful on B200) */
+    uint64_t l2_persist_bytes;     /* always 0 (reserved: keeps the layout of API version 3) */
     /* per-voxel f32 filter of VC_EXACT (counting runs only): 32-voxel rows evaluated, rows that needed the exact f64
      * re-evaluation, and filter decisions that disagreed with the exact evaluation (every decision is cross-checked
      * in a counting run; anything but 0 is a bug) */
@@ -111,9 +110,8 @@ VC_EXPORT int vc_synchronize(vc_engine* e);
  * whenever grid, slab, views, buffers or stream arguments change; VOXCARVE_NO_GRAPH=1 in the environment disables it) and
  * vc_stats.last_classify_ms stays 0.  On: plain launches in stream order with an event between classification and per-voxel
  * kernel, so that vc_stats splits the carve time and ncu sees every launch.
- * Other environment switches, read once per process, for comparisons: VOXCARVE_BLIND_FILL=0 (fresh carve: the words of all
- * non-listed bricks written by the first blocks of the per-voxel kernel from the flags, instead of the 'carved and seen' pattern
- * everywhere first + a patch pass), VOXCARVE_COMPRESSIBLE=0 (engine-owned volumes in plain cudaMalloc memory). */
+ * The only other environment switch, read once per process: VOXCARVE_COMPRESSIBLE=0 (engine-owned volumes in plain cudaMalloc
+ * memory, what a GPU that refuses compressible memory gets anyway). */
 VC_EXPORT int vc_set_profiling(vc_engine* e, int32_t on);
 
 /* ---- inputs ---------------------------------------------------------------------- */

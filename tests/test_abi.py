@@ -87,3 +87,14 @@ def test_binding_structs_match_the_header(tmp_path):
         assert int(out[cname]) == ctypes.sizeof(mirror)
         for n, _ in mirror._fields_:
             assert int(out[f"{cname}.{n}"]) == getattr(mirror, n).offset, (cname, n)
+
+
+def test_environment_switches_are_documented():
+    """The environment variables the library reads (getenv in csrc/) are exactly the ones include/voxcarve.h documents."""
+    csrc = os.path.join(ROOT, "ar_voxel_project_b200", "csrc")
+    read = set()
+    for f in os.listdir(csrc):
+        read |= set(re.findall(r'getenv\("([A-Za-z0-9_]+)"\)', open(os.path.join(csrc, f)).read()))
+    hdr = open(os.path.join(ROOT, "include", "voxcarve.h")).read()
+    documented = set(re.findall(r"\bVOXCARVE_[A-Z0-9_]+", hdr)) - {"VOXCARVE_H"}  # minus the include guard
+    assert read and read == documented, (sorted(read), sorted(documented))

@@ -1008,10 +1008,10 @@ def test_peer_gather_assembles_the_grid_in_every_engine(A, oracle):
 
 
 def test_fill_schemes_and_volume_memory_agree(A, oracle):
-    """The fresh carve's fill (blind 'carved and seen' pass next to the classification + patch, volumes in compressible memory
-    when the GPU grants it) against the flag-driven fill in plain cudaMalloc memory (VOXCARVE_BLIND_FILL=0,
-    VOXCARVE_COMPRESSIBLE=0: read once per process, hence the subprocesses) and against the oracle - whole grid, a ragged
-    slab with a partial last word, a grid whose rows are not whole quads (no blind pass there), twice in a row (graph replay)."""
+    """The fresh carve's fill (blind 'carved and seen' pass next to the classification + patch) with the volumes in compressible
+    memory when the GPU grants it, against the same in plain cudaMalloc memory (VOXCARVE_COMPRESSIBLE=0: read once per process,
+    hence the subprocesses) and against the oracle - whole grid, a ragged slab with a partial last word, a grid whose rows are
+    not whole quads (no blind pass there), twice in a row (graph replay)."""
     import json
     import subprocess
     import sys
@@ -1040,13 +1040,13 @@ for name, dims, slab in (("cube", (256, 256, 256), None), ("slab7", (200, 130, 1
 print(json.dumps(out))
 ''' % ROOT
     res = {}
-    for tag, env in (("default", {}), ("plain", {"VOXCARVE_BLIND_FILL": "0", "VOXCARVE_COMPRESSIBLE": "0"}), ("blind_plain_memory", {"VOXCARVE_COMPRESSIBLE": "0"})):
+    for tag, env in (("default", {}), ("blind_plain_memory", {"VOXCARVE_COMPRESSIBLE": "0"})):
         r = subprocess.run([sys.executable, "-c", script], capture_output=True, text=True, timeout=600, env={**os.environ, **env})
         assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
         res[tag] = json.loads(r.stdout.strip().splitlines()[-1])
     for name in ("cube", "slab7", "slabq"):
-        assert res["default"][name] == res["plain"][name] == res["blind_plain_memory"][name], (name, res)
-    assert res["plain"]["cube_compressible"] == 0
+        assert res["default"][name] == res["blind_plain_memory"][name], (name, res)
+    assert res["blind_plain_memory"]["cube_compressible"] == 0
     # ... and the default against the oracle (the other parity tests all run the default too)
     import hashlib
     from ar_voxel_project_b200.synth import Workload

@@ -29,7 +29,7 @@ with A.VoxelEngine(w.X, w.Y, w.Z, w.s, z_begin=z0, z_end=z1) as e:
         e.carve(a.mode)
         e.synchronize()
         st = e.stats()
-        print("carve ms", st["last_carve_ms"], "of which classify+fill", st["last_classify_ms"], "L2 persisting bytes", st["l2_persist_bytes"])
+        print("carve ms", st["last_carve_ms"], "of which classify+fill", st["last_classify_ms"])
     e.reset()
     e.carve(a.mode, count_executed=True)
     st = e.stats()
