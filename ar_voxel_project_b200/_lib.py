@@ -14,6 +14,7 @@ VC_EXACT, VC_FAST_F32, VC_EXACT_FLAT = 0, 1, 2
 VC_COLOR_CLOSEST, VC_COLOR_AVG = 1, 2
 VC_MASK_BITS, VC_MASK_BGR8, VC_MASK_BGR8_RAW = 0, 1, 2
 VC_MAX_TOTAL_VIEWS = 4096
+VC_RAW_MAX_SIDE = 32766  # W and H of raw (distorted) input: cv::undistort refuses a side of 32767 or more
 
 
 class GridDesc(C.Structure):

@@ -115,7 +115,7 @@ struct vc_engine {
     unsigned long long sparse_cap = 0;
     void* d_scratch = nullptr;
     size_t scratch_bytes = 0;
-    double* d_undist_ir = nullptr;       // per-stripe inverse camera matrices of the device cv::undistort (grow-only)
+    double* d_undist_ir = nullptr;       // per-stripe inverse camera matrices and row block starts of the device cv::undistort (grow-only)
     size_t undist_ir_count = 0;
     int sm_count = 148;
     uint8_t* d_images = nullptr;
@@ -632,6 +632,8 @@ int vc_set_masks(vc_engine* e, const void* masks, int32_t format) {
     if (e->V == 0) return fail(e, VC_ERR_STATE, "vc_set_masks: call vc_set_views first");
     if (format != VC_MASK_BITS && format != VC_MASK_BGR8 && format != VC_MASK_BGR8_RAW) return fail(e, VC_ERR_ARG, "vc_set_masks: unknown format %d", format);
     if (format == VC_MASK_BGR8_RAW && !e->have_calib) return fail(e, VC_ERR_STATE, "vc_set_masks: raw masks need vc_set_calibration first");
+    if (format == VC_MASK_BGR8_RAW && (e->W > VC_RAW_MAX_SIDE || e->H > VC_RAW_MAX_SIDE))
+        return fail(e, VC_ERR_ARG, "vc_set_masks: raw masks of %dx%d: cv::undistort takes W and H up to %d", e->W, e->H, VC_RAW_MAX_SIDE);
     if (bind_device(e)) return VC_ERR_CUDA;
     if (!e->d_mask) VC_CUDA(e, cudaMalloc(&e->d_mask, e->mask_bytes));
     const size_t sat_words = (size_t)e->V * (e->H + 1) * vc_sat_pitch(e->W);
@@ -681,35 +683,27 @@ int vc_set_images(vc_engine* e, const uint8_t* images_bgr) {
     return VC_OK;
 }
 
-// 3x3 inverse by Gaussian elimination with partial pivoting on [A | I] (cv::invert, DECOMP_LU), f64, no FMA
-static void inv3x3_lu(const double* A, double* inv) {
-    volatile double a[3][3], b[3][3];
-    for (int i = 0; i < 3; i++) for (int j = 0; j < 3; j++) { a[i][j] = A[i * 3 + j]; b[i][j] = i == j; }
-    for (int i = 0; i < 3; i++) {
-        int k = i;
-        for (int j = i + 1; j < 3; j++) if (fabs(a[j][i]) > fabs(a[k][i])) k = j;
-        if (k != i) for (int j = 0; j < 3; j++) { double t = a[i][j]; a[i][j] = a[k][j]; a[k][j] = t; t = b[i][j]; b[i][j] = b[k][j]; b[k][j] = t; }
-        const double d = -1 / a[i][i];
-        for (int j = i + 1; j < 3; j++) {
-            const double alpha = a[j][i] * d;
-            for (int c = i + 1; c < 3; c++) { const double t = alpha * a[i][c]; a[j][c] = a[j][c] + t; }
-            for (int c = 0; c < 3; c++) { const double t = alpha * b[i][c]; b[j][c] = b[j][c] + t; }
-        }
-    }
-    for (int i = 2; i >= 0; i--)
-        for (int j = 0; j < 3; j++) {
-            double s = b[i][j];
-            for (int k = i + 1; k < 3; k++) { const double t = a[i][k] * b[k][j]; s = s - t; }
-            b[i][j] = s / a[i][i];
-        }
-    for (int i = 0; i < 3; i++) for (int j = 0; j < 3; j++) inv[i * 3 + j] = b[i][j];
+// 3x3 inverse as cv::invert(DECOMP_LU) computes it for n == 3: the adjugate times 1/det, all zeros when det == 0.  f64 with no
+// FMA contraction (every product is rounded through a volatile), as OpenCV's core module is built for x86-64 without FMA.
+static void inv3x3_cv(const double* S, double* t) {
+    auto mul = [](double a, double b) { volatile double p = a * b; return (double)p; };
+    auto cof = [&](int a, int b, int c, int d, int e, int f, int g, int h) { return mul(S[a * 3 + b], S[c * 3 + d]) - mul(S[e * 3 + f], S[g * 3 + h]); };
+    double det = mul(S[0], cof(1, 1, 2, 2, 1, 2, 2, 1)) - mul(S[1], cof(1, 0, 2, 2, 1, 2, 2, 0));
+    det = det + mul(S[2], cof(1, 0, 2, 1, 1, 1, 2, 0));
+    if (det == 0) { for (int i = 0; i < 9; i++) t[i] = 0; return; }
+    const double d = 1. / det;
+    t[0] = mul(cof(1, 1, 2, 2, 1, 2, 2, 1), d); t[1] = mul(cof(0, 2, 2, 1, 0, 1, 2, 2), d); t[2] = mul(cof(0, 1, 1, 2, 0, 2, 1, 1), d);
+    t[3] = mul(cof(1, 2, 2, 0, 1, 0, 2, 2), d); t[4] = mul(cof(0, 0, 2, 2, 0, 2, 2, 0), d); t[5] = mul(cof(0, 2, 1, 0, 0, 0, 1, 2), d);
+    t[6] = mul(cof(1, 0, 2, 1, 1, 1, 2, 0), d); t[7] = mul(cof(0, 1, 2, 0, 0, 0, 2, 1), d); t[8] = mul(cof(0, 0, 1, 1, 0, 1, 1, 0), d);
 }
 
-// device-to-device cv::undistort of n 8UC3 images on `stream`
-// ir_buf / ir_count: optional grow-only device buffer for the per-stripe inverse matrices (an engine's); else allocated per call
+// device-to-device cv::undistort of n 8UC3 images on `stream`; W and H must be below 32767 (the callers refuse larger)
+// ir_buf / ir_count: optional grow-only device buffer (an engine's) for the per-stripe inverse matrices followed by the rows'
+// block starts, in doubles; else allocated per call
 static cudaError_t undistort_device(const uint8_t* d_src, uint8_t* d_dst, int n, int W, int H, const double* K, const double* dist8, cudaStream_t stream,
                                     double** ir_buf, size_t* ir_count) {
-    int stripe = (1 << 12) / (W > 1 ? W : 1);
+    if (W < 1 || H < 1 || W > VC_RAW_MAX_SIDE || H > VC_RAW_MAX_SIDE) return cudaErrorInvalidValue;
+    int stripe = (1 << 12) / W;
     if (stripe < 1) stripe = 1;
     if (stripe > H) stripe = H;
     const int n_stripes = (H + stripe - 1) / stripe;
@@ -718,26 +712,28 @@ static cudaError_t undistort_device(const uint8_t* d_src, uint8_t* d_dst, int n,
         double Ar[9];
         memcpy(Ar, K, sizeof Ar);
         Ar[5] = K[5] - (double)(sidx * stripe);
-        inv3x3_lu(Ar, &ir[(size_t)sidx * 9]);
+        inv3x3_cv(Ar, &ir[(size_t)sidx * 9]);
     }
+    const size_t n_doubles = ir.size() + (size_t)H * (W / 8 + 1) * 3;
     double* d_ir = nullptr;
     cudaError_t s = cudaSuccess;
-    if (ir_buf && *ir_count >= ir.size()) d_ir = *ir_buf;
+    if (ir_buf && *ir_count >= n_doubles) d_ir = *ir_buf;
     else {
-        s = cudaMalloc(&d_ir, ir.size() * sizeof(double));
+        s = cudaMalloc(&d_ir, n_doubles * sizeof(double));
         if (s != cudaSuccess) return s;
         if (ir_buf) {  // the old buffer may still be read by a kernel on this stream
             if (*ir_buf) { cudaStreamSynchronize(stream); cudaFree(*ir_buf); }
-            *ir_buf = d_ir; *ir_count = ir.size();
+            *ir_buf = d_ir; *ir_count = n_doubles;
         }
     }
     s = cudaMemcpyAsync(d_ir, ir.data(), ir.size() * sizeof(double), cudaMemcpyHostToDevice, stream);
     if (s == cudaSuccess) s = cudaStreamSynchronize(stream);  // `ir` is a local
     if (s == cudaSuccess) {
         VcUndistortParams p{};
-        p.src = d_src; p.dst = d_dst; p.ir = d_ir; p.W = W; p.H = H; p.n = n; p.stripe = stripe;
+        p.src = d_src; p.dst = d_dst; p.ir = d_ir; p.starts = d_ir + ir.size(); p.W = W; p.H = H; p.n = n; p.stripe = stripe;
         p.fx = K[0]; p.fy = K[4]; p.u0 = K[2]; p.v0 = K[5];
         p.k1 = dist8[0]; p.k2 = dist8[1]; p.p1 = dist8[2]; p.p2 = dist8[3]; p.k3 = dist8[4]; p.k4 = dist8[5]; p.k5 = dist8[6]; p.k6 = dist8[7];
+        vc_undistort_rows_kernel<<<(H + 127) / 128, 128, 0, stream>>>(p);
         vc_undistort_kernel<<<dim3((W + 255) / 256, H, n), 256, 0, stream>>>(p);
         s = cudaGetLastError();
         if (s == cudaSuccess) s = cudaStreamSynchronize(stream);
@@ -783,6 +779,8 @@ int vc_set_images_raw(vc_engine* e, const uint8_t* images_bgr) {
     if (!images_bgr) return fail(e, VC_ERR_ARG, "vc_set_images_raw: null buffer");
     if (e->V == 0) return fail(e, VC_ERR_STATE, "vc_set_images_raw: call vc_set_views first");
     if (!e->have_calib) return fail(e, VC_ERR_STATE, "vc_set_images_raw: needs vc_set_calibration first");
+    if (e->W > VC_RAW_MAX_SIDE || e->H > VC_RAW_MAX_SIDE)
+        return fail(e, VC_ERR_ARG, "vc_set_images_raw: images of %dx%d: cv::undistort takes W and H up to %d", e->W, e->H, VC_RAW_MAX_SIDE);
     if (bind_device(e)) return VC_ERR_CUDA;
     const size_t bytes = (size_t)e->V * e->H * e->W * 3;
     if (!e->d_images) VC_CUDA(e, cudaMalloc(&e->d_images, bytes));
@@ -802,6 +800,8 @@ int vc_append_views(vc_engine* e, int32_t n, const float* P, const float* M, con
     if (e->V == 0 || !e->d_mask) return fail(e, VC_ERR_STATE, "vc_append_views: call vc_set_views and vc_set_masks first");
     if (mask_format != VC_MASK_BITS && mask_format != VC_MASK_BGR8 && mask_format != VC_MASK_BGR8_RAW) return fail(e, VC_ERR_ARG, "vc_append_views: unknown mask format %d", mask_format);
     if (mask_format == VC_MASK_BGR8_RAW && !e->have_calib) return fail(e, VC_ERR_STATE, "vc_append_views: raw masks need vc_set_calibration first");
+    if (mask_format == VC_MASK_BGR8_RAW && (e->W > VC_RAW_MAX_SIDE || e->H > VC_RAW_MAX_SIDE))
+        return fail(e, VC_ERR_ARG, "vc_append_views: raw masks of %dx%d: cv::undistort takes W and H up to %d", e->W, e->H, VC_RAW_MAX_SIDE);
     if (n < 1) return fail(e, VC_ERR_ARG, "vc_append_views: n=%d views (need at least 1)", n);
     if (!P || !masks) return fail(e, VC_ERR_ARG, "vc_append_views: P and masks are required");
     if ((long long)e->V + n > VC_MAX_TOTAL_VIEWS) return fail(e, VC_ERR_ARG, "vc_append_views: %d + %d views exceed %d", e->V, n, VC_MAX_TOTAL_VIEWS);
@@ -915,6 +915,7 @@ int vc_download_images(vc_engine* e, uint8_t* images_bgr) {
 int vc_undistort_bgr(int32_t device, int32_t n, int32_t W, int32_t H, const uint8_t* src, const double K[9], const double* dist, int32_t n_dist, uint8_t* dst) {
     if (!src || !dst || !K || !dist || n < 1 || W < 1 || H < 1) return fail(nullptr, VC_ERR_ARG, "vc_undistort_bgr: bad argument");
     if (n_dist != 4 && n_dist != 5 && n_dist != 8) return fail(nullptr, VC_ERR_ARG, "vc_undistort_bgr: %d distortion coefficients (need 4, 5 or 8)", n_dist);
+    if (W > VC_RAW_MAX_SIDE || H > VC_RAW_MAX_SIDE) return fail(nullptr, VC_ERR_ARG, "vc_undistort_bgr: %dx%d: cv::undistort takes W and H up to %d", W, H, VC_RAW_MAX_SIDE);
     if (cudaSetDevice(device) != cudaSuccess) { cudaGetLastError(); return fail(nullptr, VC_ERR_CUDA, "vc_undistort_bgr: no CUDA device %d; this engine has no CPU fallback", device); }
     double d8[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     for (int i = 0; i < n_dist; i++) d8[i] = dist[i];

@@ -70,6 +70,11 @@ enum vc_carve_mode { VC_EXACT = 0, VC_FAST_F32 = 1, VC_EXACT_FLAT = 2 };
 /* values of the reference's -color flag (main.cpp:30,278-288) */
 enum vc_color_mode { VC_COLOR_CLOSEST = 1, VC_COLOR_AVG = 2 };
 enum vc_mask_format { VC_MASK_BITS = 0, VC_MASK_BGR8 = 1, VC_MASK_BGR8_RAW = 2 /* distorted: undistorted on the device, needs vc_set_calibration */ };
+/* Raw (distorted) input - VC_MASK_BGR8_RAW masks, vc_set_images_raw, vc_append_views with raw masks, vc_undistort_bgr - is
+ * undistorted on the device bit for bit as cv2 4.13.0's cv::undistort computes it on x86-64 with its AVX2 code path (DESIGN
+ * section 8 f-4).  cv::undistort refuses images with a side of 32767 or more (remap's SHRT_MAX limit), so those calls return
+ * VC_ERR_ARG for W or H above VC_RAW_MAX_SIDE and leave the engine as it was. */
+#define VC_RAW_MAX_SIDE 32766
 
 typedef struct vc_stats {
     double last_carve_ms;          /* CUDA-event time of the last vc_carve (all its kernels) */

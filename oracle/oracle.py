@@ -45,6 +45,8 @@ def lib():
         L.vo_max_threads.restype = C.c_int
         L.vo_undistort.argtypes = [C.c_int, C.c_int, u8p, np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS"),
                                    np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS"), C.c_int, u8p]
+        L.vo_undistort_map.argtypes = [C.c_int, C.c_int, np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS"),
+                                       np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS"), C.c_int, C.c_void_p, C.c_void_p]
         L.vo_closure.argtypes = [C.c_int] * 4 + [f32p, f32p]
         L.vo_marching_cubes.argtypes = [C.c_int] * 3 + [f32p, C.c_float, np.ctypeslib.ndpointer(np.int8, flags="C_CONTIGUOUS"), f32p, u32p, C.c_uint64]
         L.vo_marching_cubes.restype = C.c_uint64
@@ -209,5 +211,17 @@ def undistort(img_bgr, K, dist):
     out = np.empty_like(img)
     rc = lib().vo_undistort(W, H, img, np.ascontiguousarray(K, np.float64).reshape(9), d, len(d), out)
     if rc != 0:
-        raise ValueError("distortion vector must have 4, 5 or 8 coefficients")
+        raise ValueError("distortion vector must have 4, 5 or 8 coefficients, and W and H must be below 32767")
     return out
+
+
+def undistort_map(K, dist, W, H):
+    """the int16 map cv::undistort remaps with, stripe by stripe: (int16[H,W,2] sx/sy, uint16[H,W] (iv & 31) * 32 + (iu & 31)),
+    the layout of cv2.initUndistortRectifyMap(..., cv2.CV_16SC2)"""
+    d = np.ascontiguousarray(np.asarray(dist, np.float64).ravel())
+    sxy, frac = np.empty((H, W, 2), np.int16), np.empty((H, W), np.uint16)
+    rc = lib().vo_undistort_map(int(W), int(H), np.ascontiguousarray(K, np.float64).reshape(9), d, len(d),
+                                sxy.ctypes.data_as(C.c_void_p), frac.ctypes.data_as(C.c_void_p))
+    if rc != 0:
+        raise ValueError("distortion vector must have 4, 5 or 8 coefficients, and W and H must be below 32767")
+    return sxy, frac

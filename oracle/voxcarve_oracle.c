@@ -441,42 +441,71 @@ VO_API int vo_write_off(const char* path, uint64_t ntris, const float* verts, co
 /* ------------------------------------------------------------------------------------------------
  * cv::undistort as the reference calls it (VoxelCarving.cpp:36,86,89; ColorReconstruction.h:23,26): 8UC3 image,
  * camera matrix K (3x3 f64), distortion (k1 k2 p1 p2 [k3 [k4 k5 k6]]).  The algorithm lives in OpenCV (un-vendored,
- * un-pinned by the reference; pinned here to cv2 4.13.0 through tests/golden/undistort_kat.npz):
- *   stripes of min(max(1, 4096/cols), rows) rows; per stripe the new camera matrix is K with cy - y0 and the map is
- *   initUndistortRectifyMap(K, dist, I, K') in f64:  (x, y) = K'^-1 (j, i, 1);  radial/tangential model;  (u, v) = K (xd, yd, 1);
- *   fixed point: iu = round_half_even(u * 32), sx = iu >> 5, fx = iu & 31 (same for v);
- *   remap INTER_LINEAR, BORDER_CONSTANT(0): out = (sum_taps src * w + 2^14) >> 15 with w = (32-fx|fx)(32-fy|fy) * 32.
+ * un-pinned by the reference).  Pinned here to what cv2 4.13.0 computes on x86-64 with its AVX2 code path
+ * (tests/golden/undistort_kat.npz, tests/golden/undistort_hostile_kat.npz), W and H below 32767 (remap's limit):
+ *   stripes of min(max(1, 4096/W), H) rows; per stripe the new camera matrix K' is K with cy - y0, and the map is
+ *   initUndistortRectifyMap(K, dist, I, K', CV_16SC2) in f64:
+ *   - ir = K'^-1 by cv::invert's closed form for 3x3 (adjugate times 1/det; all zeros when det == 0);
+ *   - row i of the stripe starts at (_x, _y, _w) = fma(i, ir[1|4|7], ir[2|5|8]);
+ *   - body, columns [0, W - W%8): blocks of 8 (two AVX2 vectors); the block start advances by 8 ir[0|3|6] per block and
+ *     lane l adds l ir[0|3|6]; the polynomials are FMA chains (undistort_body);
+ *   - tail, the last W%8 columns: the scalar loop, continuing from the last block start with += ir[0|3|6] per column,
+ *     with the FMA contractions the AVX2 build gives it (undistort_tail);
+ *   - the thin-prism and tilt stages are identities here, but they turn non-finite intermediates into NaN;
+ *   - fixed point: iu = cvRound(u * 32) (round half to even; INT_MIN when NaN or outside int32), sx = iu >> 5,
+ *     fx = iu & 31 (same for v); the body saturates sx, sy to int16, the tail wraps them (a (short) cast);
+ *   remap INTER_LINEAR, BORDER_CONSTANT(0) with those int16 coordinates: out = (sum_taps src * w + 2^14) >> 15,
+ *   w = (32-fx|fx)(32-fy|fy) * 32, taps outside the image read 0.
  * ---------------------------------------------------------------------------------------------- */
-static void inv3x3_lu(const double* A, double* inv) { /* Gaussian elimination with partial pivoting on [A | I], as cv::invert(DECOMP_LU) */
-    double a[3][3], b[3][3];
-    for (int i = 0; i < 3; i++) for (int j = 0; j < 3; j++) { a[i][j] = A[i * 3 + j]; b[i][j] = i == j; }
-    for (int i = 0; i < 3; i++) {
-        int k = i;
-        for (int j = i + 1; j < 3; j++) if (fabs(a[j][i]) > fabs(a[k][i])) k = j;
-        if (k != i) for (int j = 0; j < 3; j++) { double t = a[i][j]; a[i][j] = a[k][j]; a[k][j] = t; t = b[i][j]; b[i][j] = b[k][j]; b[k][j] = t; }
-        double d = -1 / a[i][i];
-        for (int j = i + 1; j < 3; j++) {
-            double alpha = a[j][i] * d;
-            for (int c = i + 1; c < 3; c++) a[j][c] += alpha * a[i][c];
-            for (int c = 0; c < 3; c++) b[j][c] += alpha * b[i][c];
-        }
-    }
-    for (int i = 2; i >= 0; i--)
-        for (int j = 0; j < 3; j++) {
-            double s = b[i][j];
-            for (int k = i + 1; k < 3; k++) s -= a[i][k] * b[k][j];
-            b[i][j] = s / a[i][i];
-        }
-    for (int i = 0; i < 3; i++) for (int j = 0; j < 3; j++) inv[i * 3 + j] = b[i][j];
+static void inv3x3_cv(const double* S, double* t) {  /* cv::invert(DECOMP_LU) for a 3x3 f64 matrix */
+#define S_(i, j) S[(i) * 3 + (j)]
+    double d = S_(0, 0) * (S_(1, 1) * S_(2, 2) - S_(1, 2) * S_(2, 1)) - S_(0, 1) * (S_(1, 0) * S_(2, 2) - S_(1, 2) * S_(2, 0)) +
+               S_(0, 2) * (S_(1, 0) * S_(2, 1) - S_(1, 1) * S_(2, 0));
+    if (d == 0) { for (int i = 0; i < 9; i++) t[i] = 0; return; }
+    d = 1. / d;
+    t[0] = (S_(1, 1) * S_(2, 2) - S_(1, 2) * S_(2, 1)) * d; t[1] = (S_(0, 2) * S_(2, 1) - S_(0, 1) * S_(2, 2)) * d;
+    t[2] = (S_(0, 1) * S_(1, 2) - S_(0, 2) * S_(1, 1)) * d; t[3] = (S_(1, 2) * S_(2, 0) - S_(1, 0) * S_(2, 2)) * d;
+    t[4] = (S_(0, 0) * S_(2, 2) - S_(0, 2) * S_(2, 0)) * d; t[5] = (S_(0, 2) * S_(1, 0) - S_(0, 0) * S_(1, 2)) * d;
+    t[6] = (S_(1, 0) * S_(2, 1) - S_(1, 1) * S_(2, 0)) * d; t[7] = (S_(0, 1) * S_(2, 0) - S_(0, 0) * S_(2, 1)) * d;
+    t[8] = (S_(0, 0) * S_(1, 1) - S_(0, 1) * S_(1, 0)) * d;
+#undef S_
+}
+static int cv_round(double v) { /* cvtsd2si / cvtpd2dq: round half to even, INT_MIN when NaN or outside int32 */
+    const double r = nearbyint(v);
+    return r >= -2147483648.0 && r < 2147483648.0 ? (int)r : INT32_MIN;
+}
+static double cv_kr(const double* k, double r2) {
+    return fma(fma(fma(k[4], r2, k[1]), r2, k[0]), r2, 1.0) / fma(fma(fma(k[7], r2, k[6]), r2, k[5]), r2, 1.0);
+}
+/* one vector lane: (X, Y, Wh) = block start + lane * ir[0|3|6] */
+static void undistort_body(const double* k, double fx, double fy, double u0, double v0, double X, double Y, double Wh, double* u, double* v) {
+    const double m = 1.0 / Wh, x = X * m, y = Y * m;
+    const double xx = x * x, yy = y * y, r2 = xx + yy, kr = cv_kr(k, r2);
+    const double xy2 = (x * y) * 2.0;
+    double xd = fma(fma(2.0, xx, r2), k[3], x * kr), yd = fma(fma(2.0, yy, r2), k[2], y * kr);
+    xd = fma(k[2], xy2, xd); yd = fma(k[3], xy2, yd);
+    const double r4 = r2 * r2;
+    const int finite = isfinite(r4) && isfinite(xd) && isfinite(yd);  /* else the thin-prism / tilt terms give NaN */
+    *u = finite ? fma(fx, xd, u0) : NAN; *v = finite ? fma(fy, yd, v0) : NAN;
+}
+static void undistort_tail(const double* k, double fx, double fy, double u0, double v0, double X, double Y, double Wh, double* u, double* v) {
+    const double w = 1. / Wh, x = X * w, y = Y * w;
+    const double x2 = x * x, y2 = y * y, r2 = x2 + y2, _2xy = 2 * x * y, kr = cv_kr(k, r2);
+    const double xd = fma(k[3], r2 + 2 * x2, fma(x, kr, k[2] * _2xy));
+    const double yd = fma(k[3], _2xy, fma(y, kr, k[2] * (r2 + 2 * y2)));
+    const int finite = isfinite(r2) && isfinite(xd) && isfinite(yd);
+    *u = finite ? fma(fx, xd, u0) : NAN; *v = finite ? fma(fy, yd, v0) : NAN;
 }
 
-VO_API int vo_undistort(int W, int H, const uint8_t* src, const double* K, const double* dist, int n_dist, uint8_t* dst) {
+/* the int16 map of cv::undistort: per pixel sx, sy and the fraction index (iv & 31) * 32 + (iu & 31), as CV_16SC2 + CV_16UC1 */
+VO_API int vo_undistort_map(int W, int H, const double* K, const double* dist, int n_dist, int16_t* sxy, uint16_t* frac) {
     if (n_dist != 4 && n_dist != 5 && n_dist != 8) return -1;
-    double k[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    if (W < 1 || H < 1 || W >= 32767 || H >= 32767) return -1;
+    double k[8] = {0, 0, 0, 0, 0, 0, 0, 0};  /* k1 k2 p1 p2 k3 k4 k5 k6 */
     for (int i = 0; i < n_dist; i++) k[i] = dist[i];
-    const double k1 = k[0], k2 = k[1], p1 = k[2], p2 = k[3], k3 = k[4], k4 = k[5], k5 = k[6], k6 = k[7];
     const double fx = K[0], fy = K[4], u0 = K[2], v0 = K[5];
-    int stripe0 = (1 << 12) / (W > 1 ? W : 1);
+    const int W8 = W - W % 8;
+    int stripe0 = (1 << 12) / W;
     if (stripe0 < 1) stripe0 = 1;
     if (stripe0 > H) stripe0 = H;
     for (int y0 = 0; y0 < H; y0 += stripe0) {
@@ -484,33 +513,50 @@ VO_API int vo_undistort(int W, int H, const uint8_t* src, const double* K, const
         double Ar[9], ir[9];
         memcpy(Ar, K, sizeof Ar);
         Ar[5] = v0 - y0;
-        inv3x3_lu(Ar, ir);
-        for (int i = 0; i < n; i++)
+        inv3x3_cv(Ar, ir);
+        for (int i = 0; i < n; i++) {
+            double X = fma(i, ir[1], ir[2]), Y = fma(i, ir[4], ir[5]), Wh = fma(i, ir[7], ir[8]);
             for (int j = 0; j < W; j++) {
-                double _x = (i * ir[1] + ir[2]) + j * ir[0], _y = (i * ir[4] + ir[5]) + j * ir[3], _w = (i * ir[7] + ir[8]) + j * ir[6];
-                double w = 1. / _w, x = _x * w, y = _y * w;
-                double x2 = x * x, y2 = y * y, r2 = x2 + y2, _2xy = 2 * x * y;
-                double kr = (1 + ((k3 * r2 + k2) * r2 + k1) * r2) / (1 + ((k6 * r2 + k5) * r2 + k4) * r2);
-                double xd = (x * kr + p1 * _2xy) + p2 * (r2 + 2 * x2);
-                double yd = (y * kr + p1 * (r2 + 2 * y2)) + p2 * _2xy;
-                double u = fx * xd + u0, v = fy * yd + v0;
-                double ru = nearbyint(u * 32), rv = nearbyint(v * 32); /* cvRound: round half to even, saturating */
-                int iu = ru >= 2147483647.0 ? INT32_MAX : (ru <= -2147483648.0 || ru != ru ? INT32_MIN : (int)ru);
-                int iv = rv >= 2147483647.0 ? INT32_MAX : (rv <= -2147483648.0 || rv != rv ? INT32_MIN : (int)rv);
-                int sx = iu >> 5, sy = iv >> 5, ax = iu & 31, ay = iv & 31;
-                int wt[4] = {(32 - ax) * (32 - ay) * 32, ax * (32 - ay) * 32, (32 - ax) * ay * 32, ax * ay * 32};
-                uint8_t* o = dst + ((size_t)(y0 + i) * W + j) * 3;
-                for (int c = 0; c < 3; c++) {
-                    int acc = 0;
-                    for (int t = 0; t < 4; t++) {
-                        int xx = sx + (t & 1), yy = sy + (t >> 1);
-                        int val = (xx >= 0 && xx < W && yy >= 0 && yy < H) ? src[((size_t)yy * W + xx) * 3 + c] : 0;
-                        acc += val * wt[t];
-                    }
-                    acc = (acc + (1 << 14)) >> 15;
-                    o[c] = (uint8_t)(acc < 0 ? 0 : (acc > 255 ? 255 : acc));
+                double u, v;
+                const int body = j < W8;
+                if (body) {
+                    const int l = j % 8;
+                    undistort_body(k, fx, fy, u0, v0, X + ir[0] * l, Y + ir[3] * l, Wh + ir[6] * l, &u, &v);
+                    if (l == 7) { X += 8 * ir[0]; Y += 8 * ir[3]; Wh += 8 * ir[6]; }
+                } else {
+                    undistort_tail(k, fx, fy, u0, v0, X, Y, Wh, &u, &v);
+                    X += ir[0]; Y += ir[3]; Wh += ir[6];
                 }
+                const int iu = cv_round(u * 32), iv = cv_round(v * 32);
+                int sx = iu >> 5, sy = iv >> 5;
+                if (body) { sx = sx < -32768 ? -32768 : (sx > 32767 ? 32767 : sx); sy = sy < -32768 ? -32768 : (sy > 32767 ? 32767 : sy); }
+                const size_t o = (size_t)(y0 + i) * W + j;
+                sxy[o * 2] = (int16_t)sx; sxy[o * 2 + 1] = (int16_t)sy;  /* the tail's (short) cast wraps */
+                frac[o] = (uint16_t)((iv & 31) * 32 + (iu & 31));
             }
+        }
     }
     return 0;
+}
+
+VO_API int vo_undistort(int W, int H, const uint8_t* src, const double* K, const double* dist, int n_dist, uint8_t* dst) {
+    int16_t* sxy = malloc((size_t)W * H * 2 * sizeof(int16_t));
+    uint16_t* frac = malloc((size_t)W * H * sizeof(uint16_t));
+    int rc = sxy && frac ? vo_undistort_map(W, H, K, dist, n_dist, sxy, frac) : -2;
+    if (rc == 0)
+        for (size_t o = 0; o < (size_t)W * H; o++) {  /* remap INTER_LINEAR, BORDER_CONSTANT(0) */
+            const int sx = sxy[o * 2], sy = sxy[o * 2 + 1], ax = frac[o] & 31, ay = frac[o] >> 5;
+            const int wt[4] = {(32 - ax) * (32 - ay) * 32, ax * (32 - ay) * 32, (32 - ax) * ay * 32, ax * ay * 32};
+            for (int c = 0; c < 3; c++) {
+                int acc = 0;
+                for (int t = 0; t < 4; t++) {
+                    const int xx = sx + (t & 1), yy = sy + (t >> 1);
+                    acc += ((xx >= 0 && xx < W && yy >= 0 && yy < H) ? src[((size_t)yy * W + xx) * 3 + c] : 0) * wt[t];
+                }
+                acc = (acc + (1 << 14)) >> 15;
+                dst[o * 3 + c] = (uint8_t)(acc < 0 ? 0 : (acc > 255 ? 255 : acc));
+            }
+        }
+    free(sxy); free(frac);
+    return rc;
 }

@@ -16,6 +16,10 @@ What it writes
   human_literal.npz     voxel-view, VoxelCarving.cpp:39-55; colour pass
                         ColorReconstruction.h:34-74 + .cpp:22-70) on small grids.
   soft_box_1off.json    header numbers of Data/box_dataset/generated_models/1.off.
+  undistort_kat.npz     cv2.undistort known answers on dataset images and a few calibrations.
+  undistort_hostile_kat.npz  cv2.undistort on seeded noise images over hostile calibrations and
+                        sizes (`python tools/make_goldens.py undistort_hostile` writes only this
+                        file; it needs cv2 4.13.0 and undistort_kat.npz, not the datasets).
 
 Pose recipe follows PoseEstimation.h:18-76 using the cv2>=4.7 aruco API (the legacy
 free functions are gone from 4.13): detectMarkers -> interpolateCornersCharuco ->
@@ -289,8 +293,77 @@ def undistort_kat():
     print(f"  undistort_kat.npz: {len(cases)} cases (cv2 {cv2.__version__})")
 
 
+def undistort_hostile_cases():
+    """(name, W, H, K, dist, seed) of the undistort sweep: the dataset calibration at three sizes, random calibrations, round-number
+    K that put many map coordinates on rounding ties, distortion strong enough to leave int16 and int32, a rational denominator
+    that reaches 0 inside the image, and widths for every column count of the scalar tail (W % 8) and for the 4096 / W stripes."""
+    z = np.load(os.path.join(OUT, "undistort_kat.npz"))
+    K0, d0 = z["box_mask0000_K"], z["box_mask0000_dist"].ravel()  # Data/box_dataset/cameracalibration.yml
+    Km = lambda fx, fy, cx, cy, skew=0.0: np.array([[fx, skew, cx], [0, fy, cy], [0, 0, 1.0]])
+    cases = [("dataset_640x480", 640, 480, K0, d0)]
+    for f, (W, H) in [(3, (1920, 1080)), (6, (3840, 2160))]:
+        cases.append((f"dataset_{W}x{H}", W, H, K0 * [[f], [f], [1]], d0))
+    rng = np.random.default_rng(2026)
+    for t, n in enumerate([4, 5, 8, 4, 5, 8]):
+        W, H = int(rng.integers(60, 700)), int(rng.integers(30, 500))
+        f = rng.uniform(0.5, 2) * W
+        K = Km(f, f * rng.uniform(0.9, 1.1), W / 2 + rng.normal() * W / 10, H / 2 + rng.normal() * H / 10, rng.normal() * 2)
+        cases.append((f"random{t}_n{n}", W, H, K, rng.normal(size=n) * np.array([0.3, 0.5, 0.01, 0.01, 0.5, 0.3, 0.3, 0.3])[:n]))
+    ties = [("tie_500_k1", 640, 480, Km(500, 500, 320, 240), [0.25, 0, 0, 0]),
+            ("tie_512_k1k2", 643, 480, Km(512, 512, 320, 240), [0.25, -0.125, 0, 0]),
+            ("tie_512_tangential", 645, 481, Km(512, 512, 320, 240), [0, 0, 1 / 64, -1 / 32]),
+            ("tie_512_rational", 647, 479, Km(512, 512, 320, 240), [0, 0, 0, 0, 0, 0.125, -0.0625, 0.03125]),
+            ("tie_500_zero", 641, 477, Km(500, 500, 320, 240), [0, 0, 0, 0, 0])]
+    strong = [("int16_k3", 100, 40, Km(100, 100, 50, 20), [5, 500, 0, 0, 1e5]),      # |u| past 2^15
+              ("int16_tail", 1001, 77, Km(100, 100, 500, 38), [5, 50, 0.1, 0.1, 500]),
+              ("int32_k3", 103, 40, Km(100, 100, 50, 20), [5, 500, 0, 0, 1e9]),      # u * 32 past 2^31
+              ("int32_tail", 1001, 61, Km(100, 100, 0, 30), [5, 50, 0.1, 0.1, 500]),
+              ("den0_tail", 101, 41, Km(100, 100, 50, 20), [0, 0, 0, 0, 0, -4, 0, 0]),  # 1 + k4 r2 = 0 at column 100
+              ("den0_body", 104, 41, Km(100, 100, 4, 20), [0, 0, 0, 0, 0, -4, 0, 0]),   # ... at column 54
+              ("den0_wide", 333, 211, Km(120, 121, 166, 105), [0.1, 0, 0, 0, 0, -3, 0.5, 0.1])]
+    cases += [(n, W, H, K, np.array(d, np.float64)) for n, W, H, K, d in ties + strong]
+    for r in range(8):  # every W % 8, twice, with a strong random calibration
+        for W in (8 * int(rng.integers(1, 6)) + r, 8 * int(rng.integers(20, 90)) + r):
+            W = max(W, 1)
+            H = int(rng.integers(1, 90))
+            f = rng.uniform(0.3, 1.5) * W
+            n = int(rng.choice([4, 5, 8]))
+            d = rng.normal(size=n) * np.array([0.5, 0.5, 0.05, 0.05, 1, 0.5, 0.5, 0.5])[:n] * float(rng.choice([1, 10]))
+            cases.append((f"w{W}_h{H}", W, H, Km(f, f * rng.uniform(0.95, 1.05), rng.uniform(0, W), rng.uniform(0, H), rng.normal()), d))
+    cases += [("w1", 1, 300, Km(100, 100, 0, 150), np.array([0.3, 0.1, 0, 0])),
+              ("h1", 300, 1, Km(100, 100, 150, 0), np.array([0.3, 0.1, 0.01, 0])),
+              ("w1_h1", 1, 1, Km(2, 2, 0.5, 0.5), np.array([0.3, 0.1, 0, 0])),
+              ("stripe40_h77", 100, 77, Km(80, 80, 50, 38), np.array([-0.2, 0.05, 0.001, 0.002, 0.01])),   # stripe 40
+              ("stripe13_h50", 300, 50, Km(250, 250, 150, 25), np.array([0.2, -0.1, 0, 0])),              # stripe 13
+              ("stripe1_w5000", 5000, 3, Km(2500, 2500, 2500, 1.5), np.array([0.1, -0.05, 0.001, 0, 0.02])),
+              ("w32766", 32766, 2, Km(16000, 16000, 16383, 1), np.array([0.3, 0.1, 0, 0]))]
+    return [(n, W, H, np.asarray(K, np.float64), np.asarray(d, np.float64), 1000 + i) for i, (n, W, H, K, d) in enumerate(cases)]
+
+
+def undistort_hostile_kat():
+    """cv2.undistort over undistort_hostile_cases() on noise images from the seeds: the SHA-256 of every input and output, the
+    output itself for the cases of at most 20000 pixels, and the cv2 version and CPU path the answers came from."""
+    cases = undistort_hostile_cases()
+    out = {"names": np.array([c[0] for c in cases]), "cv2_version": np.array(cv2.__version__),
+           "dispatch": np.array("AVX2" if cv2.checkHardwareSupport(11) else "baseline")}
+    for name, W, H, K, d, seed in cases:
+        img = np.random.default_rng(seed).integers(0, 256, (H, W, 3), dtype=np.uint8)
+        ref = cv2.undistort(img, K, d)
+        out[f"{name}_WHseed"] = np.array([W, H, seed], np.int64)
+        out[f"{name}_K"], out[f"{name}_dist"] = K, d
+        out[f"{name}_src_sha256"] = np.array(hashlib.sha256(img.tobytes()).hexdigest())
+        out[f"{name}_sha256"] = np.array(hashlib.sha256(ref.tobytes()).hexdigest())
+        if W * H <= 20000:
+            out[f"{name}_dst"] = ref
+    np.savez_compressed(os.path.join(OUT, "undistort_hostile_kat.npz"), **out)
+    print(f"  undistort_hostile_kat.npz: {len(cases)} cases (cv2 {cv2.__version__}, {out['dispatch']})")
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
+    if sys.argv[1:] == ["undistort_hostile"]:
+        undistort_hostile_kat()
+        return
     print("cv2", cv2.__version__)
     box = build_cache("box_dataset")
     human = build_cache("human_dataset")
@@ -299,6 +372,7 @@ def main():
     literal_run(human, 20, 24, 28, 0.011, "human_literal.npz")
     soft_golden()
     undistort_kat()
+    undistort_hostile_kat()
     for f in sorted(os.listdir(OUT)):
         p = os.path.join(OUT, f)
         print(f"  {f:24s} {os.path.getsize(p):9d} B sha256={hashlib.sha256(open(p,'rb').read()).hexdigest()[:16]}")
