@@ -2126,7 +2126,7 @@ int vc_format_g(int32_t device, uint64_t n, const float* values, char* text, uin
 }
 
 int vc_selftest(int32_t device, int32_t which, uint64_t n, uint64_t seed, uint64_t* mismatches, uint64_t* checked) {
-    if (!mismatches || !checked || which < 0 || which > 1) return VC_ERR_ARG;
+    if (!mismatches || !checked || which < 0 || which > 2) return VC_ERR_ARG;
     if (cudaSetDevice(device) != cudaSuccess) return fail(nullptr, VC_ERR_CUDA, "vc_selftest: cudaSetDevice(%d) failed", device);
     unsigned long long* d = nullptr;
     if (cudaMalloc(&d, 16) != cudaSuccess) return fail(nullptr, VC_ERR_CUDA, "vc_selftest: cudaMalloc failed");

@@ -541,7 +541,7 @@ def measure_peaks(device=0):
 
 
 def selftest(which, n, seed=0, device=0):
-    """GPU self-test of the arithmetic shortcuts (0: shared-reciprocal divide, 1: pixel index). -> (mismatches, checked)"""
+    """GPU self-test of the arithmetic shortcuts (0: shared-reciprocal divide, 1: pixel index, 2: packed f32 pairs). -> (mismatches, checked)"""
     lib = L.load()
     a, b = C.c_uint64(), C.c_uint64()
     rc = lib.vc_selftest(int(device), int(which), int(n), int(seed), C.byref(a), C.byref(b))

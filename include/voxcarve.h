@@ -347,7 +347,8 @@ VC_EXPORT int vc_format_g(int32_t device, uint64_t n, const float* values, char*
  * (2 flops per FMA), timed with CUDA events, best of 5. Not part of the carve path. */
 VC_EXPORT int vc_measure_peaks(int32_t device, double* ffma_tflops, double* dfma_tflops);
 /* GPU self-test of the kernel's arithmetic shortcuts over n pseudo-random inputs:
- * which = 0 shared-reciprocal f32 divide vs IEEE div.rn; which = 1 pixel index vs (int)roundf + inside().
+ * which = 0 shared-reciprocal f32 divide vs IEEE div.rn; which = 1 pixel index vs (int)roundf + inside();
+ * which = 2 packed f32 pairs (fma / add / mul .rn.f32x2, both halves) vs the scalar IEEE operations.
  * Returns the number of disagreements and of cases compared. */
 VC_EXPORT int vc_selftest(int32_t device, int32_t which, uint64_t n, uint64_t seed, uint64_t* mismatches, uint64_t* checked);
 
