@@ -56,6 +56,7 @@ SIGNATURES = {
     "vc_carve_download_sparse": (C.c_int, [_P, _P, C.c_uint64, _P, _P, C.c_uint64, C.POINTER(C.c_uint64)]),
     "vc_fast_carve": (C.c_int, [_P, C.c_int32]),
     "vc_color": (C.c_int, [_P, C.c_int32]),
+    "vc_color_visible": (C.c_int, [_P, C.c_int32, C.c_float]),
     "vc_mc_classify": (C.c_int, [_P]),
     "vc_plan_slabs": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int32)]),
     "vc_set_slab": (C.c_int, [_P, C.c_int32, C.c_int32]),

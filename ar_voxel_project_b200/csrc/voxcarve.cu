@@ -1582,22 +1582,12 @@ static int need_halo(vc_engine* e, const char* who) {
                 who, e->g.z_begin, e->g.z_end, e->g.Z);
 }
 
-int vc_color(vc_engine* e, int32_t color_mode) {
-    if (!e) return VC_ERR_ARG;
-    PhaseRange nvtx("Coloring");
-    if (color_mode != VC_COLOR_CLOSEST && color_mode != VC_COLOR_AVG) return fail(e, VC_ERR_ARG, "vc_color: mode must be 1 (closest) or 2 (average), got %d", color_mode);
-    if (e->V == 0 || !e->d_images) return fail(e, VC_ERR_STATE, "vc_color: views and images must be set first");
-    if (!e->have_M) return fail(e, VC_ERR_STATE, "vc_color: vc_set_views was given M = NULL (camera translations are needed for the depth)");
-    int rc = need_halo(e, "vc_color");
-    if (rc) return rc;
-    if (bind_device(e)) return VC_ERR_CUDA;
-    rc = materialize_reset(e);
-    if (rc) return rc;
-    const bool global_views = e->V > VC_MAX_VIEWS;  // one pass over every group: P and camera from global memory
-    if (!global_views) { rc = ensure_constants(e); if (rc) return rc; }
+// The surface records of the slab (occupied & !isInner, ascending flatten index) into d_color_idx / n_surface: a counting
+// pass, a scan of the block counts, and an emitting pass.  Clears have_colors first; the caller sets it once its colours are in.
+static int build_surface_records(vc_engine* e, const char* who) {
     const long long n = e->slab_words;
-    if (n > 0x7fffffffLL) return fail(e, VC_ERR_ARG, "vc_color: slab of %lld words too large", n);
-    if (e->nz > 65535) return fail(e, VC_ERR_ARG, "vc_color: slab of %d planes too deep (grid dimension limit 65535)", e->nz);
+    if (n > 0x7fffffffLL) return fail(e, VC_ERR_ARG, "%s: slab of %lld words too large", who, n);
+    if (e->nz > 65535) return fail(e, VC_ERR_ARG, "%s: slab of %d planes too deep (grid dimension limit 65535)", who, e->nz);
     const unsigned chunks = (unsigned)((e->plane_words + 1023) / 1024);  // blocks of vc_surface_pass_kernel per plane
     const int nb = (int)(chunks * (unsigned)e->nz);
     const dim3 sgrid(chunks, (unsigned)e->nz);
@@ -1611,7 +1601,7 @@ int vc_color(vc_engine* e, int32_t color_mode) {
     unsigned long long total = 0;
     VC_CUDA(e, cudaMemcpyAsync(&total, e->d_block_sums + nb, sizeof total, cudaMemcpyDeviceToHost, e->stream));
     VC_CUDA(e, cudaStreamSynchronize(e->stream));
-    if (total > 0xffffffffull) return fail(e, VC_ERR_CAPACITY, "vc_color: %llu surface voxels exceed 32-bit offsets", total);
+    if (total > 0xffffffffull) return fail(e, VC_ERR_CAPACITY, "%s: %llu surface voxels exceed 32-bit offsets", who, total);
     e->n_surface = total;
     if (total) {
         if (total > e->color_capacity) {
@@ -1621,17 +1611,42 @@ int vc_color(vc_engine* e, int32_t color_mode) {
             VC_CUDA(e, cudaMalloc(&e->d_color_rgbn, total * sizeof(uchar4)));
             e->color_capacity = total;
         }
-        VcColorParams p{};
-        p.images = e->d_images;
-        p.idx_out = e->d_color_idx; p.rgbn_out = e->d_color_rgbn;
-        p.X = e->g.X; p.Y = e->g.Y; p.Wx = e->Wx; p.z_begin = e->g.z_begin;
-        p.W = e->W; p.H = e->H; p.V = e->V;
-        p.s = e->g.voxel_size;
-        p.mode = color_mode;
-        p.n_surface = total;
-        p.gview = e->d_view64; p.gcam = e->d_cam;
         vc_surface_pass_kernel<true><<<sgrid, 256, 0, e->stream>>>(g, e->g.z_begin, (unsigned)e->plane_words, e->d_block_sums, e->d_color_idx);
-        const unsigned cgrid = (unsigned)((total + 255) / 256);
+    }
+    return VC_OK;
+}
+
+static VcColorParams color_params(const vc_engine* e, int color_mode) {
+    VcColorParams p{};
+    p.images = e->d_images;
+    p.idx_out = e->d_color_idx; p.rgbn_out = e->d_color_rgbn;
+    p.X = e->g.X; p.Y = e->g.Y; p.Wx = e->Wx; p.z_begin = e->g.z_begin;
+    p.W = e->W; p.H = e->H; p.V = e->V;
+    p.s = e->g.voxel_size;
+    p.mode = color_mode;
+    p.n_surface = e->n_surface;
+    p.gview = e->d_view64; p.gcam = e->d_cam;
+    return p;
+}
+
+int vc_color(vc_engine* e, int32_t color_mode) {
+    if (!e) return VC_ERR_ARG;
+    PhaseRange nvtx("Coloring");
+    if (color_mode != VC_COLOR_CLOSEST && color_mode != VC_COLOR_AVG) return fail(e, VC_ERR_ARG, "vc_color: mode must be 1 (closest) or 2 (average), got %d", color_mode);
+    if (e->V == 0 || !e->d_images) return fail(e, VC_ERR_STATE, "vc_color: views and images must be set first");
+    if (!e->have_M) return fail(e, VC_ERR_STATE, "vc_color: vc_set_views was given M = NULL (camera translations are needed for the depth)");
+    int rc = need_halo(e, "vc_color");
+    if (rc) return rc;
+    if (bind_device(e)) return VC_ERR_CUDA;
+    rc = materialize_reset(e);
+    if (rc) return rc;
+    const bool global_views = e->V > VC_MAX_VIEWS;  // one pass over every group: P and camera from global memory
+    if (!global_views) { rc = ensure_constants(e); if (rc) return rc; }
+    rc = build_surface_records(e, "vc_color");
+    if (rc) return rc;
+    if (e->n_surface) {
+        const VcColorParams p = color_params(e, color_mode);
+        const unsigned cgrid = (unsigned)((e->n_surface + 255) / 256);
         if (global_views) {
             if (color_mode == VC_COLOR_CLOSEST) vc_surface_color_kernel<1, true><<<cgrid, 256, 0, e->stream>>>(p);
             else vc_surface_color_kernel<2, true><<<cgrid, 256, 0, e->stream>>>(p);
@@ -1639,6 +1654,70 @@ int vc_color(vc_engine* e, int32_t color_mode) {
         } else {
             if (color_mode == VC_COLOR_CLOSEST) vc_surface_color_kernel<1><<<cgrid, 256, 0, e->stream>>>(p);
             else vc_surface_color_kernel<2><<<cgrid, 256, 0, e->stream>>>(p);
+            VC_CUDA(e, cudaGetLastError());
+            rc = constants_used(e);
+            if (rc) return rc;
+        }
+    }
+    e->have_colors = true;
+    return VC_OK;
+}
+
+// Depth buffers of vc_color_visible cover as many views at a time as fit this budget (at least one view).  Every pair is
+// splatted and observed exactly once whatever the chunk, so the records do not depend on it; a chunk only bounds the memory.
+#define VC_VIS_ZBUF_BUDGET (256ull << 20)
+
+int vc_color_visible(vc_engine* e, int32_t color_mode, float tolerance) {
+    if (!e) return VC_ERR_ARG;
+    PhaseRange nvtx("Coloring");
+    // every refusal before any state changes: the previous colour records stay as they were
+    if (color_mode != VC_COLOR_CLOSEST && color_mode != VC_COLOR_AVG) return fail(e, VC_ERR_ARG, "vc_color_visible: mode must be 1 (closest) or 2 (average), got %d", color_mode);
+    if (!(tolerance >= 0.0f)) return fail(e, VC_ERR_ARG, "vc_color_visible: tolerance must be >= 0 (voxel sizes), got %g", (double)tolerance);
+    if (!e->whole_grid()) return fail(e, VC_ERR_STATE, "vc_color_visible: whole-grid engines only (slab [%d,%d) of Z=%d: occluders in other slabs are unknown)", e->g.z_begin, e->g.z_end, e->g.Z);
+    if (e->V == 0 || !e->d_images) return fail(e, VC_ERR_STATE, "vc_color_visible: views and images must be set first");
+    if (!e->have_M) return fail(e, VC_ERR_STATE, "vc_color_visible: vc_set_views was given M = NULL (camera translations are needed for the depth)");
+    if (bind_device(e)) return VC_ERR_CUDA;
+    int rc = materialize_reset(e);
+    if (rc) return rc;
+    const bool global_views = e->V > VC_MAX_VIEWS;
+    if (!global_views) { rc = ensure_constants(e); if (rc) return rc; }
+    rc = build_surface_records(e, "vc_color_visible");
+    if (rc) return rc;
+    const unsigned long long total = e->n_surface;
+    if (total) {
+        const size_t view_px = (size_t)e->W * e->H;
+        const unsigned long long vis_words = (total + 31) / 32;
+        const size_t vis_bytes = (size_t)vis_words * 4 * e->V;
+        const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)e->V, VC_VIS_ZBUF_BUDGET / (view_px * 4)));
+        void* sc = nullptr;
+        rc = ensure_scratch(e, vis_bytes + (size_t)chunk * view_px * 4, &sc);
+        if (rc) return rc;
+        VcVisParams vp{};
+        vp.idx = e->d_color_idx; vp.view = e->d_view64;
+        vp.vis = (uint32_t*)sc; vp.zbuf = (uint32_t*)((char*)sc + vis_bytes);
+        vp.n_surface = total; vp.vis_words = vis_words;
+        vp.X = e->g.X; vp.Y = e->g.Y; vp.W = e->W; vp.H = e->H;
+        vp.s = e->g.voxel_size;
+        vp.tau = tolerance * e->g.voxel_size;  // fl(tolerance * s)
+        const unsigned bx = (unsigned)((total + 255) / 256);
+        for (int v0 = 0; v0 < e->V; v0 += chunk) {
+            const int nv = std::min(chunk, e->V - v0);
+            vp.v0 = v0;
+            // 0xffffffff is above the bits of every key (+inf included) and is read nowhere: a pair reads its own centre pixel
+            VC_CUDA(e, cudaMemsetAsync(vp.zbuf, 0xff, (size_t)nv * view_px * 4, e->stream));
+            vc_vis_splat_kernel<<<dim3(bx, (unsigned)nv), 256, 0, e->stream>>>(vp);
+            vc_vis_observe_kernel<<<dim3(bx, (unsigned)nv), 256, 0, e->stream>>>(vp);
+            VC_CUDA(e, cudaGetLastError());
+        }
+        VcColorParams p = color_params(e, color_mode);
+        p.vis = vp.vis; p.vis_words = vis_words;
+        if (global_views) {
+            if (color_mode == VC_COLOR_CLOSEST) vc_surface_color_kernel<1, true, true><<<bx, 256, 0, e->stream>>>(p);
+            else vc_surface_color_kernel<2, true, true><<<bx, 256, 0, e->stream>>>(p);
+            VC_CUDA(e, cudaGetLastError());
+        } else {
+            if (color_mode == VC_COLOR_CLOSEST) vc_surface_color_kernel<1, false, true><<<bx, 256, 0, e->stream>>>(p);
+            else vc_surface_color_kernel<2, false, true><<<bx, 256, 0, e->stream>>>(p);
             VC_CUDA(e, cudaGetLastError());
             rc = constants_used(e);
             if (rc) return rc;

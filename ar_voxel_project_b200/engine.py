@@ -297,6 +297,11 @@ class VoxelEngine:
     def color(self, mode):
         self._check(self._lib.vc_color(self._h, int(mode)))
 
+    def color_visible(self, mode, tolerance=2.0):
+        """occlusion-aware colouring (vc_color_visible): each surface voxel is coloured from the views that see it; a view is
+        occluded when another surface voxel lies more than `tolerance` voxel sizes in front of it.  Whole-grid engines only."""
+        self._check(self._lib.vc_color_visible(self._h, int(mode), float(tolerance)))
+
     def mc_classify(self):
         self._check(self._lib.vc_mc_classify(self._h))
 

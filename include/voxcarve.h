@@ -201,6 +201,31 @@ VC_EXPORT int vc_fast_carve(vc_engine* e, int32_t mode);
 /* reconstructClosestColor / reconstructAvgColor (ColorReconstruction.h:131,142): colours every
  * surface voxel (alpha != 0 && !isInner, ColorReconstruction.h:46) of this slab. */
 VC_EXPORT int vc_color(vc_engine* e, int32_t color_mode);
+/* Occlusion-aware colouring: like vc_color, but a surface voxel takes its colour only from the views that see it.  The records
+ * are those of vc_color (same voxels, same order, rgbn.w = min(#observations, 255), MODEL_COLOR with n = 0 when no view
+ * observes the voxel), so vc_surface_count, vc_download_colors and apply_colors of vc_dense_from_volumes / vc_mesh_from_volumes
+ * take them unchanged.  For each surface voxel (x, y, z) and view v:
+ *   1. Sample points: the voxel and its 8 corners (x +- 1/2, y +- 1/2, z +- 1/2), world w = (fl(y' s), fl(x' s), fl(-z' s), 1)
+ *      in f32, each projected with the carve's arithmetic (f64 sequential accumulation rounded once to f32 p0, p1, p2; IEEE f32
+ *      u = p0/p2, v = p1/p2).  The centre's projection is exactly vc_color's.
+ *   2. The pair is eligible iff all 9 points have p2 > 0 and finite u, v (the reference has no depth test and point-reflects
+ *      voxels behind the camera; here they neither occlude nor observe).
+ *   3. key = min of the 9 p2; rectangle = [round(min u), round(max u)] x [round(min v), round(max v)], round half away from
+ *      zero, clipped to the image.
+ *   4. Depth buffer per view: zbuf = min(zbuf, key) over every eligible pair and every pixel of its rectangle, from +inf
+ *      (order-independent, so the result is deterministic).
+ *   5. An eligible pair observes iff its centre pixel (vc_color's pixel) is inside the image and
+ *      key <= fl(zbuf[pixel] + tau), tau = fl(tolerance * voxel_size).  A voxel never hides itself (tolerance >= 0).
+ *   6. The colour bodies of vc_color run unchanged over the observations only, in view order.
+ * tolerance is in voxel sizes.  For P = K [R|t] with K's last row (0, 0, 1), p2 is the camera-space depth in world units, so
+ * the tolerance is a depth distance; 2 (the default of the bindings) lets neighbouring voxels of one surface, whose depths
+ * differ by up to sqrt(3) voxels, see past each other's corners.  tolerance = +inf keeps every eligible pair whose centre is
+ * in the image: where every camera has the whole grid in front of it, that is exactly vc_color.
+ * Memory: the records, V * ceil(n_surface / 32) words of observation bits, and depth buffers (4 W H bytes per view) for as many
+ * views at a time as 256 MiB holds (at least one); the results do not depend on that chunking.  Works with any number of views.
+ * VC_ERR_ARG: mode not 1 or 2, tolerance NaN or negative.  VC_ERR_STATE: a slab engine (whole grid only: occluders in other
+ * slabs are unknown), no views or images, or views without M.  These refusals leave the previous records as they were. */
+VC_EXPORT int vc_color_visible(vc_engine* e, int32_t color_mode, float tolerance);
 /* Cube-index classification of marchingCubes() (MarchingCubes.cpp:12-18, MarchingCubes.h:479-488,
  * :537-552) for the cells whose lower z-plane lies in this slab (plus z = -1 on the first slab). */
 VC_EXPORT int vc_mc_classify(vc_engine* e);

@@ -131,6 +131,8 @@ class Engine {
     }
     void fastCarve(int mode = VC_EXACT) { check(vc_fast_carve(h_, mode)); }
     void color(int mode) { check(vc_color(h_, mode)); }
+    // occlusion-aware colouring (vc_color_visible): a surface voxel takes its colour only from the views that see it
+    void colorVisible(int mode, float tolerance = 2.0f) { check(vc_color_visible(h_, mode, tolerance)); }
     McSummary mcClassify() {
         McSummary s{};
         check(vc_mc_classify(h_));
@@ -531,13 +533,16 @@ bool marchingCubes(ModelT* model, float scale = 1.0f, const float* translation =
 // reconstructAvgColor (2)] -> handleUnseen -> [applyClosure(closureK), closureK = 0: none] -> marchingCubes(scale, translation,
 // threshold).  The volumes, colour records and mesh stay on the device, and the .off text is formatted there too, so grids whose
 // dense Model does not fit the GPU (2048^3: 128 GiB) are meshed too, and only the file's bytes cross PCIe.  Returns false if the file cannot be written.
+// visibilityTolerance = nullptr colours as the reference does (every view whose image holds the voxel's pixel); a tolerance in
+// voxel sizes colours each surface voxel from the views that see it (vc_color_visible).
 inline bool carveToMesh(const ViewCache& views, int X, int Y, int Z, float size, int colorMode, int closureK, float scale = 1.0f,
                         const float* translation = nullptr, float threshold = 0.5f, const std::string& outFileName = "out/mesh.off",
-                        int device = 0) {
+                        int device = 0, const float* visibilityTolerance = nullptr) {
     Engine e(X, Y, Z, size, 0, -1, device);
     e.setViews(views, colorMode != 0);
     e.carve();
-    if (colorMode) e.color(colorMode);
+    if (colorMode && visibilityTolerance) e.colorVisible(colorMode, *visibilityTolerance);
+    else if (colorMode) e.color(colorMode);
     e.meshFromVolumes(colorMode != 0, true, closureK, threshold);
     const float tx = translation ? translation[0] : 0.f, ty = translation ? translation[1] : 0.f, tz = translation ? translation[2] : 0.f;
     if (!detail::writeOff(e, outFileName, scale * size, tx, ty, tz)) {
