@@ -1378,6 +1378,9 @@ int vc_fast_carve(vc_engine* e, int32_t mode) {
     if (!e) return VC_ERR_ARG;
     PhaseRange nvtx("Carving");
     if (!e->whole_grid()) return fail(e, VC_ERR_STATE, "vc_fast_carve: the flood from voxel (0,0,0) needs the whole grid on one engine (slab [%d,%d) of Z=%d)", e->g.z_begin, e->g.z_end, e->g.Z);
+    // refusals before the reset below: a refused call leaves the volumes as they were
+    if (mode != VC_EXACT && mode != VC_FAST_F32 && mode != VC_EXACT_FLAT) return fail(e, VC_ERR_ARG, "vc_fast_carve: unknown mode %d", mode);
+    if (e->V == 0 || !e->d_mask) return fail(e, VC_ERR_STATE, "vc_fast_carve: views and masks must be set first");
     // the set carve() would carve, on a fresh Model (fastCarve starts from the constructor state, main.cpp:248-264)
     int rc = vc_reset(e);
     if (rc) return rc;

@@ -107,7 +107,9 @@ VC_EXPORT void vc_destroy(vc_engine* e);
 /* message of the last failed call on `e`; with e == NULL, of the last failed vc_create */
 VC_EXPORT const char* vc_last_error(const vc_engine* e);
 VC_EXPORT int vc_api_version(void);
-/* run all work of this engine on a caller stream (cudaStream_t as void*; NULL = engine's own) */
+/* run all work of this engine on a caller stream (cudaStream_t as void*; NULL = engine's own).  The engine's own stream does
+ * not synchronise with other streams, so a caller whose producers (e.g. of device masks) run on its own stream passes that
+ * stream here: device pointers are read in the order of the engine's stream only. */
 VC_EXPORT int vc_set_stream(vc_engine* e, void* cuda_stream);
 VC_EXPORT int vc_synchronize(vc_engine* e);
 /* Profiling mode (off by default).  Off: a whole-range VC_EXACT carve is launched as ONE cached CUDA graph (counter reset + the
@@ -151,7 +153,8 @@ VC_EXPORT int vc_append_views(vc_engine* e, int32_t n, const float* P, const flo
 /* Undistorted silhouette masks (VoxelCarving.cpp:36). VC_MASK_BITS: uint32[V][H][ceil(W/32)],
  * bit x&31 of word x>>5, 1 = background (pixel == (0,0,0), VoxelCarving.cpp:50).
  * VC_MASK_BGR8: the 8UC3 images themselves, uint8[V][H][W][3]; packed on the device. HOST memory (VC_MASK_BITS also takes a
- * DEVICE pointer: silhouettes that a segmentation stage left on the GPU).  Builds the summed-area tables of the silhouettes that
+ * DEVICE pointer: silhouettes that a segmentation stage left on the GPU; it is read in the order of the engine's stream only, so
+ * their producer runs on that stream, vc_set_stream, or the caller synchronises first).  Builds the summed-area tables of the silhouettes that
  * VC_EXACT's classifier reads (a copy + two kernels, C4: 0.16 ms). */
 VC_EXPORT int vc_set_masks(vc_engine* e, const void* masks, int32_t format);
 /* Undistorted colour images 8UC3 BGR (ColorReconstruction.h:23), uint8[V][H][W][3], HOST memory. */
@@ -196,7 +199,8 @@ VC_EXPORT int vc_sparse_dims(const vc_engine* e, uint32_t* nbx, uint32_t* nby, u
 VC_EXPORT int vc_carve_download_sparse(vc_engine* e, uint8_t* brick_flags, uint64_t flags_capacity, uint32_t* listed, uint32_t* words,
                                        uint64_t listed_capacity, uint64_t* n_listed);
 /* fastCarve() (VoxelCarving.h:31, VoxelCarving.cpp:74-167): starts from the Model constructor state (it resets the
- * volumes itself) and needs the whole grid on this engine. */
+ * volumes itself) and needs the whole grid on this engine.  Refused (a slab engine, no views or masks, an unknown mode), it
+ * leaves the volumes as they were. */
 VC_EXPORT int vc_fast_carve(vc_engine* e, int32_t mode);
 /* reconstructClosestColor / reconstructAvgColor (ColorReconstruction.h:131,142): colours every
  * surface voxel (alpha != 0 && !isInner, ColorReconstruction.h:46) of this slab. */
