@@ -98,6 +98,8 @@ SIGNATURES = {
     "vc_download_mesh_off": (C.c_int, [_P, C.c_uint64, _P, C.c_uint64]),
     "vc_format_g": (C.c_int, [C.c_int32, C.c_uint64, _P, _P, C.c_uint64, C.POINTER(C.c_uint64)]),
     "vc_selftest": (C.c_int, [C.c_int32, C.c_int32, C.c_uint64, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+    "vc_probe_boxes": (C.c_int, [_P, C.c_uint64, _P, _P]),
+    "vc_probe_voxels": (C.c_int, [_P, C.c_uint64, _P, _P]),
     "vc_measure_peaks": (C.c_int, [C.c_int32, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
 }
 

@@ -2223,6 +2223,50 @@ int vc_selftest(int32_t device, int32_t which, uint64_t n, uint64_t seed, uint64
     return VC_OK;
 }
 
+// vc_probe_boxes / vc_probe_voxels: host records in, one kernel, host records out, on the engine's stream.  Every record is
+// checked before anything is allocated or launched.
+static int probe_run(vc_engine* e, const char* what, uint64_t n, const int32_t* in, int in_words, int32_t* out, int out_words, bool boxes) {
+    if (!e) return VC_ERR_ARG;
+    if (n && (!in || !out)) return fail(e, VC_ERR_ARG, "%s: null buffer", what);
+    if (n > VC_PROBE_MAX) return fail(e, VC_ERR_ARG, "%s: %llu records, more than %llu", what, (unsigned long long)n, (unsigned long long)VC_PROBE_MAX);
+    if (e->V == 0 || !e->d_mask) return fail(e, VC_ERR_STATE, "%s: call vc_set_views and vc_set_masks first", what);
+    const vc_grid_desc& g = e->g;
+    for (uint64_t i = 0; i < n; i++) {
+        const int32_t* r = in + i * in_words;
+        const int32_t lo[3] = {r[1], r[2], r[3]}, hi[3] = {boxes ? r[4] : r[1], boxes ? r[5] : r[2], boxes ? r[6] : r[3]};
+        const int32_t glo[3] = {0, 0, g.z_begin}, ghi[3] = {g.X, g.Y, g.z_end};
+        if (r[0] < 0 || r[0] >= e->V) return fail(e, VC_ERR_ARG, "%s: record %llu: view %d outside [0,%d)", what, (unsigned long long)i, r[0], e->V);
+        for (int k = 0; k < 3; k++)
+            if (lo[k] < glo[k] || hi[k] < lo[k] || hi[k] >= ghi[k])
+                return fail(e, VC_ERR_ARG, "%s: record %llu: %c range [%d,%d] outside [%d,%d) or empty", what, (unsigned long long)i, "xyz"[k], lo[k], hi[k], glo[k], ghi[k]);
+    }
+    if (n == 0) return VC_OK;
+    if (bind_device(e)) return VC_ERR_CUDA;
+    int32_t *d_in = nullptr, *d_out = nullptr;
+    cudaError_t s = cudaMalloc(&d_in, n * in_words * sizeof(int32_t));
+    if (s == cudaSuccess) s = cudaMalloc(&d_out, n * out_words * sizeof(int32_t));
+    if (s == cudaSuccess) s = cudaMemcpyAsync(d_in, in, n * in_words * sizeof(int32_t), cudaMemcpyHostToDevice, e->stream);
+    if (s == cudaSuccess) {
+        const int ni = (int)n, threads = boxes ? ni : (ni + 1) / 2;
+        if (boxes) vc_probe_boxes_kernel<<<(threads + 255) / 256, 256, 0, e->stream>>>(d_in, d_out, ni, e->d_filt, e->d_sat, g.voxel_size, e->W, e->H);
+        else vc_probe_voxels_kernel<<<(threads + 255) / 256, 256, 0, e->stream>>>(d_in, d_out, ni, e->d_filt, e->d_view64, g.voxel_size, e->W, e->H, e->hDu, e->hDv);
+        s = cudaGetLastError();
+    }
+    if (s == cudaSuccess) s = cudaMemcpyAsync(out, d_out, n * out_words * sizeof(int32_t), cudaMemcpyDeviceToHost, e->stream);
+    if (s == cudaSuccess) s = cudaStreamSynchronize(e->stream);
+    cudaFree(d_in); cudaFree(d_out);
+    if (s != cudaSuccess) return fail(e, VC_ERR_CUDA, "%s: %s", what, cudaGetErrorString(s));
+    return VC_OK;
+}
+
+int vc_probe_boxes(vc_engine* e, uint64_t n, const int32_t* boxes, int32_t* out) {
+    return probe_run(e, "vc_probe_boxes", n, boxes, 7, out, 5, true);
+}
+
+int vc_probe_voxels(vc_engine* e, uint64_t n, const int32_t* voxels, int32_t* out) {
+    return probe_run(e, "vc_probe_voxels", n, voxels, 4, out, VC_PROBE_VOXEL_OUT, false);
+}
+
 }  // extern "C"
 
 // ---------------------------------------------------------------------------------------------

@@ -500,6 +500,23 @@ class VoxelEngine:
                 f.write(memoryview(buf)[:k])
         return n
 
+    # -- probes (tests) ------------------------------------------------------------------
+    def probe_boxes(self, boxes):
+        """the carve's brick classifier on boxes int32[n, 7] = (view, x0, y0, z0, x1, y1, z1), inclusive, global z (vc_probe_boxes)
+        -> int32[n, 5] = (code, px0, px1, py0, py1)"""
+        b = np.ascontiguousarray(boxes, np.int32).reshape(-1, 7)
+        out = np.zeros((len(b), 5), np.int32)
+        self._check(self._lib.vc_probe_boxes(self._h, len(b), C.c_void_p(b.ctypes.data), C.c_void_p(out.ctypes.data)))
+        return out
+
+    def probe_voxels(self, voxels):
+        """the carve's per-voxel filter and exact evaluation on voxel-views int32[n, 4] = (view, x, y, z), global z (vc_probe_voxels)
+        -> int32[n, 11] = (decided, inside, px, py, exact inside, exact px, exact py, then the bits of Cu, Cv, hDu, hDv)"""
+        v = np.ascontiguousarray(voxels, np.int32).reshape(-1, 4)
+        out = np.zeros((len(v), 11), np.int32)
+        self._check(self._lib.vc_probe_voxels(self._h, len(v), C.c_void_p(v.ctypes.data), C.c_void_p(out.ctypes.data)))
+        return out
+
     def stats(self):
         s = L.Stats()
         self._check(self._lib.vc_get_stats(self._h, C.byref(s)))

@@ -380,6 +380,21 @@ VC_EXPORT int vc_measure_peaks(int32_t device, double* ffma_tflops, double* dfma
  * which = 2 packed f32 pairs (fma / add / mul .rn.f32x2, both halves) vs the scalar IEEE operations.
  * Returns the number of disagreements and of cases compared. */
 VC_EXPORT int vc_selftest(int32_t device, int32_t which, uint64_t n, uint64_t seed, uint64_t* mismatches, uint64_t* checked);
+/* Probes of the exact carve's two approximations, for tests (HOST in / HOST out, on the engine's stream, synchronised).  They run
+ * the compiled code of the carve on records of the caller's choice, with the engine's views (any index in [0, V), including
+ * views past 256), masks, summed-area tables, filter constants, voxel size, W, H and slab.
+ * vc_probe_boxes: boxes[n][7] = (view, x0, y0, z0, x1, y1, z1), inclusive voxel ranges, global z -> out[n][5] = (code, px0, px1,
+ *   py0, py1): the brick classifier's answer (0 undecided, 1 every voxel outside the image, 2 every voxel inside on foreground,
+ *   3 inside on background, 4 inside but not decided by the table) and the pixel rectangle it counted in the table (codes 2-4;
+ *   zeros otherwise).
+ * vc_probe_voxels: voxels[n][4] = (view, x, y, z), global z -> out[n][11] = (decided, inside, px, py) of the per-voxel f32 filter,
+ *   (inside, px, py) of the exact evaluation, and the bit patterns of the view's Cu, Cv and the engine's hDu, hDv.  Pixels are
+ *   meaningful where inside (and, for the filter, decided).
+ * VC_ERR_ARG: a null buffer, more than VC_PROBE_MAX records, a view outside [0, V), a range outside the grid or the slab, or
+ * x1 < x0 (y, z alike).  VC_ERR_STATE: no views or no masks.  Nothing is launched on a refused call. */
+#define VC_PROBE_MAX (1ull << 26)
+VC_EXPORT int vc_probe_boxes(vc_engine* e, uint64_t n, const int32_t* boxes, int32_t* out);
+VC_EXPORT int vc_probe_voxels(vc_engine* e, uint64_t n, const int32_t* voxels, int32_t* out);
 
 #ifdef __cplusplus
 }

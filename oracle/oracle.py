@@ -43,6 +43,7 @@ def lib():
         L.vo_mc_classify.argtypes = [C.c_int] * 3 + [u32p, u8p, u64p, u64p, u64p]
         L.vo_pixel_of.argtypes = [f32p] + [C.c_int] * 3 + [C.c_float, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), f32p]
         L.vo_max_threads.restype = C.c_int
+        L.vo_box_pixel_bounds.argtypes = [f32p, C.c_float] + [C.c_int] * 9 + [np.ctypeslib.ndpointer(np.int32, flags="C_CONTIGUOUS")]
         L.vo_undistort.argtypes = [C.c_int, C.c_int, u8p, np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS"),
                                    np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS"), C.c_int, u8p]
         L.vo_undistort_map.argtypes = [C.c_int, C.c_int, np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS"),
@@ -80,6 +81,18 @@ def pixel_of(P, x, y, z, s, W, H):
     uv = np.empty(2, np.float32)
     ins = lib().vo_pixel_of(np.ascontiguousarray(P, np.float32), x, y, z, float(np.float32(s)), W, H, C.byref(px), C.byref(py), uv)
     return bool(ins), px.value, py.value, uv
+
+
+def box_pixel_bounds(P, lo, hi, s, W, H, nthreads=0):
+    """the reference's pixels over EVERY voxel of the box [lo, hi] (inclusive x, y, z) -> (all_inside, none_inside, px_min,
+    px_max, py_min, py_max, bad_depth): bad_depth = some voxel's proj_2 is <= 0 or not finite; NaN or out-of-range coordinates
+    count as INT32_MIN.  nthreads < 1: every core"""
+    out = np.empty(7, np.int32)
+    rc = lib().vo_box_pixel_bounds(np.ascontiguousarray(P, np.float32).reshape(12), float(np.float32(s)), int(W), int(H),
+                                   *(int(c) for c in lo), *(int(c) for c in hi), int(nthreads), out)
+    if rc != 0:
+        raise ValueError(f"empty box {lo} {hi}")
+    return bool(out[0]), bool(out[1]), int(out[2]), int(out[3]), int(out[4]), int(out[5]), bool(out[6])
 
 
 def _mask_args(mask_bits, mask_bgr):

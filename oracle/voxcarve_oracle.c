@@ -153,6 +153,72 @@ VO_API int vo_max_threads(void) {
     return n < 1 ? 1 : (int)n;
 }
 
+/* What the reference computes for every voxel of a box, summarised: [0] every voxel inside the image, [1] none inside,
+ * [2..5] min / max of px and of py (INT32_MIN for NaN / out-of-range coordinates, as vo_round_to_int), [6] some voxel has a
+ * depth proj_2 <= 0 or not finite. */
+typedef struct {
+    const float* P;
+    float s;
+    int W, H, x0, y0, x1, y1, z1;
+    atomic_int next_z;
+    pthread_mutex_t lock;
+    int32_t acc[7];
+} bounds_job;
+
+static void bounds_fold(int32_t* acc, const int32_t* b) {
+    acc[0] &= b[0]; acc[1] &= b[1]; acc[6] |= b[6];
+    for (int k = 2; k < 6; k += 2) {
+        if (b[k] < acc[k]) acc[k] = b[k];
+        if (b[k + 1] > acc[k + 1]) acc[k + 1] = b[k + 1];
+    }
+}
+
+static void* bounds_worker(void* arg) {
+    bounds_job* j = (bounds_job*)arg;
+    int32_t b[7] = {1, 1, INT32_MAX, INT32_MIN, INT32_MAX, INT32_MIN, 0};
+    for (;;) {
+        int z = atomic_fetch_add(&j->next_z, 1);
+        if (z > j->z1) break;
+        for (int y = j->y0; y <= j->y1; y++)
+            for (int x = j->x0; x <= j->x1; x++) {
+                float w[4], p[3];
+                int px, py;
+                vo_world(x, y, z, j->s, w);
+                vo_project(j->P, w, p);
+                int in = vo_pixel(j->P, x, y, z, j->s, j->W, j->H, &px, &py);
+                b[0] &= in; b[1] &= !in;
+                if (!(p[2] > 0.0f) || !isfinite(p[2])) b[6] = 1;
+                if (px < b[2]) b[2] = px;
+                if (px > b[3]) b[3] = px;
+                if (py < b[4]) b[4] = py;
+                if (py > b[5]) b[5] = py;
+            }
+    }
+    pthread_mutex_lock(&j->lock);
+    bounds_fold(j->acc, b);
+    pthread_mutex_unlock(&j->lock);
+    return NULL;
+}
+
+/* box = voxels [x0, x1] x [y0, y1] x [z0, z1] (inclusive); z-planes split over nthreads pthreads (< 1: all online cores) */
+VO_API int vo_box_pixel_bounds(const float* P, float s, int W, int H, int x0, int y0, int z0, int x1, int y1, int z1, int nthreads, int32_t* out) {
+    if (x1 < x0 || y1 < y0 || z1 < z0) return -1;
+    bounds_job job = {P, s, W, H, x0, y0, x1, y1, z1, 0, PTHREAD_MUTEX_INITIALIZER, {1, 1, INT32_MAX, INT32_MIN, INT32_MAX, INT32_MIN, 0}};
+    atomic_store(&job.next_z, z0);
+    if (nthreads < 1) nthreads = vo_max_threads();
+    if (nthreads > z1 - z0 + 1) nthreads = z1 - z0 + 1;
+    if (nthreads == 1) {
+        bounds_worker(&job);
+    } else {
+        pthread_t* th = (pthread_t*)malloc(sizeof(pthread_t) * nthreads);
+        for (int t = 0; t < nthreads; t++) pthread_create(&th[t], NULL, bounds_worker, &job);
+        for (int t = 0; t < nthreads; t++) pthread_join(th[t], NULL);
+        free(th);
+    }
+    memcpy(out, job.acc, sizeof job.acc);
+    return 0;
+}
+
 /* carve() VoxelCarving.cpp:60-72 on the z-slab [z0,z1) of an X*Y*Z grid. Exactly one of
  * mask_bits / mask_bgr is non-NULL. Outputs bit volumes word[((z-z0)*Y + y)*ceil(X/32) + (x>>5)],
  * bit x&31; occupied starts all-ones (Model.cpp:9-14, alpha = 1), seen all-zero.

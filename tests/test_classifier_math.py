@@ -1,11 +1,15 @@
-"""The error-radius argument behind the conservative (brick, view) classifier, checked on the CPU under far more hostile sampling
-than the GPU parity tests can afford.
+"""The error-radius argument behind the conservative (brick, view) classifier and the per-voxel filter, checked on the CPU under
+far more hostile sampling than the GPU parity tests can afford.  This file checks the DERIVATION, on a numpy restatement of the
+kernels; tests/test_carve_decisions.py checks the compiled CODE (vc_probe_boxes / vc_probe_voxels) on the device.
 
 `rect_of_box` restates `vc_classify_brick_view` (ar_voxel_project_b200/csrc/vc_kernels.cuh: f32 corner projections with an
 approximate reciprocal, error radii in f32, the widened rectangle) in numpy float32; `reference_pixels` restates the reference
 arithmetic (DESIGN.md section 2; checked below against the C oracle voxel by voxel).  Property: whenever the classifier does
 not answer "undecided", the reference pixel of EVERY voxel of the box lies inside the rectangle it hands to the SAT
-(codes 2/3/4), respectively outside the image (code 1).  The restatement is test infrastructure, like oracle/."""
+(codes 2/3/4), respectively outside the image (code 1).  The restatement is test infrastructure, like oracle/.  It is not
+bit-exact with the kernels: it takes the exact 1/q2 where they use rcp.approx.ftz (which also flushes denormal depths) and
+1.12/dmin where they use __fdividef, sums t_i in another order, rounds the Eu chain step by step where the kernel fuses it, and
+emulates an FMA with a double rounding; its answers stand for the derivation, not for the device's."""
 import numpy as np
 import pytest
 
@@ -34,8 +38,9 @@ def reference_pixels(P, xs, ys, zs, s, W, H):
     return px, py, inside
 
 
-def rect_of_box(P, lo, hi, s, W, H):
-    """-> (code, px0, px1, py0, py1): code 0 = undecided, 1 = all outside, 4 = all inside with the pixel rectangle"""
+def rect_of_box(P, lo, hi, s, W, H, zero_radius=False):
+    """-> (code, px0, px1, py0, py1): code 0 = undecided, 1 = all outside, 4 = all inside with the pixel rectangle.
+    zero_radius: Eu = Ev = 0 (an unsound classifier: test_carve_decisions.py shows that its sampling catches it)"""
     Pf = P.astype(F)
     cw = [np.array([F(lo[k]) * s, F(hi[k]) * s], F) for k in range(3)]         # voxel index -> f32 world (x, y, z); z negated below
     cw[2] = np.array([F(-lo[2]) * s, F(-hi[2]) * s], F)
@@ -69,6 +74,8 @@ def rect_of_box(P, lo, hi, s, W, H):
     Ev = F(F(3.0) * F(F(F(e[1] + F(V * e[2])) * rd) + F(V * F(2.3841858e-07))) + F(9.765625e-04))
     if not (Eu < F(0.25) and Ev < F(0.25)):
         return (0,)
+    if zero_radius:
+        Eu = Ev = F(0.0)
     down = lambda a: np.nextafter(F(a), F(-np.inf)); up = lambda a: np.nextafter(F(a), F(np.inf))   # at least as wide as __fadd_rd / _ru
     lo_u, hi_u, lo_v, hi_v = down(us.min() - Eu), up(us.max() + Eu), down(vs.min() - Ev), up(vs.max() + Ev)
     Wm, Hm = F(W) - F(0.5), F(H) - F(0.5)
@@ -195,13 +202,15 @@ def filter_constants(P, dims, s, W, H):
     """vc_filter_constants (voxcarve.cu): radius coefficients Cu, Cv of a view and the thresholds 0.5 - D, all rounded outwards"""
     up = 1.0 + 2.0 ** -22
     ax, ay, az = ((d - 1) * float(s) * up for d in dims)
-    eta = []
+    eta, ok = [], True
     for i in range(3):
         T = abs(float(P[i, 0])) * ay + abs(float(P[i, 1])) * ax + abs(float(P[i, 2])) * az + abs(float(P[i, 3]))
+        ok = ok and np.isfinite(T) and T < 2.0 ** 60   # else the filter is off for the view: Cu = Cv = +inf
         eta.append(4.0 * 2.0 ** -24 * T * (1.0 + 2.0 ** -19) + 2.0 ** -100)
     W3, H3 = W + 3.0, H + 3.0
-    Cu = np.nextafter(F((eta[0] + W3 * eta[2]) * (1.0 + 2.0 ** -19)), F(np.inf))
-    Cv = np.nextafter(F((eta[1] + H3 * eta[2]) * (1.0 + 2.0 ** -19)), F(np.inf))
+    with np.errstate(all="ignore"):
+        Cu = np.nextafter(F((eta[0] + W3 * eta[2]) * (1.0 + 2.0 ** -19)), F(np.inf)) if ok else F(np.inf)
+        Cv = np.nextafter(F((eta[1] + H3 * eta[2]) * (1.0 + 2.0 ** -19)), F(np.inf)) if ok else F(np.inf)
     hDu = np.nextafter(F(0.5 - (W3 * 2.0 ** -22 * (1.0 + 2.0 ** -10) + 2.0 ** -20)), F(-np.inf))
     hDv = np.nextafter(F(0.5 - (H3 * 2.0 ** -22 * (1.0 + 2.0 ** -10) + 2.0 ** -20)), F(-np.inf))
     return Cu, Cv, hDu, hDv
