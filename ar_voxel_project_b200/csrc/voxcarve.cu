@@ -1398,11 +1398,12 @@ int vc_fast_carve(vc_engine* e, int32_t mode) {
     vc_flood_seed_kernel<<<1, 1, 0, e->stream>>>(occ, F);
     const long long n_rows = (long long)Y * Z;
     // a round = sweeps along x, y, z; the device-side "changed" flag is read back only every VC_FLOOD_POLL rounds (a round after
-    // convergence changes nothing, so at most VC_FLOOD_POLL - 1 rounds are wasted against a host round trip saved per round)
+    // convergence changes nothing, so at most VC_FLOOD_POLL - 1 rounds are wasted against a host round trip saved per round).
+    // The flood only gains bits, and only carved ones, so a batch that changes something reaches at least one more carved voxel:
+    // the loop ends after at most (carved voxels + 1) batches without a cap, however winding the component is.
     const int VC_FLOOD_POLL = 4;
-    int rounds = 0;
+    uint64_t rounds = 0;
     for (;;) {
-        if (rounds > 100000) return fail(e, VC_ERR_STATE, "vc_fast_carve: flood did not converge");
         VC_CUDA(e, cudaMemsetAsync(d_changed, 0, sizeof(int), e->stream));
         for (int k = 0; k < VC_FLOOD_POLL; k++, rounds++) {
             vc_flood_x_kernel<<<(unsigned)((n_rows + 127) / 128), 128, 0, e->stream>>>(occ, F, Wx, n_rows, X, d_changed);
@@ -1419,7 +1420,7 @@ int vc_fast_carve(vc_engine* e, int32_t mode) {
     vc_flood_finish_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->stream>>>(F, occ, seen, X, Y, Z, Wx);
     VC_CUDA(e, cudaGetLastError());
     VC_CUDA(e, cudaStreamSynchronize(e->stream));
-    e->stats.flood_rounds = (uint64_t)rounds;
+    e->stats.flood_rounds = rounds;
     return VC_OK;
 }
 

@@ -200,7 +200,11 @@ VC_EXPORT int vc_carve_download_sparse(vc_engine* e, uint8_t* brick_flags, uint6
                                        uint64_t listed_capacity, uint64_t* n_listed);
 /* fastCarve() (VoxelCarving.h:31, VoxelCarving.cpp:74-167): starts from the Model constructor state (it resets the
  * volumes itself) and needs the whole grid on this engine.  Refused (a slab engine, no views or masks, an unknown mode), it
- * leaves the volumes as they were. */
+ * leaves the volumes as they were.  It answers for every carved set: the flood from voxel (0,0,0) runs sweep rounds until
+ * one changes nothing (vc_stats.flood_rounds).  Its cost grows with the turns on the longest path from the origin through
+ * the component.  One round follows straight runs, and staircases inside a 32-voxel word, as far as they go (C4's exterior
+ * takes 8 rounds).  On a path that turns at every voxel and crosses a word edge at every x step, a round advances only about
+ * 1.5 voxels. */
 VC_EXPORT int vc_fast_carve(vc_engine* e, int32_t mode);
 /* reconstructClosestColor / reconstructAvgColor (ColorReconstruction.h:131,142): colours every
  * surface voxel (alpha != 0 && !isInner, ColorReconstruction.h:46) of this slab. */
